@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the registration hot path on B200, measured.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One STEP = one complete ICP registration of the workload BASELINE.json quotes its metric on
 (configs[1]): an ETH-Apartment-shaped synthetic scan pair (344 sweeps x 1077 beams, ~370k points
@@ -44,6 +44,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -109,9 +110,9 @@ def _save_pair_cache(cache, src, tgt):
 
 
 def make_pair(pair_index=0, n_sweeps=344, n_beams=1077):
-    """Synthetic ETH-shaped pair; cached under /tmp because k=5 PCA normals of 370k points take seconds."""
+    """Synthetic ETH-shaped pair; cached in the temporary directory because k=5 PCA normals of 370k points take seconds."""
     from icp_variants_b200 import synth
-    cache = f"/tmp/icp_b200_pair_{n_sweeps}x{n_beams}_{pair_index}.npz"
+    cache = os.path.join(tempfile.gettempdir(), f"icp_b200_pair_{n_sweeps}x{n_beams}_{pair_index}.npz")
     hit = _load_pair_cache(cache)
     if hit is not None:
         return hit
@@ -131,7 +132,7 @@ def device_normals_fn(ctx):
 
 def make_pair_device_normals(ctx, pair_index, n_sweeps, n_beams):
     from icp_variants_b200 import synth
-    cache = f"/tmp/icp_b200_pairdn_{n_sweeps}x{n_beams}_{pair_index}.npz"
+    cache = os.path.join(tempfile.gettempdir(), f"icp_b200_pairdn_{n_sweeps}x{n_beams}_{pair_index}.npz")
     hit = _load_pair_cache(cache)
     if hit is not None:
         return hit
@@ -180,6 +181,14 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: one DIR/<name>.npy (float32) per array, so that two builds can be compared output for output on the
+    same seeded inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float32))
+
+
 def workload_config(ns, nt, max_d2):
     """The workload both arms run (BASELINE.json configs[1]); identical in both arms' lines."""
     return {"workload": WORKLOAD, "n_source": ns, "n_target": nt, "iterations": N_ITER, "max_distance_sq": max_d2,
@@ -193,7 +202,7 @@ def host_threads():
 
 def ref_registration(src, tgt, max_d2, iters, threads):
     """The reference's own LinearICPOptimizer::estimatePose (oracle/_ref) for `iters` iterations on `threads` matcher threads.
-    Returns seconds, or None when the library is unavailable."""
+    Returns (seconds, pose), or None when the library is unavailable."""
     try:
         from oracle import ref
         if ref.build() is None:
@@ -203,7 +212,7 @@ def ref_registration(src, tgt, max_d2, iters, threads):
         n, pose, _ = ref.estimate_pose(0, 1, src.points, src.normals, src.colors, tgt.points, tgt.normals, tgt.colors,
                                        src.points[:4], tgt.points[:4], n_iterations=iters, max_distance_sq=max_d2)
         dt = time.perf_counter() - t0
-        return dt if n == iters else None
+        return (dt, pose) if n == iters else None
     except Exception as e:   # noqa: BLE001 -- the baseline must never take the bench down
         print(f"bench: reference library unavailable ({e}); using the oracle port", file=sys.stderr)
         return None
@@ -216,29 +225,30 @@ def port_registration(src, tgt, max_d2, iters, threads):
     orc.set_num_threads(threads)
     cfg = orc.Config(metric=1, minimizer=0, max_distance_sq=max_d2, n_iterations=iters)
     t0 = time.perf_counter()
-    orc.estimate_pose(cfg, src.points, src.normals, src.colors, tgt.points, tgt.normals, tgt.colors)
-    return time.perf_counter() - t0
+    _, pose, _, _ = orc.estimate_pose(cfg, src.points, src.normals, src.colors, tgt.points, tgt.normals, tgt.colors)
+    return time.perf_counter() - t0, pose
 
 
 def cpu_registration(src, tgt, max_d2, iters, threads):
-    """(seconds, kind) of one CPU registration of `iters` iterations."""
-    dt = ref_registration(src, tgt, max_d2, iters, threads)
-    if dt is not None:
-        return dt, "reference"
-    return port_registration(src, tgt, max_d2, iters, threads), "port"
+    """(seconds, kind, pose) of one CPU registration of `iters` iterations."""
+    r = ref_registration(src, tgt, max_d2, iters, threads)
+    if r is not None:
+        return r[0], "reference", r[1]
+    dt, pose = port_registration(src, tgt, max_d2, iters, threads)
+    return dt, "port", pose
 
 
 def cpu_baseline_block(src, tgt, max_d2):
     """cpu_baseline of the GPU arm's line: one full registration on all host threads (the value), a bounded 1-thread sample, and
     the FLANN-like approximate matcher with its match rate."""
     cores = host_threads()
-    dt, kind = cpu_registration(src, tgt, max_d2, N_ITER, cores)
+    dt, kind, _ = cpu_registration(src, tgt, max_d2, N_ITER, cores)
     out = {"value": 1.0 / dt, "unit": "reg/s", "cores": cores, "kind": kind, "seconds": dt,
            "sample": f"one full {N_ITER}-iteration registration of the same {len(src)}-point pair (index build included), exact kd-tree matcher on "
                      f"{cores} OpenMP threads, the rest of the loop single-threaded as in the reference"}
     # the reference is single-threaded apart from Ceres (no OpenMP flag, CMakeLists.txt:50-63): 1-thread figure from a bounded sample
-    t1, _ = cpu_registration(src, tgt, max_d2, 1, 1)
-    t2, _ = cpu_registration(src, tgt, max_d2, 2, 1)
+    t1, _, _ = cpu_registration(src, tgt, max_d2, 1, 1)
+    t2, _, _ = cpu_registration(src, tgt, max_d2, 2, 1)
     one = t1 + (N_ITER - 1) * max(t2 - t1, 0.0)
     out["one_core"] = {"value": 1.0 / one, "unit": "reg/s", "cores": 1, "seconds_estimated": one,
                        "sample": f"bounded: a 1-iteration ({t1:.2f} s) and a 2-iteration ({t2:.2f} s) run on one thread, extended to {N_ITER} iterations "
@@ -267,11 +277,13 @@ def run_reference(args):
     os.environ["OMP_NUM_THREADS"] = str(cores)          # torchrun exports 1; the baseline may use every host core
     kind = "port"
     for _ in range(args.warmup):
-        _, kind = cpu_registration(src, tgt, args.max_dist2, N_ITER, cores)
+        _, kind, _ = cpu_registration(src, tgt, args.max_dist2, N_ITER, cores)
     times = []
     for _ in range(args.steps):
-        dt, kind = cpu_registration(src, tgt, args.max_dist2, N_ITER, cores)
+        dt, kind, pose = cpu_registration(src, tgt, args.max_dist2, N_ITER, cores)
         times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"pose": pose})
     per_reg = statistics.mean(times)
     value = 1.0 / per_reg
     sample = (f"every step = one full {N_ITER}-iteration registration of the same {len(src)}-point pair (index build included); exact kd-tree "
@@ -300,7 +312,7 @@ def pair_queue_block(torch, dist, capi, ctx, stream, world, rank, dev, args):
     dynamic = world > 1 and not args.static_deal and hasattr(dist.distributed_c10d, "_get_default_store")
     mine = parallel.shard_pairs(N_SEQUENCE_PAIRS, world, rank)
     t0 = time.perf_counter()
-    pairs = {k: make_pair_device_normals(ctx, k, args.sweeps, args.beams) for k in mine}     # (also fills the /tmp cache)
+    pairs = {k: make_pair_device_normals(ctx, k, args.sweeps, args.beams) for k in mine}     # (also fills the pair cache)
     if dynamic:
         # every rank must be able to read every pair: the ranks generated disjoint shares into the cache, now each loads the rest
         dist.barrier()
@@ -463,7 +475,12 @@ def main():
     ap.add_argument("--pageable-queue", action="store_true", help="pair_queue_44 from pageable host arrays (default: page-locked)")
     ap.add_argument("--no-sharded", action="store_true", help="skip sharded_3m only")
     ap.add_argument("--no-flush", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the 4x4 pose each timed arm returned in its last step (rank 0) as DIR/pose.npy "
+                         "(device-resident clouds; with --impl reference, the CPU registration) and DIR/pose_e2e.npy (host arrays), float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -555,6 +572,8 @@ def main():
     total_ms, launches, pose = timed(step_resident, args.steps, args.warmup)
     e2e_ms, _, pose_e2e = timed(step_e2e, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"pose": pose, "pose_e2e": pose_e2e})
 
     # per-kernel timing of the dominant kernel: one extra registration, launch by launch with CUDA events
     ctx.set_target_dev(d["tp"].data_ptr(), d["tn"].data_ptr(), d["tc"].data_ptr(), nt)

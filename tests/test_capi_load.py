@@ -34,10 +34,10 @@ def test_abi_version_and_default_config(lib):
     assert abs(c.max_distance_sq - 0.0003) < 1e-9 and c.color_icp == 0 and c.multires == 0 and c.lm_max_iterations == 10
 
 
-def test_config_struct_layout_matches_header():
+def test_config_struct_layout_matches_header(tmp_path):
     """sizeof(icp_gpu_config) as the C compiler sees it == the ctypes mirror."""
     src = '#include "icp_gpu.h"\n#include <stdio.h>\nint main(){printf("%zu %zu %zu", sizeof(icp_gpu_config), sizeof(icp_gpu_timings), sizeof(icp_gpu_stats));return 0;}'
-    exe = "/tmp/icp_gpu_sizeof"
+    exe = str(tmp_path / "icp_gpu_sizeof")
     subprocess.run(["gcc", "-x", "c", "-", "-I", os.path.dirname(capi.HEADER_PATH), "-o", exe], input=src, text=True, check=True)
     sizes = [int(x) for x in subprocess.run([exe], stdout=subprocess.PIPE, text=True, check=True).stdout.split()]
     assert sizes == [C.sizeof(capi.Config), C.sizeof(capi.Timings), C.sizeof(capi.Stats)]
@@ -58,11 +58,11 @@ def test_pose_layout_roundtrip():
     assert np.array_equal(capi.pose_from_c(v), p)
 
 
-def test_header_constants_match_the_python_mirror():
+def test_header_constants_match_the_python_mirror(tmp_path):
     """Error codes and the peer-exchange constants as the C compiler sees them == capi.py."""
     src = ('#include "icp_gpu.h"\n#include <stdio.h>\nint main(){printf("%d %d %d %d %d %d %d %d %d", ICP_GPU_E_CUDA, ICP_GPU_E_ARG, ICP_GPU_E_STATE, '
            'ICP_GPU_E_NO_MATCHES, ICP_GPU_E_NUMERIC, ICP_GPU_E_PEER, ICP_GPU_MAX_PEERS, ICP_GPU_PEER_HANDLE_BYTES, ICP_GPU_MAX_PARTIALS);return 0;}')
-    exe = "/tmp/icp_gpu_consts"
+    exe = str(tmp_path / "icp_gpu_consts")
     subprocess.run(["gcc", "-x", "c", "-", "-I", os.path.dirname(capi.HEADER_PATH), "-o", exe], input=src, text=True, check=True)
     vals = [int(x) for x in subprocess.run([exe], stdout=subprocess.PIPE, text=True, check=True).stdout.split()]
     assert vals == [capi.E_CUDA, capi.E_ARG, capi.E_STATE, capi.E_NO_MATCHES, capi.E_NUMERIC, capi.E_PEER, capi.MAX_PEERS,

@@ -10,32 +10,38 @@ import pytest
 from icp_variants_b200 import capi
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EXE = "/tmp/icp_b200_bunny_driver"
 
 
-def build_driver():
+def build_driver(out_dir):
     capi.build()
     libdir = os.path.dirname(capi.LIB_PATH)
+    exe = str(out_dir / "icp_b200_bunny_driver")
     cmd = ["g++", "-std=c++14", "-Wall", "-Wextra", "-Werror", "-I", os.path.join(ROOT, "include"),
-           os.path.join(ROOT, "examples", "bunny_driver.cpp"), "-o", EXE, "-L", libdir, "-licp_gpu", f"-Wl,-rpath,{libdir}"]
+           os.path.join(ROOT, "examples", "bunny_driver.cpp"), "-o", exe, "-L", libdir, "-licp_gpu", f"-Wl,-rpath,{libdir}"]
     subprocess.run(cmd, check=True)
-    return EXE
+    return exe
 
 
-def test_dropin_headers_compile_as_cpp14():
-    build_driver()
-    # the matcher classes alone, as a reference user would instantiate them
+def build_nn_check(out_dir):
+    """The matcher classes alone, as a reference user would instantiate them."""
     src = '#include "icp_b200/NearestNeighbor.h"\nint main(){ NearestNeighborSearchFlann f; NearestNeighborSearchProjective p; NearestNeighborSearchBruteForce b; f.setMatchingMaxDistance(0.1f); return (int)f.queryMatches({}).size(); }\n'
     libdir = os.path.dirname(capi.LIB_PATH)
-    subprocess.run(["g++", "-std=c++14", "-x", "c++", "-", "-I", os.path.join(ROOT, "include"), "-o", "/tmp/icp_b200_nn_check",
+    exe = str(out_dir / "icp_b200_nn_check")
+    subprocess.run(["g++", "-std=c++14", "-x", "c++", "-", "-I", os.path.join(ROOT, "include"), "-o", exe,
                     "-L", libdir, "-licp_gpu", f"-Wl,-rpath,{libdir}"], input=src, text=True, check=True)
+    return exe
 
 
-def test_driver_without_gpu_reports_and_does_not_hang():
+def test_dropin_headers_compile_as_cpp14(tmp_path):
+    build_driver(tmp_path)
+    build_nn_check(tmp_path)
+
+
+def test_driver_without_gpu_reports_and_does_not_hang(tmp_path):
     if capi.lib().icp_gpu_device_count() > 0:
         pytest.skip("a GPU is present")
-    exe = build_driver()
-    r = subprocess.run(["/tmp/icp_b200_nn_check"], stdout=subprocess.PIPE, text=True, timeout=60)
+    exe = build_driver(tmp_path)
+    r = subprocess.run([build_nn_check(tmp_path)], stdout=subprocess.PIPE, text=True, timeout=60)
     assert "no usable CUDA device" in r.stdout and r.returncode == 0
     assert os.path.exists(exe)
 
@@ -49,12 +55,13 @@ def _dump(path, cloud):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("linear,metric", [(1, 0), (1, 1), (1, 2), (0, 1)])
-def test_cpp_driver_matches_python_binding(bunny, linear, metric):
+def test_cpp_driver_matches_python_binding(bunny, linear, metric, tmp_path):
     src, tgt, _, _ = bunny
-    exe = build_driver()
-    _dump("/tmp/icp_b200_src.bin", src)
-    _dump("/tmp/icp_b200_tgt.bin", tgt)
-    r = subprocess.run([exe, "/tmp/icp_b200_src.bin", "/tmp/icp_b200_tgt.bin", str(linear), str(metric), "20"],
+    exe = build_driver(tmp_path)
+    src_bin, tgt_bin = str(tmp_path / "src.bin"), str(tmp_path / "tgt.bin")
+    _dump(src_bin, src)
+    _dump(tgt_bin, tgt)
+    r = subprocess.run([exe, src_bin, tgt_bin, str(linear), str(metric), "20"],
                        stdout=subprocess.PIPE, text=True, check=True, timeout=120)
     line = [l for l in r.stdout.splitlines() if l.startswith("POSE")][0]
     pose_cpp = capi.pose_from_c(np.array(line.split()[1:], np.float32))
@@ -75,18 +82,18 @@ def test_cpp_driver_matches_python_binding(bunny, linear, metric):
     assert float(f[3]) == pytest.approx(orc.benchmark_error(pose_py, src.points[gs], tgt.points[gt]), rel=1e-6)
 
 
-def build_value_driver():
+def build_value_driver(out_dir):
     capi.build()
     libdir = os.path.dirname(capi.LIB_PATH)
-    exe = "/tmp/icp_b200_value_driver"
+    exe = str(out_dir / "icp_b200_value_driver")
     cmd = ["g++", "-std=c++14", "-Wall", "-Wextra", "-Werror", "-I", os.path.join(ROOT, "include"),
            os.path.join(ROOT, "examples", "value_classes_driver.cpp"), "-o", exe, "-L", libdir, "-licp_gpu", f"-Wl,-rpath,{libdir}"]
     subprocess.run(cmd, check=True)
     return exe
 
 
-def test_value_classes_compile_as_cpp14():
-    build_value_driver()
+def test_value_classes_compile_as_cpp14(tmp_path):
+    build_value_driver(tmp_path)
 
 
 def _fingerprint(a):
@@ -96,16 +103,17 @@ def _fingerprint(a):
 
 
 @pytest.mark.gpu
-def test_value_classes_driver_equals_oracle(bunny):
+def test_value_classes_driver_equals_oracle(bunny, tmp_path):
     """PointSelection, WeightingMethod, the three functors, ProcrustesAligner, PoseIncrement, transformPoints / transformNormals,
     PointCloud::change_pose and ConvergenceMeasure as a C++ user of the reference holds them -- each a thin class over an icp_gpu_* call
     (include/icp_b200/) -- against the oracle: bit-exact transforms / matches / weights, 1e-5 poses, the functor values to 1e-12."""
     from oracle import oracle as orc
     src, tgt, _, _ = bunny
-    exe = build_value_driver()
-    _dump("/tmp/icp_b200_src.bin", src)
-    _dump("/tmp/icp_b200_tgt.bin", tgt)
-    r = subprocess.run([exe, "/tmp/icp_b200_src.bin", "/tmp/icp_b200_tgt.bin"], stdout=subprocess.PIPE, text=True, check=True, timeout=120)
+    exe = build_value_driver(tmp_path)
+    src_bin, tgt_bin = str(tmp_path / "src.bin"), str(tmp_path / "tgt.bin")
+    _dump(src_bin, src)
+    _dump(tgt_bin, tgt)
+    r = subprocess.run([exe, src_bin, tgt_bin], stdout=subprocess.PIPE, text=True, check=True, timeout=120)
     out = {l.split()[0]: l.split()[1:] for l in r.stdout.splitlines() if l and l.split()[0].isupper()}
     pose = capi.pose_from_c(np.array(out["POSE"], np.float32))
     x = np.array([0.01, -0.02, 0.03, 0.001, 0.002, -0.001])

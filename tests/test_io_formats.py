@@ -7,8 +7,9 @@ import pytest
 
 from icp_variants_b200 import io as fio
 from icp_variants_b200 import synth
+from oracle import ref as R
 
-REF_DATA = "/root/reference/Data"
+REF_DATA = os.path.join(R.REFERENCE_ROOT, "Data")
 
 
 def test_off_round_trip_and_rules(tmp_path, bunny):
@@ -36,9 +37,8 @@ def test_off_round_trip_and_rules(tmp_path, bunny):
         fio.read_off(p)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="bundled .off files live in /root/reference")
+@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="the reference's bundled .off files (ICP_REFERENCE_ROOT/Data) are absent")
 def test_off_reader_equals_reference_loader(tmp_path, bunny):
-    from oracle import ref as R
     src, tgt, _, _ = bunny
     for name, cloud in (("bunny_part1.off", tgt), ("bunny_part2_trans.off", src)):
         v, c, f = fio.read_off(os.path.join(REF_DATA, name))

@@ -11,6 +11,12 @@ defaults, ICPOptimizer.h:352-360), so its answer is not the minimiser but lies w
 require   cost(x_LM) <= cost(x*) * (1 + 2e-6)   and   |x_LM - x*| <= 5e-4   for the oracle's LM, for the reference build's LM and for
 the device's LM.  What stays unpinned: Ceres' exact iterate sequence (radius schedule, accept / reject decisions) when it does NOT
 converge within max_num_iterations = 10 -- no Ceres binary exists in this environment to compare with.
+
+Where the reference build is absent the residuals are the functors' closed forms in oracle/oracle_as_ref.py, checked against the
+build by tests/test_oracle_vs_reference.py::test_oracle_as_ref_answers_like_the_reference where it exists and against scipy's
+axis-angle rotation in every checkout (tests/test_reference_golden.py).  They are numpy, not the oracle's C jets, so the oracle's and
+the device's LM reaching their minimum still pins two independent statements of the functors against each other; the reference
+build's own LM is then not run.
 """
 import numpy as np
 import pytest
@@ -19,9 +25,9 @@ from scipy.spatial.transform import Rotation
 
 from icp_variants_b200 import synth
 from oracle import oracle as O
-from oracle import ref as R
+from oracle import oracle_as_ref, ref
 
-pytestmark = pytest.mark.skipif(not R.available(), reason="oracle/_ref/libicp_ref.so not built")
+R = ref if ref.available() else oracle_as_ref
 
 
 def _problem(metric):
@@ -61,6 +67,8 @@ def test_oracle_and_reference_lm_reach_the_independent_minimum(metric):
     assert _cost(residuals, x) <= sol.cost * (1 + 2e-6)
     assert np.abs(x - sol.x).max() <= 5e-4
     assert _cost(residuals, np.zeros(6)) > 1.2 * sol.cost                      # the problem is not trivial
+    if not ref.available():
+        return
     # the reference's CeresICPOptimizer (over the Ceres stand-in), one outer iteration from the identity
     n, pose_r, _ = R.estimate_pose(1, metric, src.points, src.normals, src.colors, tgt.points, tgt.normals, tgt.colors, src.points[:4], tgt.points[:4],
                                    n_iterations=1, max_distance_sq=0.0003)

@@ -1,5 +1,5 @@
 """Pins oracle/icp_oracle.c against the reference's OWN code: oracle/_ref/libicp_ref.so is the
-reference's headers (/root/reference/icp-variants/*.h) compiled where they lie against the
+reference's headers (ICP_REFERENCE_ROOT/icp-variants/*.h) compiled where they lie against the
 stand-ins of oracle/ref_shim/ (Eigen / FLANN / Ceres / PCL are not installed; see
 oracle/ref_driver.cpp for what that does and does not pin).
 
@@ -17,7 +17,7 @@ import pytest
 from oracle import oracle as O
 from oracle import ref as R
 
-pytestmark = pytest.mark.skipif(not R.available(), reason="neither /root/reference nor a prebuilt oracle/_ref/libicp_ref.so")
+pytestmark = pytest.mark.skipif(not R.available(), reason="neither the reference sources (ICP_REFERENCE_ROOT) nor a prebuilt oracle/_ref/libicp_ref.so")
 
 ROT_TOL = 1e-5   # rad
 TRANS_TOL = 1e-5  # m
@@ -52,11 +52,11 @@ def test_describe_says_what_is_pinned():
     assert "stand-ins" in R.describe()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/Data"), reason="bundled .off files live in /root/reference")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(R.REFERENCE_ROOT, "Data")), reason="the reference's bundled .off files (ICP_REFERENCE_ROOT/Data) are absent")
 def test_bunny_fixture_equals_reference_loader(bunny):
     src, tgt, _, _ = bunny
     for cloud, name in ((tgt, "bunny_part1.off"), (src, "bunny_part2_trans.off")):
-        p, n = R.cloud_from_off(f"/root/reference/Data/{name}")      # SimpleMesh::loadMesh + PointCloud(mesh)
+        p, n = R.cloud_from_off(os.path.join(R.REFERENCE_ROOT, "Data", name))      # SimpleMesh::loadMesh + PointCloud(mesh)
         assert np.array_equal(p, cloud.points)
         assert np.array_equal(n, cloud.normals)
 
@@ -440,3 +440,59 @@ def test_reference_brute_force_as_written_norm_threshold():
         m = O.knn_brute_norm(tgt, qry, max_d)
         assert np.array_equal(idx, m["idx"]) and np.array_equal(w, m["weight"])
     assert (R.knn_brute(tgt, qry, 0.05)[0] < 0).any() and (R.knn_brute(tgt, qry, 0.05)[0] >= 0).any()
+
+
+def test_oracle_as_ref_answers_like_the_reference(bunny, small_eth_pair):
+    """oracle/oracle_as_ref.py -- what the device-vs-reference tests call where this build is absent -- through the same calls
+    those tests make, against the reference build, at their tolerances: matching / weighting / rejection, projective, the
+    brute-force norm threshold and the depth constructor bit-exact, the functor residuals to 1e-12, the linear solvers and the
+    three setter orders to 1e-5 rad / 1e-5 m."""
+    from icp_variants_b200 import synth
+    from oracle import oracle_as_ref as S
+    src, tgt, _ = small_eth_pair
+    sc, tc = synth.procedural_colors(src.points), synth.procedural_colors(tgt.points)
+    pose = _pose(2, 0.05, 2.0)
+    q, qn = S.transform_points(pose, src.points), S.transform_normals(pose, src.normals)
+    assert np.array_equal(q, R.transform_points(pose, src.points), equal_nan=True)
+    assert np.array_equal(qn, R.transform_normals(pose, src.normals), equal_nan=True)
+    for color in (False, True):
+        a = (tc, sc) if color else (None, None)
+        i0, w0 = R.knn_flann(tgt.points, q, 0.5, *a)
+        assert all(np.array_equal(x, y) for x, y in zip(S.knn_flann(tgt.points, q, 0.5, *a), (i0, w0)))
+        for method in (0, 1, 2, 3):
+            r = R.prune(qn, tgt.normals, *R.apply_weights(method, 0.5, q, qn, sc, tgt.points, tgt.normals, tc, i0, w0))
+            s = S.prune(qn, tgt.normals, *S.apply_weights(method, 0.5, q, qn, sc, tgt.points, tgt.normals, tc, i0, w0))
+            assert np.array_equal(r[0], s[0]) and np.array_equal(r[1], s[1], equal_nan=True)
+    w, h = 160, 120
+    ps, pt, K, gt = synth.tum_pair(seed=13, width=w, height=h)
+    qp = S.transform_points(gt, ps.points)
+    r, s = (M.projective(pt.points, w, h, K[0, 0], K[1, 1], K[0, 2], K[1, 2], qp, 0.1) for M in (R, S))
+    fin = np.isfinite(qp).all(1)
+    assert np.array_equal(r[0][fin], s[0][fin]) and (r[0] >= 0).sum() > 1000
+    bt, _, _ = _cloud(1500, 6, quant=8)
+    bq, _, _ = _cloud(1000, 7, quant=8)
+    for max_d in (0.05, 0.3):
+        assert all(np.array_equal(x, y) for x, y in zip(R.knn_brute(bt, bq, max_d), S.knn_brute(bt, bq, max_d)))
+    depth, _ = synth.render_depth(synth.make_room(3), np.array([3.0, 5.0, 1.4]), 10.0, 0.0, 96, 72, 78.75, 78.75, 47.5, 35.5, seed=3)
+    rgbx = np.random.default_rng(1).integers(0, 256, 4 * 96 * 72, dtype=np.uint8)
+    for keep, ds in ((True, 1), (False, 1), (False, 8)):
+        r, s = (M.cloud_from_depth(depth, rgbx, 78.75, 78.75, 47.5, 35.5, None, keep, ds, 0.1) for M in (R, S))
+        assert all(np.array_equal(x, y, equal_nan=True) for x, y in zip(r, s))
+    keep = i0 >= 0
+    s_, d_, ns_, nt_ = q[keep], tgt.points[i0[keep]], qn[keep], tgt.normals[i0[keep]]
+    wt = np.random.default_rng(2).uniform(0.2, 1.0, len(s_)).astype(np.float32)
+    c0 = d_.mean(0)
+    for metric in (0, 1, 2):
+        ss, dd = ((s_ - c0).astype(np.float32), (d_ - c0).astype(np.float32)) if metric == 0 else (s_, d_)
+        (rc_r, pr), (rc_s, ps_) = R.solve_linear(metric, ss, dd, ns_, nt_, wt), S.solve_linear(metric, ss, dd, ns_, nt_, wt)
+        assert rc_r == rc_s == 0 and rot_err(pr, ps_) < ROT_TOL and np.abs(pr[:3, 3] - ps_[:3, 3]).max() < TRANS_TOL
+    rng = np.random.default_rng(3)
+    for x in (np.zeros(6), np.r_[1e-9, -2e-9, 1e-9, 0.1, 0.2, 0.3], rng.normal(0, 0.3, 6)):
+        v = [rng.normal(size=3).astype(np.float32) for _ in range(4)]
+        for kind in (0, 1, 2):
+            assert np.allclose(S.residuals(kind, x, *v, 0.7), R.residuals(kind, x, *v, 0.7), rtol=0, atol=1e-12)
+    bs, bt_, gs, gt_ = bunny
+    for order in (0, 1, 2):
+        r, s = (M.estimate_pose(0, 1, bs.points, bs.normals, bs.colors, bt_.points, bt_.normals, bt_.colors, bs.points[gs], bt_.points[gt_],
+                                n_iterations=5, max_distance_sq=0.002, weighting=1, setter_order=order) for M in (R, S))
+        assert r[0] == s[0] == 5 and rot_err(r[1], s[1]) < ROT_TOL and np.abs(r[1][:3, 3] - s[1][:3, 3]).max() < TRANS_TOL

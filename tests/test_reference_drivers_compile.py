@@ -7,19 +7,21 @@ How: an overlay directory of symbolic links (nothing is copied) -- the drivers a
 drop-in where one exists.  Third-party headers are the stand-ins of oracle/ref_shim (Eigen, PCL, Ceres) and tests/cpp_shim (FreeImage,
 boost::split).  Compile only (-c): the object files would need FreeImage to link and a GPU to run; the running counterpart is
 tests/test_cpp_dropin.py (examples/bunny_driver.cpp mirrors main.cpp's bunny path and is compared with the Python binding on the GPU).
-CPU only, and only where /root/reference exists."""
+CPU only, and only where the reference sources are present (ICP_REFERENCE_ROOT, see oracle/ref.py)."""
 import os
 import subprocess
 
 import pytest
 
+from oracle import ref as R
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/icp-variants"
+REF = os.path.join(R.REFERENCE_ROOT, "icp-variants")
 DROPIN = ["ConvergenceMeasure.h", "Eigen.h", "ICPOptimizer.h", "NearestNeighbor.h", "PointCloud.h", "ProcrustesAligner.h", "TimeMeasure.h",
           "constraints.h", "detail.h", "selection.h", "utils.h", "weighting.h"]
 KEPT = ["SimpleMesh.h", "BunnyDataLoader.h", "DataLoader.h", "ETHDataLoader.h", "CSVReader.h", "VirtualSensor.h", "FreeImageHelper.h"]
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="the reference sources live in /root/reference")
+pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="the reference sources (ICP_REFERENCE_ROOT/icp-variants) are absent")
 
 
 @pytest.fixture(scope="module")
