@@ -22,6 +22,7 @@ HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "icp_gpu.h")
 OK, E_CUDA, E_ARG, E_STATE, E_NO_MATCHES, E_NUMERIC, E_PEER = 0, -1, -2, -3, -4, -5, -6
 MAX_PARTIALS = 32
 MAX_PEERS, PEER_HANDLE_BYTES = 8, 64
+BATCH_MAX_TARGET = 8192
 
 
 class IcpGpuError(RuntimeError):
@@ -107,6 +108,8 @@ def lib():
             "icp_gpu_max_iterations": (C.c_int, [vp]),
             "icp_gpu_estimate_pose_async": (C.c_int, [vp, pf]),
             "icp_gpu_estimate_pose_finish": (C.c_int, [vp, pf, pf, C.POINTER(i32)]),
+            "icp_gpu_estimate_pose_batch": (C.c_int, [vp, i32, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf]),
+            "icp_gpu_estimate_pose_batch_dev": (C.c_int, [vp, i32, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf]),
             "icp_gpu_get_stats": (C.c_int, [vp, C.POINTER(Stats)]),
             "icp_gpu_measure_fp32_peak": (C.c_int, [vp, i32, C.POINTER(C.c_double)]),
             "icp_gpu_alignment_error": (C.c_int, [vp, pf, pf, C.POINTER(C.c_double)]),
@@ -175,6 +178,31 @@ def _u8(a):
     if a.ndim != 2 or a.shape[1] != 4:
         raise ValueError(f"expected [N,4] uint8, got {a.shape}")
     return a
+
+
+def _concat_clouds(clouds):
+    """Sequence of synth.Cloud / [N,3] arrays -> (points [N,3], normals [N,3] or None, offsets [B+1] int64)."""
+    pts = [_f32(getattr(c, "points", c), 3) for c in clouds]
+    nrm = [getattr(c, "normals", None) for c in clouds]
+    off = np.zeros(len(pts) + 1, np.int64)
+    off[1:] = np.cumsum([len(p) for p in pts])
+    xyz = np.concatenate(pts) if pts else np.zeros((0, 3), np.float32)
+    if all(n is None for n in nrm):
+        return xyz, None, off
+    n3 = np.concatenate([np.zeros((len(p), 3), np.float32) if n is None else _f32(n, 3) for p, n in zip(pts, nrm)]) if pts else None
+    if n3 is not None and len(n3) != len(xyz):
+        raise ValueError("every cloud needs one normal per point")
+    return xyz, n3, off
+
+
+def _batch_poses(poses, B):
+    """[B,4,4] row-major (None = identity) -> [B,16] column-major."""
+    if poses is None:
+        return np.tile(np.eye(4, dtype=np.float32).reshape(16), (B, 1))
+    p = np.asarray(poses, np.float32)
+    if p.shape != (B, 4, 4):
+        raise ValueError(f"expected [{B},4,4] poses, got {p.shape}")
+    return np.ascontiguousarray(p.transpose(0, 2, 1).reshape(B, 16))
 
 
 class Context:
@@ -288,6 +316,81 @@ class Context:
         n_it = C.c_int32(0)
         self._check(lib().icp_gpu_estimate_pose_finish(self._h, _ptr(p), None, C.byref(n_it)))
         return pose_from_c(p), n_it.value
+
+    # -- many small registrations in one launch (one thread block per pair)
+    def estimate_pose_batch(self, sources, targets, init_poses=None, want_history=False):
+        """B independent registrations with the context's configuration.  sources / targets: sequences of synth.Cloud or
+        [N,3] point arrays (no normals = zero normals); init_poses: [B,4,4] or None (identity).  Returns (poses [B,4,4],
+        n_iterations [B], status [B] (OK / E_NO_MATCHES / E_NUMERIC per pair)[, history [B, n_iterations, 4, 4], rows past
+        a pair's last iteration 0]).  A pair whose target has more than BATCH_MAX_TARGET points is refused (E_ARG)."""
+        if len(sources) != len(targets):
+            raise ValueError(f"{len(sources)} sources, {len(targets)} targets")
+        B = len(sources)
+        sp, sn, so = _concat_clouds(sources)
+        tp, tn, to = _concat_clouds(targets)
+        pin = _batch_poses(init_poses, B)
+        pout = np.zeros((B, 16), np.float32)
+        n_it = np.zeros(B, np.int32)
+        status = np.zeros(B, np.int32)
+        n_cap = self.get_config().n_iterations
+        hist = np.zeros((B, n_cap, 16), np.float32) if want_history else None
+        self._check(lib().icp_gpu_estimate_pose_batch(self._h, B, _ptr(sp), _ptr(sn), _ptr(so), _ptr(tp), _ptr(tn), _ptr(to), _ptr(pin), _ptr(pout),
+                                                      _ptr(n_it), _ptr(status), _ptr(hist)))
+        out = (pout.reshape(B, 4, 4).transpose(0, 2, 1).copy(), n_it, status)
+        return out + (hist.reshape(B, n_cap, 4, 4).transpose(0, 1, 3, 2).copy(),) if want_history else out
+
+    def estimate_pose_batch_dev(self, src_xyz, src_off, tgt_xyz, tgt_off, src_nrm=None, tgt_nrm=None, init_poses=None, want_history=False):
+        """The same on CUDA torch tensors of the context's device, without a host round trip of the clouds: concatenated
+        points / normals [N,3] float32, offsets [B+1] int64, init_poses [B,4,4] float32 (None = identity).  Returns CUDA
+        tensors (poses [B,4,4], n_iterations [B] int32, status [B] int32[, history [B, n_iterations, 4, 4]]).  Work queued on
+        the current torch stream is waited for; the results are complete when the call returns."""
+        import torch
+        dev = torch.device("cuda", self.device)
+
+        def arr(x, name, cols):
+            if x is None:
+                return None
+            if not (isinstance(x, torch.Tensor) and x.device == dev and x.dtype == torch.float32 and x.dim() == 2 and x.shape[1] == cols):
+                raise ValueError(f"{name}: expected a float32 [N,{cols}] tensor on {dev}")
+            return x.contiguous()
+
+        def offs(x, name):
+            if not (isinstance(x, torch.Tensor) and x.device == dev and x.dtype == torch.int64 and x.dim() == 1 and len(x) >= 1):
+                raise ValueError(f"{name}: expected an int64 [B+1] tensor on {dev}")
+            return x.contiguous()
+
+        sp, tp = arr(src_xyz, "src_xyz", 3), arr(tgt_xyz, "tgt_xyz", 3)
+        sn, tn = arr(src_nrm, "src_nrm", 3), arr(tgt_nrm, "tgt_nrm", 3)
+        so, to = offs(src_off, "src_off"), offs(tgt_off, "tgt_off")
+        if len(so) != len(to):
+            raise ValueError(f"{len(so) - 1} source pairs, {len(to) - 1} target pairs")
+        for x, n, name in ((sn, len(sp), "src_nrm"), (tn, len(tp), "tgt_nrm")):
+            if x is not None and len(x) != n:
+                raise ValueError(f"{name}: {len(x)} rows for {n} points")
+        ends = torch.stack([so[-1], to[-1]]).tolist()
+        if ends != [len(sp), len(tp)]:
+            raise IcpGpuError(E_ARG, f"batch: the offsets end at {ends[0]} / {ends[1]}, the clouds hold {len(sp)} / {len(tp)} points")
+        B = len(so) - 1
+        if init_poses is None:
+            pin = torch.eye(4, dtype=torch.float32, device=dev).expand(B, 4, 4)
+        else:
+            pin = init_poses
+            if not (isinstance(pin, torch.Tensor) and pin.device == dev and pin.dtype == torch.float32 and tuple(pin.shape) == (B, 4, 4)):
+                raise ValueError(f"init_poses: expected a float32 [{B},4,4] tensor on {dev}")
+        pin = pin.transpose(1, 2).contiguous()               # column-major per pose (Eigen::Matrix4f::data())
+        pout = torch.empty((B, 4, 4), dtype=torch.float32, device=dev)
+        n_it = torch.empty(B, dtype=torch.int32, device=dev)
+        status = torch.empty(B, dtype=torch.int32, device=dev)
+        hist = torch.empty((B, self.get_config().n_iterations, 4, 4), dtype=torch.float32, device=dev) if want_history else None
+
+        def p(x):
+            return None if x is None else C.c_void_p(x.data_ptr())
+
+        torch.cuda.current_stream(dev).synchronize()
+        self._check(lib().icp_gpu_estimate_pose_batch_dev(self._h, B, p(sp), p(sn), p(so), p(tp), p(tn), p(to), p(pin), p(pout), p(n_it), p(status),
+                                                          p(hist)))
+        out = (pout.transpose(1, 2).contiguous(), n_it, status)
+        return out + (hist.transpose(2, 3).contiguous(),) if want_history else out
 
     def cloud_from_depth(self, depth, rgbx, K, extrinsics=None, keep_original_size=False, downsample=1, max_distance=0.1,
                          role: int = 2, download: bool = True):

@@ -108,6 +108,7 @@ struct icp_gpu_ctx {
     DeviceBuf nrm_out_dev;
     DeviceBuf prep_in, prep_tmp, prep_out, gt_src, gt_ref, met_partial, met_out;
     DeviceBuf scratch[16];                                   // operands of the value-level entry points (transform, weights, solve)
+    DeviceBuf batch_io, batch_scratch;                       // icp_gpu_estimate_pose_batch: uploaded operands + results, symmetric match slices
     long long n_gt = 0; int last_iters = 0;
     float* h_pose = nullptr; float* h_history = nullptr; DevState* h_state = nullptr;   // pinned
     IterDesc* h_desc = nullptr;                                                       // pinned, DESC_TOTAL
@@ -148,9 +149,10 @@ int fail(icp_gpu_ctx* c, int code, const char* fmt, ...) {
         if (e__ != cudaSuccess) return fail(ctx, ICP_GPU_E_CUDA, "%s: %s", #call, cudaGetErrorString(e__)); \
     } while (0)
 
-int ensure(icp_gpu_ctx* ctx, DeviceBuf& b, size_t bytes) {
+// graph_reads = false: a buffer no captured graph refers to (the batch entry points'), so growing it keeps the cached graph
+int ensure(icp_gpu_ctx* ctx, DeviceBuf& b, size_t bytes, bool graph_reads = true) {
     if (bytes <= b.cap && b.p) return 0;
-    if (ctx->graph_exec) { cudaGraphExecDestroy(ctx->graph_exec); ctx->graph_exec = nullptr; ctx->graph_key.clear(); }
+    if (graph_reads && ctx->graph_exec) { cudaGraphExecDestroy(ctx->graph_exec); ctx->graph_exec = nullptr; ctx->graph_key.clear(); }
     if (b.p) { cudaStreamSynchronize(ctx->stream); if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream); if (ctx->aux_stream) cudaStreamSynchronize(ctx->aux_stream); cudaFree(b.p); b.p = nullptr; b.cap = 0; }
     size_t want = bytes + bytes / 8 + 256;
     CU(cudaMalloc(&b.p, want));
@@ -791,7 +793,7 @@ int icp_gpu_destroy(icp_gpu_ctx* ctx) {
                          &ctx->match_pos, &ctx->match_w, &ctx->match_idx, &ctx->partials, &ctx->pose_dev, &ctx->history,
                          &ctx->src_raw_pts, &ctx->src_raw_nrm, &ctx->sgrid, &ctx->order_dev,
                          &ctx->nn_pos, &ctx->bvh_box, &ctx->bvh_desc, &ctx->leaf_start, &ctx->leaf_rank, &ctx->node_rank, &ctx->child_start, &ctx->qbuf, &ctx->adj, &ctx->adj_box, &ctx->adj_gap, &ctx->adj1, &ctx->adj1_box, &ctx->voxel_table, &ctx->nn_leaf, &ctx->seedbuf,
-                         &ctx->nrm_out_dev, &ctx->prep_in, &ctx->prep_tmp, &ctx->prep_out, &ctx->gt_src, &ctx->gt_ref, &ctx->met_partial, &ctx->met_out};
+                         &ctx->nrm_out_dev, &ctx->batch_io, &ctx->batch_scratch, &ctx->prep_in, &ctx->prep_tmp, &ctx->prep_out, &ctx->gt_src, &ctx->gt_ref, &ctx->met_partial, &ctx->met_out};
     for (DeviceBuf* b : bufs) if (b->p) cudaFree(b->p);
     for (DeviceBuf& b : ctx->scratch) if (b.p) cudaFree(b.p);
     if (ctx->h_pose) cudaFreeHost(ctx->h_pose);
@@ -1396,6 +1398,114 @@ int icp_gpu_solve_linear(icp_gpu_ctx* ctx, int32_t metric, const float* src_xyz,
     if (st.status != 0) return fail(ctx, st.status, "singular / non-finite system");
     memcpy(pose_out, st.pose, 16 * sizeof(float));
     return ICP_GPU_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------- batched registration of small pairs (batch.cu)
+namespace {
+// dev = false: every array is a host array, uploaded into batch_io and the results copied back; dev = true: every array is a
+// device array on the context's device, read and written in place.  Either way the call waits for the batch.
+int estimate_pose_batch(icp_gpu_ctx* ctx, int32_t n_pairs, const float* src_xyz, const float* src_nrm, const int64_t* src_off,
+                        const float* tgt_xyz, const float* tgt_nrm, const int64_t* tgt_off, const float* poses_in, float* poses_out,
+                        int32_t* n_iterations_out, int32_t* status_out, float* pose_history, bool dev) {
+    if (!ctx) return ICP_GPU_E_ARG;
+    if (n_pairs < 0) return fail(ctx, ICP_GPU_E_ARG, "n_pairs %d", n_pairs);
+    if (!src_off || !tgt_off || !poses_in || !poses_out || !n_iterations_out || !status_out)
+        return fail(ctx, ICP_GPU_E_ARG, "batch: offsets, poses_in, poses_out, n_iterations_out and status_out are required");
+    if (ctx->pending) return fail(ctx, ICP_GPU_E_STATE, "a registration is pending; call icp_gpu_estimate_pose_finish first");
+    const icp_gpu_config& cfg = ctx->cfg;
+    if (cfg.minimizer != ICP_GPU_MIN_LINEAR) return fail(ctx, ICP_GPU_E_ARG, "batch: the linear minimiser only (Levenberg-Marquardt runs through icp_gpu_estimate_pose)");
+    if (cfg.multires) return fail(ctx, ICP_GPU_E_ARG, "batch: no multi-resolution schedule (run it through icp_gpu_estimate_pose)");
+    if (cfg.matching != ICP_GPU_MATCH_KNN) return fail(ctx, ICP_GPU_E_ARG, "batch: k-NN matching only (projective matching runs through icp_gpu_estimate_pose)");
+    if (cfg.color_icp) return fail(ctx, ICP_GPU_E_ARG, "batch: 3-D matching only (colour ICP runs through icp_gpu_estimate_pose)");
+    if (cfg.nn_algorithm == ICP_GPU_NN_BRUTE_NORM) return fail(ctx, ICP_GPU_E_ARG, "batch: squared-distance matching only (no norm-thresholded brute force)");
+    if (cfg.selection == ICP_GPU_SELECT_RANDOM && cfg.selection_rng != ICP_GPU_RNG_DEVICE)
+        return fail(ctx, ICP_GPU_E_ARG, "batch: random selection needs the device stream (selection_rng = ICP_GPU_RNG_DEVICE); mt19937 selection runs through icp_gpu_estimate_pose");
+    if (bind(ctx)) return ICP_GPU_E_CUDA;
+    if (n_pairs == 0) return ICP_GPU_OK;
+    const size_t B = (size_t)n_pairs;
+    std::vector<int64_t> so(B + 1), to(B + 1);
+    if (dev) {
+        CU(cudaMemcpyAsync(so.data(), src_off, (B + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaMemcpyAsync(to.data(), tgt_off, (B + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+    } else {
+        memcpy(so.data(), src_off, (B + 1) * 8); memcpy(to.data(), tgt_off, (B + 1) * 8);
+    }
+    if (so[0] != 0 || to[0] != 0) return fail(ctx, ICP_GPU_E_ARG, "batch: the offsets must start at 0 (src %lld, tgt %lld)", (long long)so[0], (long long)to[0]);
+    int max_tgt = 0;
+    for (size_t b = 0; b < B; ++b) {
+        if (so[b + 1] < so[b] || to[b + 1] < to[b]) return fail(ctx, ICP_GPU_E_ARG, "batch: offsets of pair %zu are not monotone", b);
+        const int64_t nt = to[b + 1] - to[b];
+        if (nt > ICP_BATCH_MAX_TARGET)
+            return fail(ctx, ICP_GPU_E_ARG, "batch: pair %zu has %lld target points, more than the %d a block stages; register it with icp_gpu_estimate_pose",
+                        b, (long long)nt, ICP_BATCH_MAX_TARGET);
+        if (nt > max_tgt) max_tgt = (int)nt;
+    }
+    const int64_t ns = so[B], nt = to[B];
+    if (ns > 0x7fffffff / 4 || nt > 0x7fffffff / 4) return fail(ctx, ICP_GPU_E_ARG, "batch: %lld source / %lld target points in all", (long long)ns, (long long)nt);
+    if ((ns > 0 && !src_xyz) || (nt > 0 && !tgt_xyz)) return fail(ctx, ICP_GPU_E_ARG, "batch: null point array");
+    const int n_it = cfg.n_iterations;
+    const size_t hist_floats = B * (size_t)n_it * 16;
+
+    BatchArgs a; memset(&a, 0, sizeof(a));
+    a.src_xyz = src_xyz; a.src_nrm = src_nrm; a.src_off = (const long long*)src_off;
+    a.tgt_xyz = tgt_xyz; a.tgt_nrm = tgt_nrm; a.tgt_off = (const long long*)tgt_off;
+    a.poses_in = poses_in; a.poses_out = poses_out; a.n_iter_out = n_iterations_out; a.status_out = status_out; a.history = pose_history;
+    if (!dev) {
+        // one upload area, segments 256-byte aligned: inputs, then the results the kernel writes
+        const size_t sizes[] = {(size_t)ns * 12, src_nrm ? (size_t)ns * 12 : 0, (size_t)nt * 12, tgt_nrm ? (size_t)nt * 12 : 0, (B + 1) * 8, (B + 1) * 8,
+                                B * 64, B * 64, B * 4, B * 4, pose_history ? hist_floats * 4 : 0};
+        const void* host_in[] = {src_xyz, src_nrm, tgt_xyz, tgt_nrm, src_off, tgt_off, poses_in};
+        size_t off[11], total = 0;
+        for (int k = 0; k < 11; ++k) { off[k] = total; total += (sizes[k] + 255) / 256 * 256; }
+        if (ensure(ctx, ctx->batch_io, total, false)) return ICP_GPU_E_CUDA;
+        char* base = (char*)ctx->batch_io.p;
+        for (int k = 0; k < 7; ++k) if (sizes[k]) CU(cudaMemcpyAsync(base + off[k], host_in[k], sizes[k], cudaMemcpyHostToDevice, ctx->stream));
+        a.src_xyz = (const float*)(base + off[0]); a.src_nrm = src_nrm ? (const float*)(base + off[1]) : nullptr;
+        a.tgt_xyz = (const float*)(base + off[2]); a.tgt_nrm = tgt_nrm ? (const float*)(base + off[3]) : nullptr;
+        a.src_off = (const long long*)(base + off[4]); a.tgt_off = (const long long*)(base + off[5]); a.poses_in = (const float*)(base + off[6]);
+        a.poses_out = (float*)(base + off[7]); a.n_iter_out = (int*)(base + off[8]); a.status_out = (int*)(base + off[9]);
+        a.history = pose_history ? (float*)(base + off[10]) : nullptr;
+    }
+    if (a.history && hist_floats) CU(cudaMemsetAsync(a.history, 0, hist_floats * 4, ctx->stream));   // rows past a pair's last iteration read 0
+    if (cfg.metric == ICP_GPU_METRIC_SYMMETRIC) {
+        if (ensure(ctx, ctx->batch_scratch, (size_t)(ns > 0 ? ns : 1) * sizeof(int2), false)) return ICP_GPU_E_CUDA;
+        a.scratch = (int2*)ctx->batch_scratch.p;
+    }
+    a.metric = cfg.metric; a.n_iterations = n_it; a.weighting = cfg.weighting; a.rejection = cfg.rejection;
+    a.max_d2 = cfg.max_distance_sq;
+    a.weight_max_d2 = cfg.weight_max_distance_sq > 0.f ? cfg.weight_max_distance_sq : cfg.max_distance_sq;
+    a.proba = cfg.selection == ICP_GPU_SELECT_RANDOM ? (float)cfg.proba : -1.0f;
+    a.seed = cfg.seed;
+    a.stop_rot = cfg.early_stop_rotation; a.stop_trans = cfg.early_stop_translation;
+    CU(icp_launch_batch(a, n_pairs, max_tgt, ctx->stream));
+    if (!dev) {
+        CU(cudaMemcpyAsync(poses_out, a.poses_out, B * 64, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaMemcpyAsync(n_iterations_out, a.n_iter_out, B * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaMemcpyAsync(status_out, a.status_out, B * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        if (pose_history && hist_floats) CU(cudaMemcpyAsync(pose_history, a.history, hist_floats * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    CU(cudaStreamSynchronize(ctx->stream));
+    return ICP_GPU_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int icp_gpu_estimate_pose_batch(icp_gpu_ctx* ctx, int32_t n_pairs, const float* src_xyz, const float* src_nrm, const int64_t* src_off,
+                                const float* tgt_xyz, const float* tgt_nrm, const int64_t* tgt_off, const float* poses_in, float* poses_out,
+                                int32_t* n_iterations_out, int32_t* status_out, float* pose_history) {
+    return estimate_pose_batch(ctx, n_pairs, src_xyz, src_nrm, src_off, tgt_xyz, tgt_nrm, tgt_off, poses_in, poses_out, n_iterations_out,
+                               status_out, pose_history, false);
+}
+
+int icp_gpu_estimate_pose_batch_dev(icp_gpu_ctx* ctx, int32_t n_pairs, const float* src_xyz, const float* src_nrm, const int64_t* src_off,
+                                    const float* tgt_xyz, const float* tgt_nrm, const int64_t* tgt_off, const float* poses_in, float* poses_out,
+                                    int32_t* n_iterations_out, int32_t* status_out, float* pose_history) {
+    return estimate_pose_batch(ctx, n_pairs, src_xyz, src_nrm, src_off, tgt_xyz, tgt_nrm, tgt_off, poses_in, poses_out, n_iterations_out,
+                               status_out, pose_history, true);
 }
 
 }  // extern "C"

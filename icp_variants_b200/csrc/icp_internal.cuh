@@ -200,6 +200,24 @@ struct ReduceArgs {
     PeerXchg peer;           // world > 1: the summed row is all-reduced over the peers' mailboxes before the solve
 };
 
+// batch.cu: B independent small registrations, one thread block per pair running every iteration of its loop
+#define ICP_BATCH_MAX_TARGET ICP_GPU_BATCH_MAX_TARGET    // target points staged in shared memory per pair (float4: 128 KB of the 227 KB a block may use)
+#define ICP_BATCH_THREADS 512
+struct BatchArgs {
+    const float* src_xyz; const float* src_nrm; const long long* src_off;   // packed float[3n]; nrm nullable (= zero normals)
+    const float* tgt_xyz; const float* tgt_nrm; const long long* tgt_off;
+    const float* poses_in;   // [B][16] column-major
+    float* poses_out; int* n_iter_out; int* status_out;
+    float* history;          // [B][n_iterations][16] or null
+    int2* scratch;           // symmetric metric: one {target index or -1, weight bits} per source point, kept between the two passes
+    int metric, n_iterations, weighting, rejection;
+    float max_d2, weight_max_d2;
+    float proba;             // device selection stream: keep a query iff hash < proba; < 0 = select all
+    unsigned int seed;
+    float stop_rot, stop_trans;
+};
+cudaError_t icp_launch_batch(const BatchArgs& a, int n_pairs, int max_tgt, cudaStream_t s);
+
 // standalone.cu: the reference API's value-level operations outside the loop
 cudaError_t icp_launch_transform(const float* in, long long n, const float pose16[16], int normals, float* out, cudaStream_t s);
 cudaError_t icp_launch_apply_weights(int method, float max_d2, const float* sp, const float* sn, const unsigned int* sc, const float* tp, const float* tn,

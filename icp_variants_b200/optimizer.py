@@ -253,6 +253,23 @@ class ICPOptimizer:
                 cm.benchmarkErrors.extend(float(b) for b in bench)
         return pose
 
+    def estimatePoseBatch(self, sources, targets, initialPoses=None):
+        """Many independent small registrations with this optimizer's configuration in one launch (one thread block per pair;
+        targets of at most capi.BATCH_MAX_TARGET points).  Returns the list of estimated poses.  last_error becomes a list with
+        one entry per pair: None, or the message of a pair that stopped without a surviving match or on a singular system
+        (that pair's pose is its last good one, as estimatePose returns it)."""
+        self._ctx.set_config(self.config())
+        poses, n_it, status = self._ctx.estimate_pose_batch(sources, targets, initialPoses)
+        self.last_error = []
+        for s, n in zip(status, n_it):
+            if s == capi.OK:
+                self.last_error.append(None)
+            elif s == capi.E_NO_MATCHES:
+                self.last_error.append(f"iteration {n} had no surviving correspondence")
+            else:
+                self.last_error.append(f"iteration {n}: singular / non-finite normal equations")
+        return list(poses)
+
     def estimateNormals(self, points, k: int = 5, viewpoint=None):
         """PointCloud(pcl cloud) (PointCloud.h:41-76): k-NN PCA normals of a cloud, computed on the device.  The cloud is
         indexed as the target to do so (set the registration's target afterwards if it is another cloud)."""

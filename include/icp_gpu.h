@@ -195,6 +195,30 @@ int icp_gpu_max_iterations(const icp_gpu_ctx* ctx);
 int icp_gpu_estimate_pose_async(icp_gpu_ctx* ctx, const float pose_in[16]);
 int icp_gpu_estimate_pose_finish(icp_gpu_ctx* ctx, float pose_out[16], float* pose_history, int32_t* n_iterations_out);
 
+/* B independent registrations with the context's configuration, one thread block per pair, one launch: for many small
+ * pairs (bunny-sized trials, multi-start registration), where the per-pair index build and launch chain of
+ * icp_gpu_estimate_pose cost more than the work.  Clouds are concatenated; pair b owns source points
+ * [src_off[b], src_off[b+1]) and target points [tgt_off[b], tgt_off[b+1]) (B+1 offsets each, starting at 0, monotone).
+ * Indices are local to the pair (the device selection stream hashes the pair-local source index).  src_nrm / tgt_nrm
+ * nullable (= zero normals); no colours (the colour weighting sees equal colours).  poses_in / poses_out: B x 16 floats;
+ * n_iterations_out[b] = iterations applied; status_out[b] = ICP_GPU_OK / ICP_GPU_E_NO_MATCHES / ICP_GPU_E_NUMERIC per pair,
+ * a failed pair keeping its last good pose (the call itself returns OK once the batch ran).  pose_history (nullable) =
+ * B x n_iterations x 16 floats, rows past a pair's last iteration 0.
+ * Supported: k-NN matching (exact, the brute-force scan's correspondences), the linear minimiser, every metric, weighting
+ * and rejection, select-all or ICP_GPU_RNG_DEVICE random selection, early stop.  Refused with ICP_GPU_E_ARG: LM,
+ * multi-resolution, projective, colour ICP, ICP_GPU_NN_BRUTE_NORM, mt19937 selection, a pair with more than
+ * ICP_GPU_BATCH_MAX_TARGET target points (register it with icp_gpu_estimate_pose), bad offsets.  ICP_GPU_E_STATE while a
+ * registration is pending.  The context's own clouds, index and graphs are left as they are; the call runs on the
+ * context's stream and returns when the batch is done.
+ * _dev: every array (offsets included) is a device pointer on the context's device; the offsets are read back to check them. */
+#define ICP_GPU_BATCH_MAX_TARGET 8192
+int icp_gpu_estimate_pose_batch(icp_gpu_ctx* ctx, int32_t n_pairs, const float* src_xyz, const float* src_nrm, const int64_t* src_off,
+                                const float* tgt_xyz, const float* tgt_nrm, const int64_t* tgt_off, const float* poses_in, float* poses_out,
+                                int32_t* n_iterations_out, int32_t* status_out, float* pose_history);
+int icp_gpu_estimate_pose_batch_dev(icp_gpu_ctx* ctx, int32_t n_pairs, const float* src_xyz, const float* src_nrm, const int64_t* src_off,
+                                    const float* tgt_xyz, const float* tgt_nrm, const int64_t* tgt_off, const float* poses_in, float* poses_out,
+                                    int32_t* n_iterations_out, int32_t* status_out, float* pose_history);
+
 int icp_gpu_get_stats(icp_gpu_ctx* ctx, icp_gpu_stats* out);
 /* The FP32 (non-tensor) roofline denominator of the context's device, measured with a register-resident microbenchmark on
  * the context's stream (SURVEY.md 8d; the reference has no counterpart): mode 0 = FFMA (2 flop / instruction), mode 1 =
