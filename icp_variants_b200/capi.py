@@ -110,6 +110,9 @@ def lib():
             "icp_gpu_estimate_pose_finish": (C.c_int, [vp, pf, pf, C.POINTER(i32)]),
             "icp_gpu_estimate_pose_batch": (C.c_int, [vp, i32, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf]),
             "icp_gpu_estimate_pose_batch_dev": (C.c_int, [vp, i32, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf]),
+            "icp_gpu_iterations_bound": (C.c_int, [C.POINTER(Config), i64]),
+            "icp_gpu_estimate_pose_batch_configs": (C.c_int, [vp, i32, C.POINTER(Config), i32, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, i32]),
+            "icp_gpu_estimate_pose_batch_configs_dev": (C.c_int, [vp, i32, C.POINTER(Config), i32, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, i32]),
             "icp_gpu_get_stats": (C.c_int, [vp, C.POINTER(Stats)]),
             "icp_gpu_measure_fp32_peak": (C.c_int, [vp, i32, C.POINTER(C.c_double)]),
             "icp_gpu_alignment_error": (C.c_int, [vp, pf, pf, C.POINTER(C.c_double)]),
@@ -147,6 +150,25 @@ def default_config() -> Config:
     c = Config()
     lib().icp_gpu_default_config(C.byref(c))
     return c
+
+
+def iterations_bound(cfg: Config, n_source: int) -> int:
+    """The number of iterations estimate_pose runs at most for cfg and a source of n_source points (n_iterations, or
+    max(n_iterations, pyramid levels) with multires)."""
+    rc = int(lib().icp_gpu_iterations_bound(C.byref(cfg), int(n_source)))
+    if rc < 0:
+        raise IcpGpuError(rc, f"iterations_bound: n_source {n_source}")
+    return rc
+
+
+def _config_table(configs, config_index, B):
+    """Sequence of Config -> (ctypes Config array, int32 [B] config_index)."""
+    configs = list(configs)
+    table = (Config * max(len(configs), 1))(*configs)
+    ci = np.ascontiguousarray(config_index, dtype=np.int32)
+    if ci.shape != (B,):
+        raise ValueError(f"config_index: expected [{B}] indices, got {ci.shape}")
+    return table, len(configs), ci
 
 
 def pose_to_c(pose) -> np.ndarray:
@@ -347,6 +369,19 @@ class Context:
         import torch
         dev = torch.device("cuda", self.device)
 
+        def run(sp, sn, so, tp, tn, to, pin, pout, n_it, status, p):
+            hist = torch.empty((len(so) - 1, self.get_config().n_iterations, 4, 4), dtype=torch.float32, device=dev) if want_history else None
+            self._check(lib().icp_gpu_estimate_pose_batch_dev(self._h, len(so) - 1, p(sp), p(sn), p(so), p(tp), p(tn), p(to), p(pin), p(pout), p(n_it),
+                                                              p(status), p(hist)))
+            return hist
+
+        return self._batch_dev(run, src_xyz, src_off, tgt_xyz, tgt_off, src_nrm, tgt_nrm, init_poses)
+
+    def _batch_dev(self, run, src_xyz, src_off, tgt_xyz, tgt_off, src_nrm, tgt_nrm, init_poses):
+        """Checks and lays out the torch operands of the _dev batch forms; run(...) makes the call and returns the history or None."""
+        import torch
+        dev = torch.device("cuda", self.device)
+
         def arr(x, name, cols):
             if x is None:
                 return None
@@ -381,16 +416,64 @@ class Context:
         pout = torch.empty((B, 4, 4), dtype=torch.float32, device=dev)
         n_it = torch.empty(B, dtype=torch.int32, device=dev)
         status = torch.empty(B, dtype=torch.int32, device=dev)
-        hist = torch.empty((B, self.get_config().n_iterations, 4, 4), dtype=torch.float32, device=dev) if want_history else None
 
         def p(x):
             return None if x is None else C.c_void_p(x.data_ptr())
 
         torch.cuda.current_stream(dev).synchronize()
-        self._check(lib().icp_gpu_estimate_pose_batch_dev(self._h, B, p(sp), p(sn), p(so), p(tp), p(tn), p(to), p(pin), p(pout), p(n_it), p(status),
-                                                          p(hist)))
+        hist = run(sp, sn, so, tp, tn, to, pin, pout, n_it, status, p)
         out = (pout.transpose(1, 2).contiguous(), n_it, status)
-        return out + (hist.transpose(2, 3).contiguous(),) if want_history else out
+        return out + (hist.transpose(2, 3).contiguous(),) if hist is not None else out
+
+    def estimate_pose_batch_configs(self, configs, config_index, sources, targets, init_poses=None, want_history=False):
+        """B independent registrations, pair b with configs[config_index[b]] (the context's own configuration is not used).
+        Clouds and poses as estimate_pose_batch.  Returns (poses [B,4,4], n_iterations [B], status [B][, history [B, R, 4, 4]]),
+        R = the largest iterations_bound of the batch's pairs, rows past a pair's last iteration 0."""
+        if len(sources) != len(targets):
+            raise ValueError(f"{len(sources)} sources, {len(targets)} targets")
+        B = len(sources)
+        table, n_cfg, ci = _config_table(configs, config_index, B)
+        sp, sn, so = _concat_clouds(sources)
+        tp, tn, to = _concat_clouds(targets)
+        pin = _batch_poses(init_poses, B)
+        pout = np.zeros((B, 16), np.float32)
+        n_it = np.zeros(B, np.int32)
+        status = np.zeros(B, np.int32)
+        rows = 0
+        if want_history:
+            rows = max([iterations_bound(table[int(k)], so[b + 1] - so[b]) for b, k in enumerate(ci) if 0 <= k < n_cfg] + [0])
+        hist = np.zeros((B, rows, 16), np.float32) if want_history else None
+        self._check(lib().icp_gpu_estimate_pose_batch_configs(self._h, n_cfg, table, B, _ptr(ci), _ptr(sp), _ptr(sn), _ptr(so), _ptr(tp), _ptr(tn),
+                                                              _ptr(to), _ptr(pin), _ptr(pout), _ptr(n_it), _ptr(status), _ptr(hist) if rows else None,
+                                                              rows))
+        out = (pout.reshape(B, 4, 4).transpose(0, 2, 1).copy(), n_it, status)
+        return out + (hist.reshape(B, rows, 4, 4).transpose(0, 1, 3, 2).copy(),) if want_history else out
+
+    def estimate_pose_batch_configs_dev(self, configs, config_index, src_xyz, src_off, tgt_xyz, tgt_off, src_nrm=None, tgt_nrm=None,
+                                        init_poses=None, want_history=False):
+        """The same on CUDA torch tensors of the context's device, shaped as estimate_pose_batch_dev's; config_index: an int32 [B]
+        tensor on the device, configs: a sequence of Config (host).  Returns CUDA tensors (poses [B,4,4], n_iterations [B],
+        status [B][, history [B, R, 4, 4]])."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        B = len(src_off) - 1
+        if not (isinstance(config_index, torch.Tensor) and config_index.device == dev and config_index.dtype == torch.int32
+                and tuple(config_index.shape) == (B,)):
+            raise ValueError(f"config_index: expected an int32 [{B}] tensor on {dev}")
+        table, n_cfg, _ = _config_table(configs, np.zeros(B, np.int32), B)
+        ci = config_index.contiguous()
+        rows = 0
+        if want_history:
+            ns = (src_off[1:] - src_off[:-1]).tolist()
+            rows = max([iterations_bound(table[int(k)], n) for k, n in zip(ci.tolist(), ns) if 0 <= k < n_cfg] + [0])
+
+        def run(sp, sn, so, tp, tn, to, pin, pout, n_it, status, p):
+            hist = torch.zeros((B, rows, 4, 4), dtype=torch.float32, device=dev) if want_history else None
+            self._check(lib().icp_gpu_estimate_pose_batch_configs_dev(self._h, n_cfg, table, B, p(ci), p(sp), p(sn), p(so), p(tp), p(tn), p(to),
+                                                                      p(pin), p(pout), p(n_it), p(status), p(hist) if rows else None, rows))
+            return hist
+
+        return self._batch_dev(run, src_xyz, src_off, tgt_xyz, tgt_off, src_nrm, tgt_nrm, init_poses)
 
     def cloud_from_depth(self, depth, rgbx, K, extrinsics=None, keep_original_size=False, downsample=1, max_distance=0.1,
                          role: int = 2, download: bool = True):

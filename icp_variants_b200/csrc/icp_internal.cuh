@@ -78,6 +78,36 @@ struct IterDesc {
     int pad0, pad1, pad2;
 };
 
+// The multi-resolution schedule of estimatePose (ICPOptimizer.h:503-525, :634-655) for a source of n points: the level strides
+// coarsest, coarsest / 2, ..., 1, one iteration at every stride above 1, the remaining iterations at stride 1.  make_plan,
+// icp_gpu_iterations_bound and the batch kernels all read it from here.
+struct IcpSchedule {
+    int coarsest;   // stride of iteration 0 (a power of two; 1 without multires)
+    int levels;     // log2(coarsest) + 1
+    int n_iters;    // iterations run at most: n_iterations, or max(n_iterations, levels) with multires
+};
+__host__ __device__ inline IcpSchedule icp_schedule(int n_iterations, int multires, long long n) {
+    IcpSchedule s; s.coarsest = 1; s.levels = 1; s.n_iters = n_iterations;
+    if (!multires) return s;
+    float res = 1.0f; int sz = (int)n;                                    // ICPOptimizer.h:503-516
+    for (;;) { sz = (int)(sz / 2.0); if (sz < 100) break; res *= 2.0f; }
+    s.coarsest = (int)res;
+    for (int c = s.coarsest; c > 1; c /= 2) ++s.levels;
+    if (s.levels > s.n_iters) s.n_iters = s.levels;
+    return s;
+}
+// stride and pyramid level (0 = coarsest) of iteration i
+__host__ __device__ inline int icp_schedule_stride(const IcpSchedule& s, int i) { return i < s.levels ? s.coarsest >> i : 1; }
+__host__ __device__ inline int icp_schedule_level(const IcpSchedule& s, int i) { return i < s.levels ? i : s.levels - 1; }
+
+// Levenberg-Marquardt trust-region state of one outer iteration (lm.cuh); lives in DevState (lm.cu) or in a batch block's shared
+// memory (batch.cu)
+struct LmState {
+    double x[6], cand[6], cost, H[36], g[6], scale[6], diag[6];
+    double radius, decrease, model_change;
+    int iter, done, reuse_diag, invalid, step_ok, have_cand;
+};
+
 // Device-resident loop state; one per context.
 struct DevState {
     float pose[16];      // current estimate, column-major
@@ -91,10 +121,7 @@ struct DevState {
     float mean_d[3];
     double mean_s64[3], mean_d64[3];
     unsigned long long n_queries, n_matched, n_evals, n_nodes;
-    // Levenberg-Marquardt state (lm.cu)
-    double lm_x[6], lm_cand[6], lm_cost, lm_H[36], lm_g[6], lm_scale[6], lm_diag[6];
-    double lm_radius, lm_decrease, lm_model_change;
-    int lm_iter, lm_done, lm_reuse_diag, lm_invalid, lm_step_ok, lm_have_cand;
+    LmState lm;          // Levenberg-Marquardt state (lm.cu)
     double shard_partials[ICP_NRED];
     unsigned int xchg_seq;   // peer exchanges completed since the mailboxes were attached (never reset by pose_init)
     int pad_xchg;
@@ -203,20 +230,32 @@ struct ReduceArgs {
 // batch.cu: B independent small registrations, one thread block per pair running every iteration of its loop
 #define ICP_BATCH_MAX_TARGET ICP_GPU_BATCH_MAX_TARGET    // target points staged in shared memory per pair (float4: 128 KB of the 227 KB a block may use)
 #define ICP_BATCH_THREADS 512
+#define ICP_BATCH_LM_THREADS 256                         // batch_lm_kernel: the fp64 jets need up to 255 registers a thread
+// What the batch kernels read of a pair's configuration (one table entry per configuration of the call).
+struct BatchCfg {
+    int n_iterations, multires, weighting, rejection, lm_max_iterations;
+    int mt_mask;             // 1: mt19937 selection, the pair's masks at BatchArgs::mask + mask_off[pair]
+    float max_d2, weight_max_d2;
+    float proba;             // device selection stream: keep a query iff hash < proba; < 0 = off
+    unsigned int seed;
+    float stop_rot, stop_trans;
+};
 struct BatchArgs {
     const float* src_xyz; const float* src_nrm; const long long* src_off;   // packed float[3n]; nrm nullable (= zero normals)
     const float* tgt_xyz; const float* tgt_nrm; const long long* tgt_off;
     const float* poses_in;   // [B][16] column-major
     float* poses_out; int* n_iter_out; int* status_out;
-    float* history;          // [B][n_iterations][16] or null
-    int2* scratch;           // symmetric metric: one {target index or -1, weight bits} per source point, kept between the two passes
-    int metric, n_iterations, weighting, rejection;
-    float max_d2, weight_max_d2;
-    float proba;             // device selection stream: keep a query iff hash < proba; < 0 = select all
-    unsigned int seed;
-    float stop_rot, stop_trans;
+    float* history;          // [B][history_rows][16] or null
+    int history_rows;
+    int2* scratch;           // symmetric metric and LM: one {target index or -1, weight bits} per source point, kept between the passes
+    const BatchCfg* cfgs; const int* cfg_index;   // pair b runs with cfgs[cfg_index[b]]
+    const int* pairs;        // block k of the launch registers pair pairs[k]
+    // mt19937 selection: iteration i's mask of pair b (one bit per pair-local source index) is the ceil(max(n_s, 1) / 32) words at
+    // mask + mask_off[b] + i * that many; pairs with the same masks share one copy
+    const unsigned int* mask; const long long* mask_off;
 };
-cudaError_t icp_launch_batch(const BatchArgs& a, int n_pairs, int max_tgt, cudaStream_t s);
+// metric: ICP_GPU_METRIC_*, lm: the minimiser; pairs: n_pairs block indices in device memory (BatchArgs::pairs)
+cudaError_t icp_launch_batch(const BatchArgs& a, int metric, int lm, int n_pairs, int max_tgt, cudaStream_t s);
 
 // standalone.cu: the reference API's value-level operations outside the loop
 cudaError_t icp_launch_transform(const float* in, long long n, const float pose16[16], int normals, float* out, cudaStream_t s);

@@ -212,7 +212,7 @@ __global__ void pose_init_kernel(DevState* st, const float* pose16, float stop_r
     st->iter = 0; st->iters_done = 0; st->status = 0; st->ticket = 0; st->ticket2 = 0;
     st->n_queries = 0; st->n_matched = 0; st->n_evals = 0; st->n_nodes = 0;
     for (int k = 0; k < 3; ++k) { st->mean_s[k] = 0.f; st->mean_d[k] = 0.f; }
-    st->lm_done = 0; st->lm_iter = 0;
+    st->lm.done = 0; st->lm.iter = 0;
     st->stop_rot = stop_rot; st->stop_trans = stop_trans; st->converged = 0;
 }
 

@@ -45,8 +45,8 @@ def read_experiments(path: str) -> list:
     return out
 
 
-def _optimizer(e: Experiment, device: int, seed: int):
-    opt = (LinearICPOptimizer if e.useLinear else CeresICPOptimizer)(device=device)
+def _optimizer(e: Experiment, device: int, seed: int, ctx=None):
+    opt = (LinearICPOptimizer if e.useLinear else CeresICPOptimizer)(device=device, ctx=ctx)
     opt.seed = seed                                                  # the reference seeds from std::random_device (selection.h:76-79)
     opt.setMetric(e.useMetric)
     opt.setNbOfIterations(e.numIterations)
@@ -59,17 +59,21 @@ def write_rmse(path: str, values):
             f.write(f"{np.float32(v):g}\n")                         # operator<<(float): 6 significant digits
 
 
+def _configure_bunny(opt, e: Experiment):
+    opt.setMatchingMethod(0)
+    opt.setMatchingMaxDistance(e.maxMatchingDist)
+    opt.setSelectionMethod(e.selectionMethod, e.samplingProba)
+    opt.setWeightingMethod(e.weightingMethod)
+    opt.enableMultiResolution(bool(e.useMultiresolution))
+
+
 def run_experiment(e: Experiment, inputs: dict, out_dir: str = ".", device: int = 0, seed: int = 0) -> dict:
     """One row.  Returns {"pose" | "poses", "rmse", "file"}."""
     os.makedirs(out_dir, exist_ok=True)
     opt = _optimizer(e, device, seed)
     if e.expType == "bunny":                                        # experiment.cpp:22-141
         src, tgt, gs, gt = inputs["bunny"]
-        opt.setMatchingMethod(0)
-        opt.setMatchingMaxDistance(e.maxMatchingDist)
-        opt.setSelectionMethod(e.selectionMethod, e.samplingProba)
-        opt.setWeightingMethod(e.weightingMethod)
-        opt.enableMultiResolution(bool(e.useMultiresolution))
+        _configure_bunny(opt, e)
         cm = ConvergenceMeasure(src.points[gs], tgt.points[gt]); tm = TimeMeasure()
         opt.setConvergenceMeasure(cm); opt.setTimeMeasure(tm)
         pose = opt.estimatePose(src, tgt, np.eye(4, dtype=np.float32))
@@ -107,6 +111,40 @@ def run_experiment(e: Experiment, inputs: dict, out_dir: str = ".", device: int 
     raise ValueError(f"unknown experiment type {e.expType!r}")
 
 
-def run_experiments(path: str, inputs: dict, out_dir: str = ".", device: int = 0, seed: int = 0) -> list:
-    """main() of experiment.cpp: every row of the file, in order."""
-    return [run_experiment(e, inputs, out_dir, device, seed) for e in read_experiments(path)]
+def _run_bunny_batch(exps: list, inputs: dict, out_dir: str, device: int, seed: int) -> list:
+    """The "bunny" rows in one batched registration, one configuration per row (Context.estimate_pose_batch_configs); each
+    row's RMSE per iteration is the device ConvergenceMeasure of its pose history."""
+    from . import capi
+    src, tgt, gs, gt = inputs["bunny"]
+    out = []
+    with capi.Context(device) as ctx:
+        configs = []
+        for e in exps:
+            opt = _optimizer(e, device, seed, ctx=ctx)
+            _configure_bunny(opt, e)
+            configs.append(opt.config())
+        B = len(exps)
+        poses, n_it, _, hist = ctx.estimate_pose_batch_configs(configs, np.arange(B, dtype=np.int32), [src] * B, [tgt] * B,
+                                                                    want_history=True)
+        ctx.set_correspondences(src.points[gs], tgt.points[gt])
+        for k, e in enumerate(exps):                             # a pair that stopped early keeps its last good pose, as estimatePose does
+            rmse = [ctx.alignment_error(hist[k, i])[0] for i in range(n_it[k])]
+            path = os.path.join(out_dir, e.expName + "_RMSE.txt")
+            write_rmse(path, rmse)
+            out.append({"pose": poses[k], "rmse": rmse, "file": path})
+    return out
+
+
+def run_experiments(path: str, inputs: dict, out_dir: str = ".", device: int = 0, seed: int = 0, batched: bool = False) -> list:
+    """main() of experiment.cpp: every row of the file, in order.  batched=True: all "bunny" rows of the file run in one batched
+    registration, one configuration per row; the other rows run as with batched=False."""
+    exps = read_experiments(path)
+    if not batched:
+        return [run_experiment(e, inputs, out_dir, device, seed) for e in exps]
+    os.makedirs(out_dir, exist_ok=True)
+    rows = [i for i, e in enumerate(exps) if e.expType == "bunny"]
+    out = [None] * len(exps)
+    if rows:
+        for i, r in zip(rows, _run_bunny_batch([exps[i] for i in rows], inputs, out_dir, device, seed)):
+            out[i] = r
+    return [r if r is not None else run_experiment(e, inputs, out_dir, device, seed) for e, r in zip(exps, out)]

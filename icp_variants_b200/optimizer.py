@@ -254,12 +254,12 @@ class ICPOptimizer:
         return pose
 
     def estimatePoseBatch(self, sources, targets, initialPoses=None):
-        """Many independent small registrations with this optimizer's configuration in one launch (one thread block per pair;
-        targets of at most capi.BATCH_MAX_TARGET points).  Returns the list of estimated poses.  last_error becomes a list with
-        one entry per pair: None, or the message of a pair that stopped without a surviving match or on a singular system
-        (that pair's pose is its last good one, as estimatePose returns it)."""
-        self._ctx.set_config(self.config())
-        poses, n_it, status = self._ctx.estimate_pose_batch(sources, targets, initialPoses)
+        """Many independent small registrations with this optimizer's configuration (one thread block per pair; targets of at
+        most capi.BATCH_MAX_TARGET points): either minimiser, multi-resolution and mt19937 selection included.  Returns the list
+        of estimated poses.  last_error becomes a list with one entry per pair: None, or the message of a pair that stopped
+        without a surviving match or on a singular system (that pair's pose is its last good one, as estimatePose returns it)."""
+        poses, n_it, status = self._ctx.estimate_pose_batch_configs([self.config()], np.zeros(len(sources), np.int32), sources, targets,
+                                                                    initialPoses)
         self.last_error = []
         for s, n in zip(status, n_it):
             if s == capi.OK:

@@ -206,7 +206,8 @@ int icp_gpu_estimate_pose_finish(icp_gpu_ctx* ctx, float pose_out[16], float* po
  * B x n_iterations x 16 floats, rows past a pair's last iteration 0.
  * Supported: k-NN matching (exact, the brute-force scan's correspondences), the linear minimiser, every metric, weighting
  * and rejection, select-all or ICP_GPU_RNG_DEVICE random selection, early stop.  Refused with ICP_GPU_E_ARG: LM,
- * multi-resolution, projective, colour ICP, ICP_GPU_NN_BRUTE_NORM, mt19937 selection, a pair with more than
+ * multi-resolution, projective, colour ICP, ICP_GPU_NN_BRUTE_NORM, mt19937 selection (LM, multi-resolution and mt19937
+ * selection run through icp_gpu_estimate_pose_batch_configs), a pair with more than
  * ICP_GPU_BATCH_MAX_TARGET target points (register it with icp_gpu_estimate_pose), bad offsets.  ICP_GPU_E_STATE while a
  * registration is pending.  The context's own clouds, index and graphs are left as they are; the call runs on the
  * context's stream and returns when the batch is done.
@@ -218,6 +219,37 @@ int icp_gpu_estimate_pose_batch(icp_gpu_ctx* ctx, int32_t n_pairs, const float* 
 int icp_gpu_estimate_pose_batch_dev(icp_gpu_ctx* ctx, int32_t n_pairs, const float* src_xyz, const float* src_nrm, const int64_t* src_off,
                                     const float* tgt_xyz, const float* tgt_nrm, const int64_t* tgt_off, const float* poses_in, float* poses_out,
                                     int32_t* n_iterations_out, int32_t* status_out, float* pose_history);
+
+/* The number of iterations estimate_pose runs at most for configuration cfg and a source of n_source points: n_iterations, or
+ * max(n_iterations, pyramid levels) with multires (ICPOptimizer.h:503-525, :634-655).  A pure function of its arguments, no
+ * context or device needed; ICP_GPU_E_ARG for a null cfg or n_source outside [0, INT32_MAX]. */
+int icp_gpu_iterations_bound(const icp_gpu_config* cfg, int64_t n_source);
+
+/* B registrations with one configuration per pair: pair b runs with configs[config_index[b]] (n_configs >= 1 entries; the
+ * context's own configuration is not used).  Cloud, offset, pose and status layout as icp_gpu_estimate_pose_batch.
+ * pose_history (nullable) = B x history_rows x 16 floats, history_rows >= the largest icp_gpu_iterations_bound of the batch's
+ * pairs; rows past a pair's last iteration 0.  n_iterations_out[b] = iterations applied.
+ * Accepted per configuration: both minimisers (one block per pair either way), every metric and weighting, rejection on or off,
+ * select-all, random selection with mt19937 (reference-compatible, masks drawn on the host and shared by every pair with the
+ * same configuration, source size and, with multires, the same finite points) or with the device stream, the STRIDE
+ * multi-resolution schedule, early stop, lm_max_iterations.  Every field is checked as icp_gpu_set_config checks it.
+ * Refused with ICP_GPU_E_ARG, the message naming the pair or configuration: projective matching, colour ICP,
+ * ICP_GPU_NN_BRUTE_NORM, the VOXEL pyramid, a target above ICP_GPU_BATCH_MAX_TARGET points, a config_index out of range,
+ * n_configs < 1, history_rows below the bound when a history is asked for, bad offsets.
+ * Pairs are grouped by (minimiser, metric); the groups run concurrently, one launch each, and the call returns when all are done.
+ * _dev: every per-pair array (offsets and config_index included) is a device pointer on the context's device; configs stays a
+ * host array.  The offsets and config_index are read back to check them and plan the groups; with multires and mt19937
+ * selection the sources' points and normals are read back too (once per call), for the finite flags the masks depend on. */
+int icp_gpu_estimate_pose_batch_configs(icp_gpu_ctx* ctx, int32_t n_configs, const icp_gpu_config* configs, int32_t n_pairs,
+                                        const int32_t* config_index, const float* src_xyz, const float* src_nrm, const int64_t* src_off,
+                                        const float* tgt_xyz, const float* tgt_nrm, const int64_t* tgt_off, const float* poses_in,
+                                        float* poses_out, int32_t* n_iterations_out, int32_t* status_out, float* pose_history,
+                                        int32_t history_rows);
+int icp_gpu_estimate_pose_batch_configs_dev(icp_gpu_ctx* ctx, int32_t n_configs, const icp_gpu_config* configs, int32_t n_pairs,
+                                            const int32_t* config_index, const float* src_xyz, const float* src_nrm, const int64_t* src_off,
+                                            const float* tgt_xyz, const float* tgt_nrm, const int64_t* tgt_off, const float* poses_in,
+                                            float* poses_out, int32_t* n_iterations_out, int32_t* status_out, float* pose_history,
+                                            int32_t history_rows);
 
 int icp_gpu_get_stats(icp_gpu_ctx* ctx, icp_gpu_stats* out);
 /* The FP32 (non-tensor) roofline denominator of the context's device, measured with a register-resident microbenchmark on
