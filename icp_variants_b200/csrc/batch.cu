@@ -6,7 +6,7 @@
 //
 //   staging   the pair's target points (float4, D1 layout) in dynamic shared memory, once; normals stay in global memory
 //             and are read for the matched point only
-//   selection the query set of iteration `it` exactly as make_plan (api.cu) describes it: the level stride of the multi-resolution
+//   selection the query set of iteration `it` exactly as make_plan (registration.cu) describes it: the level stride of the multi-resolution
 //             schedule with its finite filter, the mt19937 mask drawn on the host, or the device selection stream keyed by the seed
 //             and the iteration; masks and hash are indexed by the pair-local source index
 //   search    one thread per query, every thread scans the staged target in index order: all lanes read the same entry
@@ -92,7 +92,7 @@ __device__ __forceinline__ BatchPair batch_stage(const BatchArgs& a, BatchCfg& c
     return q;
 }
 
-// The query set of iteration `it` (make_plan, api.cu): the level stride and finite filter of the multi-resolution schedule, the
+// The query set of iteration `it` (make_plan, registration.cu): the level stride and finite filter of the multi-resolution schedule, the
 // mt19937 mask or the device selection stream (keyed by the seed and the iteration)
 __device__ __forceinline__ IterDesc batch_iter_desc(const BatchCfg& c, const IcpSchedule& sch, int it, int mask_words) {
     IterDesc d;

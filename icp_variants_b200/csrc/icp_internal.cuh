@@ -201,7 +201,7 @@ struct MatchArgs {
     int group_min;           // knn_group_kernel: fewest handed-over queries among 32 consecutive positions that share one descent
 };
 
-// Concurrency inside one iteration (api.cu, match.cu): the queries are cut into chunks, each chunk's {prep, walk} chain runs on its own
+// Concurrency inside one iteration (registration.cu, match.cu): the queries are cut into chunks, each chunk's {prep, walk} chain runs on its own
 // stream between a fork and a join event; the per-query results do not depend on the cut.
 #define ICP_MAX_MATCH_CHUNKS 8
 struct MatchChunks {
