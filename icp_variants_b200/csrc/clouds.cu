@@ -1,17 +1,12 @@
 // clouds.cu -- the context's clouds: upload, the target's index build (buildIndex) and the source's sort, clouds from depth maps
 // and PCA normals of the target.  Host code only; the kernels live in grid.cu, prep.cu and normals.cu.
 #include "context.cuh"
-#include <stdlib.h>
 
 static int pick_T(int n, bool source = false) {
     // Target: the finest grid the 32-bit keys hold (10 bits per axis) -- the radix sort costs the same for any T, and fine
     // cells give compact leaves.  Source: 4 cells per point; its grid also defines the voxel pyramid levels, which the
     // oracle restates (oracle/icp_oracle.c:orc_pick_T).
-    if (!source) {
-        int T = 3 * ICP_MAX_BITS_PER_AXIS;
-        if (const char* e = getenv("ICP_GPU_TARGET_GRID_BITS")) { const int v = atoi(e); if (v >= 3 && v <= 3 * ICP_MAX_BITS_PER_AXIS) T = v; }   // tuning knob
-        return T;
-    }
+    if (!source) return 3 * ICP_MAX_BITS_PER_AXIS;
     int T = 3;
     while (T < 24 && (1ll << T) < (long long)ICP_SOURCE_CELLS_PER_POINT * (long long)(n > 0 ? n : 1)) ++T;
     if (T > 3 * ICP_MAX_BITS_PER_AXIS) T = 3 * ICP_MAX_BITS_PER_AXIS;
@@ -98,21 +93,21 @@ static int build_grid(icp_gpu_ctx* ctx) {
                              (float4*)ctx->tgt_nrm_sorted.p, (unsigned int*)ctx->tsort.msd.p, &ctx->tsort.keys_sorted, &ctx->tsort.msd_shift,
                              ctx->late_pending[0] ? &ctx->late[0] : nullptr, ctx->stream, &launches));
     if (ctx->late_pending[0]) { CU(cudaEventRecord(ctx->ev_packed[0], ctx->stream)); ctx->packed_once[0] = true; ctx->late_pending[0] = false; }
-    cudaStream_t ts = getenv("ICP_GPU_NO_AUX_STREAM") ? ctx->stream : ctx->aux_stream;       // tuning knob (A/B measurement)
-    if (ts != ctx->stream) { CU(cudaEventRecord(ctx->ev_fork, ctx->stream)); CU(cudaStreamWaitEvent(ts, ctx->ev_fork, 0)); }
+    cudaStream_t ts = ctx->aux_stream;
+    CU(cudaEventRecord(ctx->ev_fork, ctx->stream)); CU(cudaStreamWaitEvent(ts, ctx->ev_fork, 0));
     CU(icp_launch_bvh_build((float4*)ctx->tgt_pts_sorted.p, (float4*)ctx->tgt_nrm_sorted.p, n, ctx->T, ctx->tsort.keys_sorted,
                             (const unsigned int*)ctx->bbox.p + 7, (unsigned char*)ctx->lv_flags.p, (unsigned int*)ctx->lv_tiles.p, (int*)ctx->delta_a.p,
                             (int*)ctx->delta_b.p, (unsigned int*)ctx->leaf_rank.p, (unsigned int*)ctx->leaf_start.p, (unsigned int*)ctx->node_rank.p,
                             (unsigned int*)ctx->child_start.p, (BvhDesc*)ctx->bvh_desc.p, (float4*)ctx->bvh_box.p, ctx->n_sms, ts, &launches));
-    const bool bottom_up = !getenv("ICP_GPU_ADJ_FROM_ROOT");                                  // tuning knob (A/B measurement)
     CU(icp_launch_leaf_adjacency((const BvhDesc*)ctx->bvh_desc.p, (const float4*)ctx->bvh_box.p, (const unsigned int*)ctx->child_start.p,
-                                 (unsigned int*)ctx->adj1.p, (float4*)ctx->adj1_box.p, ctx->adj1_capacity, 1, nullptr, nullptr, nullptr, 0, ctx->n_sms, ts, &launches));
+                                 (unsigned int*)ctx->adj1.p, (float4*)ctx->adj1_box.p, ctx->adj1_capacity, 1, nullptr, nullptr, nullptr, 0, ctx->n_sms, ts, &launches,
+                                 nullptr));
     CU(icp_launch_leaf_adjacency((const BvhDesc*)ctx->bvh_desc.p, (const float4*)ctx->bvh_box.p, (const unsigned int*)ctx->child_start.p,
                                  (unsigned int*)ctx->adj.p, (float4*)ctx->adj_box.p, ctx->adj_capacity, 0, (const unsigned int*)ctx->node_rank.p,
-                                 bottom_up ? (const unsigned int*)ctx->adj1.p : nullptr, (const float4*)ctx->adj1_box.p, ctx->adj1_capacity, ctx->n_sms, ts, &launches,
+                                 (const unsigned int*)ctx->adj1.p, (const float4*)ctx->adj1_box.p, ctx->adj1_capacity, ctx->n_sms, ts, &launches,
                                  (float*)ctx->adj_gap.p));
     CU(cudaEventRecord(ctx->ev[1], ts));
-    if (ts != ctx->stream) { CU(cudaEventRecord(ctx->ev_index_ready, ts)); ctx->index_pending = true; }
+    CU(cudaEventRecord(ctx->ev_index_ready, ts)); ctx->index_pending = true;
     ctx->stats.n_kernel_launches += (uint64_t)launches;
     ctx->grid_built = true;
     return 0;

@@ -16,7 +16,6 @@
 // two adjacency kernels.
 #include "icp_internal.cuh"
 #include <string.h>
-#include <stdlib.h>
 
 // ---------------------------------------------------------------------------- pack AoS3 -> float4, bounding box
 __device__ __forceinline__ unsigned int enc_f(float f) { unsigned int b = __float_as_uint(f); return (b & 0x80000000u) ? ~b : (b | 0x80000000u); }
@@ -886,8 +885,9 @@ cudaError_t icp_launch_voxel_level(const float4* pts_sorted, const float4* nrm_s
 
 // ---------------------------------------------------------------------------- leaf adjacency
 // One warp per leaf l: all other leaves whose box meets box(l) inflated by R, found by a box query on the BVH
-// (lane = child).  R starts at twice the leaf's largest extent and is halved until the list fits in 32 entries.
+// (lane = child).  R starts at ADJ_R_FACTOR times the leaf's largest extent and is halved until the list fits in 32 entries.
 #define ADJ_WARPS 4
+#define ADJ_R_FACTOR 2.0f      // 1.5 / 3 / 4 measured no different (round 2, DESIGN §4)
 __device__ __forceinline__ bool boxes_meet(const float* lo, const float* hi, const float4 blo, const float4 bhi) {
     return blo.x <= hi[0] && bhi.x >= lo[0] && blo.y <= hi[1] && bhi.y >= lo[1] && blo.z <= hi[2] && bhi.z >= lo[2];
 }
@@ -895,7 +895,7 @@ __device__ __forceinline__ bool boxes_meet(const float* lo, const float* hi, con
 __global__ void __launch_bounds__(ADJ_WARPS * 32) leaf_adjacency_kernel(const BvhDesc* __restrict__ bvh, const float4* __restrict__ box,
                                                                          const unsigned int* __restrict__ child_start,
                                                                          unsigned int* __restrict__ adj, float4* __restrict__ adj_box,
-                                                                         int capacity, float r_factor, int lv,
+                                                                         int capacity, int lv,
                                                                          const unsigned int* __restrict__ node_rank, const unsigned int* __restrict__ adj1,
                                                                          const float4* __restrict__ adj1_box, int adj1_capacity, float* __restrict__ adj_gap) {
     __shared__ unsigned int s_node[ADJ_WARPS][32 * ICP_BVH_MAX_LEVELS];
@@ -912,7 +912,7 @@ __global__ void __launch_bounds__(ADJ_WARPS * 32) leaf_adjacency_kernel(const Bv
     const unsigned int lt = (1u << lane) - 1u;
     for (int l = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; l < n_leaves; l += warps) {
         const float4 mlo = box[2 * (size_t)(b.offset[lv] + l)], mhi = box[2 * (size_t)(b.offset[lv] + l) + 1];
-        float R = r_factor * fmaxf(fmaxf(mhi.x - mlo.x, mhi.y - mlo.y), mhi.z - mlo.z);
+        float R = ADJ_R_FACTOR * fmaxf(fmaxf(mhi.x - mlo.x, mhi.y - mlo.y), mhi.z - mlo.z);
         int count = 0; bool ok = false;
         // Leaves (lv = 0) with the level-1 lists already built: while the leaf's inflated box lies inside the inflated box of its
         // level-1 node m, every leaf that meets it is a child of a node of m's list -- two rounds of box tests (the <= 32 nodes
@@ -1028,16 +1028,14 @@ __global__ void __launch_bounds__(ADJ_WARPS * 32) leaf_adjacency_kernel(const Bv
     }
 }
 
-// level 1 first; the level-0 call then takes the level-1 lists (node_rank, adj1, adj1_box; nullable = walk from the root)
+// level 1 first; the level-0 call then takes the level-1 lists (node_rank, adj1, adj1_box)
 cudaError_t icp_launch_leaf_adjacency(const BvhDesc* bvh_dev, const float4* box, const unsigned int* child_start, unsigned int* adj,
                                       float4* adj_box, int capacity, int level, const unsigned int* node_rank, const unsigned int* adj1,
                                       const float4* adj1_box, int adj1_capacity, int n_sms, cudaStream_t s, int* n_launches, float* adj_gap) {
     long long nb = ((long long)capacity + ADJ_WARPS - 1) / ADJ_WARPS;
     if (nb > 16ll * n_sms) nb = 16ll * n_sms;
     if (nb < 1) nb = 1;
-    float r_factor = 2.0f;
-    if (const char* e = getenv("ICP_GPU_ADJ_FACTOR")) r_factor = (float)atof(e);   // tuning knob
-    leaf_adjacency_kernel<<<(int)nb, ADJ_WARPS * 32, 0, s>>>(bvh_dev, box, child_start, adj, adj_box, capacity, r_factor, level,
+    leaf_adjacency_kernel<<<(int)nb, ADJ_WARPS * 32, 0, s>>>(bvh_dev, box, child_start, adj, adj_box, capacity, level,
                                                              node_rank, adj1, adj1_box, adj1_capacity, adj_gap);
     if (n_launches) *n_launches += 1;
     return cudaGetLastError();

@@ -30,6 +30,12 @@ __device__ __forceinline__ float padd(float a, float b) { return __fadd_rn(a, b)
 __device__ __forceinline__ float psub(float a, float b) { return __fsub_rn(a, b); }
 __device__ __forceinline__ float pdiv(float a, float b) { return __fdiv_rn(a, b); }
 __device__ __forceinline__ bool finite3(float x, float y, float z) { return isfinite(x) && isfinite(y) && isfinite(z); }
+// The ball of radius r around (x, y, z) lies inside the box [lo, hi].  The ball's bounds are rounded outwards by the explicit _rd / _ru
+// operations, so the answer does not depend on FMA contraction (-fmad) and holds for the exact ball.
+__device__ __forceinline__ bool ball_inside(float x, float y, float z, float r, const float4 lo, const float4 hi) {
+    return __fsub_rd(x, r) >= lo.x && __fadd_ru(x, r) <= hi.x && __fsub_rd(y, r) >= lo.y &&
+           __fadd_ru(y, r) <= hi.y && __fsub_rd(z, r) >= lo.z && __fadd_ru(z, r) <= hi.z;
+}
 
 // Implicit binary tree over a dense table of 2^T Morton-ordered cells (see grid.cu).
 struct GridParams {
@@ -171,7 +177,7 @@ struct MatchArgs {
     // adj_box[2*l] = {lo - R, n as int bits}, adj_box[2*l+1] = {hi + R, _}; an inverted box (lo > hi) means "no list".
     // A query whose search ball lies inside the inflated box needs no tree walk.
     const unsigned int* adj; const float4* adj_box; int adj_capacity;
-    const float* adj_gap;    // squared box-to-box gap of every list entry to its leaf, ascending along the list (rounded down)
+    const float* adj_gap;    // squared box-to-box gap of every list entry to its leaf, ascending along the list (rounded down); never null
     // the same one level up: adj1[32*m ..] = the level-1 nodes (m itself included) whose box meets box(m) inflated; node_rank
     // maps a leaf to its level-1 node (node_rank[coffset[1] + leaf + 1] - 1)
     const unsigned int* adj1; const float4* adj1_box; int adj1_capacity; const unsigned int* node_rank;
@@ -191,10 +197,8 @@ struct MatchArgs {
                              // scan the fast path already made (w = -2: not scanned, the walk starts from nn_pos itself)
     float4* qbuf;            // transformed query points of the current iteration {x,y,z,rgba}; x = NaN: not searched
     int desc_index;          // >= 0: fixed descriptor (query_matches); -1: use state->iter
-    int use_seed;
     int brute_norm;          // brute force on rounded Euclidean norms, max_d2 = a plain distance (NearestNeighborSearchBruteForce, NearestNeighbor.h:81-97)
-    int proj_tiled;          // projective matching of a full-frame source: src arrays are in ORIGINAL (pixel) order, one 32x8 tile per block
-    int fast_path;           // knn_prep_kernel answers the queries whose search ball stays inside their seed leaf's inflated box
+    int proj_tiled;          // projective matching of a full-frame source: src arrays are in ORIGINAL (pixel) order, one 32x4 tile per block
     int collect_stats;       // work counters in DevState (atomics); off in timed runs
     int skip_finish;         // BVH path: the reduction evaluates stages 3-4 itself (ReduceArgs::fused), no match records
     int q_begin, q_end;      // BVH path: the sorted-source positions [q_begin, q_end) this launch searches (a chunk; the whole cloud by default)
@@ -291,12 +295,12 @@ cudaError_t icp_launch_bvh_build(float4* pts_sorted, float4* nrm_sorted, int n, 
 // One voxel pyramid level (depth D of the source grid) as a selection mask; table: scratch of 2^D entries.
 cudaError_t icp_launch_voxel_level(const float4* pts_sorted, const float4* nrm_sorted, int n, const GridParams* grid, int T, int D,
                                    unsigned int* table, unsigned int* mask, size_t mask_words, cudaStream_t s, int* n_launches);
-// Adjacency lists of the nodes [0, min(count[level], capacity)) of `level` (0 leaves, 1 their parents).  The level-0 call can take
-// the level-1 lists (node_rank, adj1, adj1_box; nullable = every query walks from the root).
+// Adjacency lists of the nodes [0, min(count[level], capacity)) of `level` (0 leaves, 1 their parents).  The level-0 call takes the
+// level-1 lists (node_rank, adj1, adj1_box); the level-1 call passes null there.  adj_gap (non-null: the level-0 call): sort the
+// entries by their gap to the node and store the gaps.
 cudaError_t icp_launch_leaf_adjacency(const BvhDesc* bvh_dev, const float4* box, const unsigned int* child_start, unsigned int* adj,
                                       float4* adj_box, int capacity, int level, const unsigned int* node_rank, const unsigned int* adj1,
-                                      const float4* adj1_box, int adj1_capacity, int n_sms, cudaStream_t s, int* n_launches,
-                                      float* adj_gap = nullptr);   // adj_gap: sort the entries by their gap to the node and store the gaps
+                                      const float4* adj1_box, int adj1_capacity, int n_sms, cudaStream_t s, int* n_launches, float* adj_gap);
 cudaError_t icp_launch_extract_order(const float4* pts_sorted, int n, int* order, cudaStream_t s);
 cudaError_t icp_launch_fill_int(int* p, int n, int v, cudaStream_t s);
 // Seeds (nn_pos / nn_leaf) for the queries that have none (reset: for every query), from the target's sorted keys at the pose in `st`.

@@ -27,7 +27,7 @@
 //                     leaves its own ball meets.  What it finishes the walk skips; what outgrows its stage it leaves to the walk.
 //   knn_brute_kernel  small targets: one warp per query over the whole target, warp-shuffle arg-min.
 //   projective_kernel one thread per query over its 25 x 25 pixel window, staged in shared memory per block
-//                     (32 x 8 pixel tiles of a full-frame source, else 256 Morton-consecutive points).
+//                     (32 x 4 pixel tiles of a full-frame source, else 64 or 256 Morton-consecutive points).
 #include "icp_internal.cuh"
 #include <limits.h>
 
@@ -169,9 +169,7 @@ extern "C" int icp_gpu_debug_timeline(unsigned long long* out, int reset) {
 #endif
 
 // ---------------------------------------------------------------------------- BVH search, one warp per query
-#ifndef BVH_WARPS
 #define BVH_WARPS 4
-#endif
 #define BVH_STACK (32 * ICP_BVH_MAX_LEVELS)   // <= 32 pushed children per level
 
 // fp32 lower bound (under D1's rounding and association, by monotonicity) of the squared distance from q
@@ -286,12 +284,8 @@ __device__ __forceinline__ void thread_scan_leaf(const MatchArgs& a, const Query
 // itself -- same candidates, same (d, idx) order, hence the same answer as the walk -- and marks the query as done
 // (qbuf.x = NaN).  The 32 queries of a warp are spatial neighbours (sorted source), so their leaves coincide and the
 // loads are mostly broadcasts.  Everything else (no neighbour yet, ball leaving the box) is left to knn_bvh_kernel.
-#ifndef PREP_THREADS
 #define PREP_THREADS 256
-#endif
-#ifndef PREP_MIN_BLOCKS
 #define PREP_MIN_BLOCKS 5          // measured 5 / 6 / 7 / 8 blocks per SM: 60 / 67 / 78 / 79 us per launch (more blocks = spills)
-#endif
 template <bool COLOR, bool STATS>
 __global__ void __launch_bounds__(PREP_THREADS, PREP_MIN_BLOCKS * 256 / PREP_THREADS) knn_prep_kernel(const MatchArgs a) {
     __shared__ PoseSm sm;
@@ -318,8 +312,7 @@ __global__ void __launch_bounds__(PREP_THREADS, PREP_MIN_BLOCKS * 256 / PREP_THR
             xform_point(sm.P, p4.x, p4.y, p4.z, x, y, z);
             if (finite3(x, y, z)) {
                 o.x = x; o.y = y; o.z = z;
-                const int sp = (a.fast_path && a.use_seed) ? sp_raw : -1;
-                const int seed_leaf = (sp >= 0 && sp < a.n_tgt) ? leaf_raw : -1;
+                const int seed_leaf = (sp_raw >= 0 && sp_raw < a.n_tgt) ? leaf_raw : -1;
                 if (seed_leaf >= 0 && seed_leaf < a.adj_capacity) {
                     Query q; q.x = x; q.y = y; q.z = z;
                     const unsigned int s_rgba = __float_as_uint(n4.w);
@@ -332,9 +325,7 @@ __global__ void __launch_bounds__(PREP_THREADS, PREP_MIN_BLOCKS * 256 / PREP_THR
                     if (b.d < FLT_BIG) {
                         const float r = __fmul_ru(__fsqrt_ru(b.d), 1.00001f);
                         const float4 ilo = __ldg(&a.adj_box[2 * (size_t)seed_leaf]), ihi = __ldg(&a.adj_box[2 * (size_t)seed_leaf + 1]);
-                        const bool inside = __fsub_rd(x, r) >= ilo.x && __fadd_ru(x, r) <= ihi.x && __fsub_rd(y, r) >= ilo.y &&
-                                            __fadd_ru(y, r) <= ihi.y && __fsub_rd(z, r) >= ilo.z && __fadd_ru(z, r) <= ihi.z;
-                        if (inside) {                                           // never true for the inverted "no list" box
+                        if (ball_inside(x, y, z, r, ilo, ihi)) {                // never true for the inverted "no list" box
                             const int na = __float_as_int(ilo.w);
                             const unsigned int* list = a.adj + (size_t)seed_leaf * 32;
                             // two phases, so that the lanes of a warp scan their leaves side by side instead of one
@@ -343,10 +334,10 @@ __global__ void __launch_bounds__(PREP_THREADS, PREP_MIN_BLOCKS * 256 / PREP_THR
                             // the list is in the order of the entries' gaps to the seed leaf's box: with the best candidate inside that
                             // box, an entry whose gap exceeds twice the search radius (4 x in squares, rounded up) cannot hold a nearer
                             // point, nor can any entry after it
-                            const float* gap = a.adj_gap ? a.adj_gap + (size_t)seed_leaf * 32 : nullptr;
-                            const float lim = (gap && bleaf == seed_leaf) ? __fmul_ru(__fmul_ru(4.0f, b.d), 1.00001f) : FLT_BIG;
+                            const float* gap = a.adj_gap + (size_t)seed_leaf * 32;
+                            const float lim = bleaf == seed_leaf ? __fmul_ru(__fmul_ru(4.0f, b.d), 1.00001f) : FLT_BIG;
                             for (int j = 0; j < na; ++j) {
-                                if (gap && __ldg(&gap[j]) > lim) break;
+                                if (__ldg(&gap[j]) > lim) break;
                                 const unsigned int leaf = __ldg(&list[j]);
                                 const float clb = box_dist2c<COLOR>(q, __ldg(&a.bvh_box[2 * (size_t)leaf]), __ldg(&a.bvh_box[2 * (size_t)leaf + 1]));
                                 if (!(clb > b.d)) todo |= 1u << j;
@@ -367,8 +358,7 @@ __global__ void __launch_bounds__(PREP_THREADS, PREP_MIN_BLOCKS * 256 / PREP_THR
                             const int m = (int)(__ldg(&a.node_rank[a.bvh->coffset[1] + seed_leaf + 1]) - 1u);
                             if (m < a.adj1_capacity) {
                                 const float4 jlo = __ldg(&a.adj1_box[2 * (size_t)m]), jhi = __ldg(&a.adj1_box[2 * (size_t)m + 1]);
-                                if (__fsub_rd(x, r) >= jlo.x && __fadd_ru(x, r) <= jhi.x && __fsub_rd(y, r) >= jlo.y &&
-                                    __fadd_ru(y, r) <= jhi.y && __fsub_rd(z, r) >= jlo.z && __fadd_ru(z, r) <= jhi.z) seed.w = __int_as_float(m);
+                                if (ball_inside(x, y, z, r, jlo, jhi)) seed.w = __int_as_float(m);
                             }
                         }
                     }
@@ -397,24 +387,13 @@ __global__ void __launch_bounds__(PREP_THREADS, PREP_MIN_BLOCKS * 256 / PREP_THR
 // same (d, idx) rule, hence the same answer as the walk.  A group whose frontier or list outgrows its stage (a run
 // that jumps across the scene, a member without a neighbour inside the threshold) is left to the walk untouched.  A finished query
 // is marked like one the fast path finished (qbuf.x = NaN), so the walk skips it.
-#ifndef GROUP_CAP
 #define GROUP_CAP 48           // candidate leaves per group   (the kernel ends with its longest group: 128 / 128 / unlimited measured
-#endif                         //                               4.39 -> 5.3 ms on the bench pair against 4.25 with 48 / 64 / 160)
-#ifndef GROUP_FRONT
+                               //                               4.39 -> 5.3 ms on the bench pair against 4.25 with 48 / 64 / 160)
 #define GROUP_FRONT 64         // frontier nodes per level
-#endif
-#ifndef GROUP_WARPS
 #define GROUP_WARPS 4
-#endif
-#ifndef GROUP_UNROLL
 #define GROUP_UNROLL 3
-#endif
-#ifndef GROUP_STEP_LIMIT
 #define GROUP_STEP_LIMIT 160   // (member, leaf) scans per group
-#endif
-#ifndef GROUP_SIZE
 #define GROUP_SIZE 32          // consecutive positions per group (the members sit in the warp's first GROUP_SIZE lanes)
-#endif
 static_assert(GROUP_CAP <= GROUP_FRONT, "pass A keeps the want masks of the listed leaves in cfirst[]");
 struct GroupStage {
     unsigned int front[2][GROUP_FRONT];                       // frontier of the level being expanded / of the next level
@@ -681,9 +660,24 @@ __global__ void __launch_bounds__(GROUP_WARPS * 32, 6) knn_group_kernel(const Ma
     }
 }
 
-#ifndef WALK_MIN_BLOCKS
 #define WALK_MIN_BLOCKS 16         // 32 registers: all 64 warp slots of an SM (the walk is latency-bound: 11 / 8 / 5 resident blocks
-#endif                             // measured 150 / 196 / 241 us per launch against 118 at 16)
+                                   // measured 150 / 196 / 241 us per launch against 118 at 16)
+#define WALK_GRID_PER_SM 64        // blocks of 4 warps per SM in the walk's grid: 128 / 192 / 256 measured 4.65 / 4.88 / 4.86 ms per
+                                   // registration against 4.53 (DESIGN §4)
+
+// The warp scans one leaf, lane = point; every lane keeps its own best.
+template <bool COLOR>
+__device__ __forceinline__ void warp_scan_leaf(const MatchArgs& a, const Query& q, Best& b, unsigned int leaf, int lane, unsigned int& ev) {
+    const unsigned int i = __ldg(&a.leaf_start[leaf]) + lane;
+    if (i < __ldg(&a.leaf_start[leaf + 1])) {
+        const float4 c = __ldg(&a.tgt_pts[i]);
+        const float dd = dist2<COLOR>(q, c, b.d, a.tgt_nrm, i);
+        const int idx = __float_as_int(c.w);
+        if (better_key(dd, idx, b)) { b.d = dd; b.idx = idx; b.pos = (int)i; }
+        ++ev;
+    }
+}
+
 template <bool COLOR, bool STATS>
 __global__ void __launch_bounds__(BVH_WARPS * 32, WALK_MIN_BLOCKS) knn_bvh_kernel(const MatchArgs a) {
     __shared__ unsigned int s_node[BVH_WARPS][BVH_STACK];
@@ -730,61 +724,24 @@ __global__ void __launch_bounds__(BVH_WARPS * 32, WALK_MIN_BLOCKS) knn_bvh_kerne
         if (handed) {
             if (lane == 0) { b.d = sb.x; b.idx = __float_as_int(sb.y); b.pos = __float_as_int(sb.z); }
         } else {
-            const int sp = a.use_seed ? a.nn_pos[p] : -1;
+            // not handed over: no seed, or a seed leaf beyond the adjacency lists' capacity
+            const int sp = a.nn_pos[p];
             if (sp >= 0 && sp < a.n_tgt) {
                 seed_leaf = a.nn_leaf[p];
-                const unsigned int i = __ldg(&a.leaf_start[seed_leaf]) + lane;
-                if (i < __ldg(&a.leaf_start[seed_leaf + 1])) {
-                    const float4 c = __ldg(&a.tgt_pts[i]);
-                    const float dd = dist2<COLOR>(q, c, b.d, a.tgt_nrm, i);
-                    const int idx = __float_as_int(c.w);
-                    if (better_key(dd, idx, b)) { b.d = dd; b.idx = idx; b.pos = (int)i; }
-                    ++ev;
-                }
+                warp_scan_leaf<COLOR>(a, q, b, (unsigned int)seed_leaf, lane, ev);
                 if (lane == 0) ++nd;
             }
         }
         bool done = false;
-        if (!handed && seed_leaf >= 0 && seed_leaf < a.adj_capacity) {
-            // Shortcut without the tree: if the search ball lies inside the seed leaf's inflated box, every leaf that
-            // meets the ball is in that leaf's adjacency list (built with the same inflated box, grid.cu).
-            float bnd = __uint_as_float(__reduce_min_sync(FULL, __float_as_uint(b.d)));
-            if (bnd < FLT_BIG) {
-                const float r = __fmul_ru(__fsqrt_ru(bnd), 1.00001f);
-                const float4 ilo = __ldg(&a.adj_box[2 * (size_t)seed_leaf]), ihi = __ldg(&a.adj_box[2 * (size_t)seed_leaf + 1]);
-                const bool inside = __fsub_rd(q.x, r) >= ilo.x && __fadd_ru(q.x, r) <= ihi.x && __fsub_rd(q.y, r) >= ilo.y &&
-                                    __fadd_ru(q.y, r) <= ihi.y && __fsub_rd(q.z, r) >= ilo.z && __fadd_ru(q.z, r) <= ihi.z;
-                if (inside) {                                                   // never true for the inverted "no list" box
-                    const int na = __float_as_int(ilo.w);
-                    unsigned int ls = 0u, le = 0u; float clb = FLT_BIG; bool keep = false;
-                    if (lane < na) {
-                        const unsigned int leaf = __ldg(&a.adj[(size_t)seed_leaf * 32 + lane]);
-                        const float4 lo = __ldg(&a.bvh_box[2 * (size_t)leaf]), hi = __ldg(&a.bvh_box[2 * (size_t)leaf + 1]);
-                        ls = __ldg(&a.leaf_start[leaf]); le = __ldg(&a.leaf_start[leaf + 1]);
-                        clb = box_dist2c<COLOR>(q, lo, hi);
-                        keep = !(clb > bnd);
-                    }
-                    if (lane == 0) ++nd;
-                    bvh_scan_leaves<COLOR>(a, q, b, bnd, ls, le, clb, keep, lane, ev, nd);
-                    done = true;
-                }
-            }
-        }
-        if (!done && (handed ? __float_as_int(sb.w) >= 0 : seed_leaf >= 0) && top_level >= 1 && a.adj1_capacity > 0) {
-            // The same shortcut one level up: the ball inside the inflated box of the seed leaf's level-1 node => every
-            // level-1 node that meets the ball is in that node's list; their leaves are tested 32 at a time.
+        if ((handed ? __float_as_int(sb.w) >= 0 : seed_leaf >= 0) && bvh.n_levels >= 2 && a.adj1_capacity > 0) {
+            // Shortcut without the whole tree: the ball inside the inflated box of the seed leaf's level-1 node => every level-1
+            // node that meets the ball is in that node's list (grid.cu); their leaves are tested 32 at a time.  For a query handed
+            // over with a node (sb.w = m) the fast path made the containment test.
             const int m = handed ? __float_as_int(sb.w) : (int)(__ldg(&a.node_rank[bvh.coffset[1] + seed_leaf + 1]) - 1u);
             float bnd = __uint_as_float(__reduce_min_sync(FULL, __float_as_uint(b.d)));
             if (m < a.adj1_capacity && bnd < FLT_BIG) {
                 const float4 ilo = __ldg(&a.adj1_box[2 * (size_t)m]);
-                bool inside = true;                                             // handed over: tested by the fast path
-                if (!handed) {
-                    const float r = __fmul_ru(__fsqrt_ru(bnd), 1.00001f);
-                    const float4 ihi = __ldg(&a.adj1_box[2 * (size_t)m + 1]);
-                    inside = __fsub_rd(q.x, r) >= ilo.x && __fadd_ru(q.x, r) <= ihi.x && __fsub_rd(q.y, r) >= ilo.y &&
-                             __fadd_ru(q.y, r) <= ihi.y && __fsub_rd(q.z, r) >= ilo.z && __fadd_ru(q.z, r) <= ihi.z;
-                }
-                if (inside) {
+                if (handed || ball_inside(q.x, q.y, q.z, __fmul_ru(__fsqrt_ru(bnd), 1.00001f), ilo, __ldg(&a.adj1_box[2 * (size_t)m + 1]))) {
                     const int na = __float_as_int(ilo.w);
                     unsigned int node = 0; unsigned int key = 0xFFFFFFFFu;
                     unsigned int cfirst = 0u, clast = 0u;                        // the node's children, loaded with the boxes (not after the pick)
@@ -809,7 +766,7 @@ __global__ void __launch_bounds__(BVH_WARPS * 32, WALK_MIN_BLOCKS) knn_bvh_kerne
                 }
             }
         }
-        if (!done && !__any_sync(FULL, b.pos >= 0) && top_level > 0) {
+        if (!done && !__any_sync(FULL, b.pos >= 0) && bvh.n_levels > 1) {
             // No neighbour remembered (first iteration): follow the nearest node down to one leaf and take its best
             // point as the starting bound, so that the walk below prunes from its first step on.
             int L = top_level; unsigned int first = 0, last = n_top;
@@ -830,14 +787,7 @@ __global__ void __launch_bounds__(BVH_WARPS * 32, WALK_MIN_BLOCKS) knn_bvh_kerne
                 first = __ldg(&a.child_start[bvh.coffset[L] + best_node]); last = __ldg(&a.child_start[bvh.coffset[L] + best_node + 1]);
                 --L;
             }
-            const unsigned int i = __ldg(&a.leaf_start[best_node]) + lane;
-            if (i < __ldg(&a.leaf_start[best_node + 1])) {
-                const float4 c = __ldg(&a.tgt_pts[i]);
-                const float dd = dist2<COLOR>(q, c, b.d, a.tgt_nrm, i);
-                const int idx = __float_as_int(c.w);
-                if (better_key(dd, idx, b)) { b.d = dd; b.idx = idx; b.pos = (int)i; }
-                ++ev;
-            }
+            warp_scan_leaf<COLOR>(a, q, b, best_node, lane, ev);
         }
         float bound = __uint_as_float(__reduce_min_sync(FULL, __float_as_uint(b.d)));
         int top = 0;
@@ -1063,8 +1013,7 @@ cudaError_t icp_launch_match(const MatchArgs& a, int algorithm, int n_sms, cudaS
     const int T = ICP_MATCH_THREADS;
     int launches = 0;
     if (algorithm == 2) {
-        static const bool no_small = getenv("ICP_GPU_NO_SMALL_PROJ_BLOCKS") != nullptr;                // tuning knob (A/B measurement)
-        if (!a.proj_tiled && a.n_src < 2 * 256 * n_sms && !no_small) {
+        if (!a.proj_tiled && a.n_src < 2 * 256 * n_sms) {
             projective_kernel<64, PROJ_TILE_MAX, 5><<<(unsigned int)((a.n_src + 63) / 64), 64, 0, s>>>(a);
         } else if (a.proj_tiled) {
             // full frames: 32 x 4 pixel tiles, 2400 blocks of 128 threads at 640 x 480 over 148 x 6 slots -- with 32 x 8 tiles the 1200
@@ -1091,7 +1040,6 @@ cudaError_t icp_launch_match(const MatchArgs& a, int algorithm, int n_sms, cudaS
         long long per = ((long long)a.n_src + K - 1) / K;
         per = (per + 255) / 256 * 256;                                         // whole prep blocks
         if (K > 1) cudaEventRecord(chunks->fork, s);
-        static const int mult = getenv("ICP_GPU_WALK_GRID") ? atoi(getenv("ICP_GPU_WALK_GRID")) : 64;     // tuning knob
         for (int c = 0; c < K; ++c) {
             MatchArgs ac = a;
             ac.q_begin = (int)std::min<long long>((long long)c * per, a.n_src);
@@ -1110,9 +1058,9 @@ cudaError_t icp_launch_match(const MatchArgs& a, int algorithm, int n_sms, cudaS
             // main.cpp:361) -- runs of far queries with a neighbour are what the group search is for (3 M-point pair 61.7 -> 47.8 ms,
             // 44-pair queue 291 -> 324 pairs/s, far-heavy pairs -18 %; the bench pair +0.5 %); with a tight threshold (0.1 in the
             // experiment runner) the far queries have no neighbour, the groups that remain cost more than they save (4.0 -> 4.75 ms).
-            const int group_min = getenv("ICP_GPU_GROUP_MIN") ? atoi(getenv("ICP_GPU_GROUP_MIN")) : (a.max_d2 >= 1.0f ? 8 : 0);   // knob; 0 = off
+            const int group_min = getenv("ICP_GPU_GROUP_MIN") ? atoi(getenv("ICP_GPU_GROUP_MIN")) : (a.max_d2 >= 1.0f ? 8 : 0);   // test hook; 0 = off
             // (3-D search only: a 6-D bound holds colour differences too, as a radius in space it makes every group too wide)
-            if (group_min > 0 && a.fast_path && a.use_seed && !a.color_icp) {
+            if (group_min > 0 && !a.color_icp) {
                 ac.group_min = group_min;
                 const int ng = (nq + GROUP_SIZE * GROUP_WARPS - 1) / (GROUP_SIZE * GROUP_WARPS);
                 if (a.collect_stats) knn_group_kernel<true><<<ng, GROUP_WARPS * 32, 0, cs>>>(ac); else knn_group_kernel<false><<<ng, GROUP_WARPS * 32, 0, cs>>>(ac);
@@ -1121,7 +1069,7 @@ cudaError_t icp_launch_match(const MatchArgs& a, int algorithm, int n_sms, cudaS
             // every chunk's walk gets the full grid (its warps then take fewer positions each): a heavy chunk left alone at the end
             // of the iteration still fills the machine
             int nb = (nq + BVH_WARPS - 1) / BVH_WARPS;
-            const int cap = std::max(1, mult * n_sms * 4 / BVH_WARPS);
+            const int cap = std::max(1, WALK_GRID_PER_SM * n_sms * 4 / BVH_WARPS);
             if (nb > cap) nb = cap;
             if (a.collect_stats) { if (a.color_icp) knn_bvh_kernel<true, true><<<nb, BVH_WARPS * 32, 0, cs>>>(ac); else knn_bvh_kernel<false, true><<<nb, BVH_WARPS * 32, 0, cs>>>(ac); }
             else { if (a.color_icp) knn_bvh_kernel<true, false><<<nb, BVH_WARPS * 32, 0, cs>>>(ac); else knn_bvh_kernel<false, false><<<nb, BVH_WARPS * 32, 0, cs>>>(ac); }

@@ -102,9 +102,7 @@ __global__ void __launch_bounds__(128) pca_normals_kernel(const NormalArgs a) {
         if (b.m == k && leaf < a.adj_capacity) {
             const float r = __fmul_ru(__fsqrt_ru(b.d[k - 1]), 1.00001f);
             const float4 ilo = __ldg(&a.adj_box[2 * (size_t)leaf]), ihi = __ldg(&a.adj_box[2 * (size_t)leaf + 1]);
-            const bool inside = __fsub_rd(qx, r) >= ilo.x && __fadd_ru(qx, r) <= ihi.x && __fsub_rd(qy, r) >= ilo.y &&
-                                __fadd_ru(qy, r) <= ihi.y && __fsub_rd(qz, r) >= ilo.z && __fadd_ru(qz, r) <= ihi.z;
-            if (inside) {                                        // never true for the inverted "no list" box
+            if (ball_inside(qx, qy, qz, r, ilo, ihi)) {          // never true for the inverted "no list" box
                 const int na = __float_as_int(ilo.w);
                 for (int j = 0; j < na; ++j) {
                     const unsigned int l2 = __ldg(&a.adj[(size_t)leaf * 32 + j]);

@@ -130,7 +130,7 @@ static int make_plan(icp_gpu_ctx* ctx, Plan& plan) {
 // Projective matching of a full-frame source (one point per pixel of the camera the target was taken with): the kernels
 // then address the source in its original pixel order (the unsorted upload) instead of the Morton order.
 static bool proj_tiled(const icp_gpu_ctx* c, int algo) {
-    return algo == 2 && c->n_src > 0 && (long long)c->width * c->height == (long long)c->n_src && !getenv("ICP_GPU_NO_PROJ_TILES");
+    return algo == 2 && c->n_src > 0 && (long long)c->width * c->height == (long long)c->n_src;
 }
 
 // The clouds the search and the reduction read: the target in grid order for the BVH search, else in upload order; the source in
@@ -151,12 +151,10 @@ void fill_match_args(icp_gpu_ctx* c, MatchArgs& a, int algo, int desc_index, boo
     a.bvh_box = (const float4*)c->bvh_box.p; a.bvh = (const BvhDesc*)c->bvh_desc.p; a.leaf_start = (const unsigned int*)c->leaf_start.p;
     a.leaf_rank = (const unsigned int*)c->leaf_rank.p; a.child_start = (const unsigned int*)c->child_start.p;
     a.adj = (const unsigned int*)c->adj.p; a.adj_box = (const float4*)c->adj_box.p; a.adj_capacity = c->adj_capacity;
-    a.adj_gap = getenv("ICP_GPU_NO_ADJ_GAP") ? nullptr : (const float*)c->adj_gap.p;   // tuning knob (A/B measurement)
+    a.adj_gap = (const float*)c->adj_gap.p;
     a.nn_leaf = (int*)c->nn_leaf.p;
     a.adj1 = (const unsigned int*)c->adj1.p; a.adj1_box = (const float4*)c->adj1_box.p; a.adj1_capacity = c->adj1_capacity;
     a.node_rank = (const unsigned int*)c->node_rank.p;
-    if (getenv("ICP_GPU_NO_ADJACENCY1")) a.adj1_capacity = 0;   // tuning knob
-    if (getenv("ICP_GPU_NO_ADJACENCY")) a.adj_capacity = 0;   // tuning knob
     if (c->have_camera) { a.fx = c->K[0]; a.fy = c->K[4]; a.cx = c->K[6]; a.cy = c->K[7]; }   // column-major Matrix3f
     a.width = c->width; a.height = c->height;
     a.weighting = c->cfg.weighting; a.rejection = c->cfg.rejection; a.color_icp = c->cfg.color_icp;
@@ -166,9 +164,7 @@ void fill_match_args(icp_gpu_ctx* c, MatchArgs& a, int algo, int desc_index, boo
     a.nn_pos = (int*)c->nn_pos.p; a.qbuf = (float4*)c->qbuf.p; a.seedbuf = (float4*)c->seedbuf.p;
     a.desc_index = desc_index;
     a.q_begin = 0; a.q_end = c->n_src;
-    a.use_seed = algo == 0 ? 1 : 0;
     a.brute_norm = c->cfg.nn_algorithm == ICP_GPU_NN_BRUTE_NORM ? 1 : 0;
-    a.fast_path = getenv("ICP_GPU_NO_FASTPATH") ? 0 : 1;   // tuning knob (A/B measurement)
     a.collect_stats = c->cfg.collect_stats;
 }
 
@@ -201,7 +197,7 @@ void fill_reduce_args(icp_gpu_ctx* c, ReduceArgs& r, int algo, int solve) {
 // (grid.cu; queries that still have a neighbour keep it), or reset to "none".
 int refresh_seeds(icp_gpu_ctx* ctx, int algo, bool allow_seed) {
     if (algo != 0 || ctx->n_src <= 0 || !ctx->nn_pos.p) return 0;
-    const bool seed = allow_seed && ctx->n_tgt > 0 && ctx->grid_built && !getenv("ICP_GPU_NO_GRID_SEED");
+    const bool seed = allow_seed && ctx->n_tgt > 0 && ctx->grid_built;
     if (seed) {
         CU(icp_launch_seed_from_keys((const float4*)ctx->src_pts.p, ctx->n_src, (const DevState*)ctx->state.p, (const GridParams*)ctx->grid.p,
                                      ctx->tsort.keys_sorted, ctx->n_tgt, (const unsigned int*)ctx->bbox.p + 7, (const unsigned int*)ctx->tsort.msd.p,
@@ -226,7 +222,7 @@ static int enqueue_iterations(icp_gpu_ctx* ctx, const Plan& plan, int algo, std:
     if (algo == 0 && ctx->cfg.minimizer == ICP_GPU_MIN_LINEAR && !ctx->cfg.collect_stats) { ma.skip_finish = 1; ra.fused = 1; }
     int launches = 0;
     const int nb = ctx->n_reduce_blocks;
-    // Two chunks of >= 64k queries (tuning knob: ICP_GPU_MATCH_CHUNKS).  Measured at 370k queries: 1 / 2 / 3 / 4 chunks
+    // Two chunks of >= 64k queries (test hook: ICP_GPU_MATCH_CHUNKS).  Measured at 370k queries: 1 / 2 / 3 / 4 chunks
     // 4.78 / 4.54 / 4.58 / 4.69 ms per 30-iteration registration.
     MatchChunks mc = ctx->chunks;
     mc.n = ctx->n_src >= 131072 ? 2 : 1;

@@ -11,7 +11,6 @@
 // estimatePoseSymmetricICP (:784-898), pose accumulation (:614-620).
 #include "icp_internal.cuh"
 #include "solve.cuh"
-#include <stdlib.h>
 
 struct PoseSmR { float P[16]; };
 
@@ -168,11 +167,13 @@ __global__ void __launch_bounds__(ICP_REDUCE_THREADS) reduce_kernel(const Reduce
     }
 }
 
+// Blocks of reduce_kernel per SM: 1 / 4 measured 6.46 / 6.36 ms per registration, both slower than 2 (round 1, profiles/README.md);
+// 3 do not fit the registers (DESIGN §4).
+#define REDUCE_BLOCKS_PER_SM 2
+
 int icp_reduce_blocks(int n_src, int n_sms) {
     int nb = (n_src + ICP_REDUCE_THREADS - 1) / ICP_REDUCE_THREADS;
-    int per_sm = 2;
-    if (const char* e = getenv("ICP_GPU_REDUCE_BLOCKS_PER_SM")) { const int v = atoi(e); if (v >= 1 && v <= 32) per_sm = v; }   // tuning knob
-    if (nb > per_sm * n_sms) nb = per_sm * n_sms;
+    if (nb > REDUCE_BLOCKS_PER_SM * n_sms) nb = REDUCE_BLOCKS_PER_SM * n_sms;
     if (nb < 1) nb = 1;
     return nb;
 }

@@ -627,18 +627,17 @@ def test_bench_config_as_run_370k_30_iterations(ctx, full_eth_pair):
     assert worst[0] <= ROT_TOL and worst[1] <= TRANS_TOL, worst        # every iteration of the trajectory, not only the last
 
 
-def test_chunk_chains_and_adjacency_early_exit_change_no_bit(full_eth_pair, monkeypatch):
+def test_chunk_chains_graph_and_group_search_change_no_bit(full_eth_pair, monkeypatch):
     """How the search is scheduled is invisible in the results: one, two or three {prep, walk} chunk chains per iteration
-    (ICP_GPU_MATCH_CHUNKS; two is the default from 131 072 queries on), launched one by one or as a graph, the fast path with
-    or without its early exit from the gap-sorted adjacency lists (ICP_GPU_NO_ADJ_GAP), and runs of deferred neighbours searched
-    with one shared descent or each by its own walk (ICP_GPU_GROUP_MIN: 0 = off, 1 = every run) give the same trajectory and the same
-    correspondences bit for bit.  The variables are read when a registration is enqueued; a fresh context per variant keeps the
-    graph caches apart."""
+    (ICP_GPU_MATCH_CHUNKS; two is the default from 131 072 queries on), launched one by one or as a graph, and runs of deferred
+    neighbours searched with one shared descent or each by its own walk (ICP_GPU_GROUP_MIN: 0 = off, 1 = every run) give the same
+    trajectory and the same correspondences bit for bit.  The variables are read when a registration is enqueued; a fresh context
+    per variant keeps the graph caches apart."""
     src, tgt, _ = full_eth_pair
     runs = []
-    for env in ({"ICP_GPU_MATCH_CHUNKS": "1", "ICP_GPU_GROUP_MIN": "0"}, {}, {"ICP_GPU_MATCH_CHUNKS": "3"}, {"ICP_GPU_NO_ADJ_GAP": "1"},
+    for env in ({"ICP_GPU_MATCH_CHUNKS": "1", "ICP_GPU_GROUP_MIN": "0"}, {}, {"ICP_GPU_MATCH_CHUNKS": "3"},
                 {"ICP_GPU_MATCH_CHUNKS": "2", "use_graph": 0}, {"ICP_GPU_GROUP_MIN": "1"}, {"ICP_GPU_GROUP_MIN": "32"}):
-        for k in ("ICP_GPU_MATCH_CHUNKS", "ICP_GPU_NO_ADJ_GAP", "ICP_GPU_GROUP_MIN"):
+        for k in ("ICP_GPU_MATCH_CHUNKS", "ICP_GPU_GROUP_MIN"):
             monkeypatch.delenv(k, raising=False)
         for k, v in env.items():
             if k.startswith("ICP_"):
