@@ -25,8 +25,7 @@
 // system (ICP_GPU_E_NUMERIC); a failed pair keeps its last good pose.
 #include "solve.cuh"
 #include "lm.cuh"
-
-#define FLT_BIG 3.4028234e38f
+#include "search.cuh"
 
 static_assert(ICP_BATCH_THREADS % 32 == 0 && ICP_BATCH_THREADS <= 1024 && ICP_BATCH_LM_THREADS % 32 == 0, "whole warps");
 
@@ -41,9 +40,7 @@ __device__ __forceinline__ int nearest_staged(const float4* __restrict__ tgt, in
     float bd = bound; int bj = -1;
 #pragma unroll 4
     for (int j = 0; j < n_t; ++j) {
-        const float4 c = tgt[j];
-        const float dx = psub(qx, c.x), dy = psub(qy, c.y), dz = psub(qz, c.z);
-        const float d = padd(padd(pmul(dx, dx), pmul(dy, dy)), pmul(dz, dz));     // D1
+        const float d = dist3(qx, qy, qz, tgt[j]);
         if (d < bd) { bd = d; bj = j; }
     }
     return bj;

@@ -792,10 +792,10 @@ __global__ void __launch_bounds__(UP_THREADS) upper_levels_kernel(int* delta_a, 
 
 // one warp per node (grid-stride): level 0 reads the leaf's points, level l > 0 reads its (<= 32) child boxes
 // The w components of the two box entries carry the node's COLOUR range (min / max of r, g, b as packed bytes), which the
-// 6-D colour search adds to its lower bounds (match.cu: box_dist2c).
+// 6-D colour search adds to its lower bounds (search.cuh: box_dist2c).
 // Level 0 also re-orders every leaf's records by ORIGINAL index (they arrive in (cell code, original index) order): a scan of
 // the leaf in storage order with a strict '<' on the distance then returns the lowest original index among equal distances --
-// contract D2 inside a leaf without comparing indices per candidate (match.cu: thread_scan_leaf).
+// contract D2 inside a leaf without comparing indices per candidate (knn.cu: thread_scan_leaf).
 __global__ void bvh_level_kernel(float4* __restrict__ pts, float4* __restrict__ nrm, const unsigned int* __restrict__ leaf_start,
                                  const unsigned int* __restrict__ child_start, const BvhDesc* __restrict__ bvh, float4* __restrict__ box,
                                  int level) {

@@ -29,6 +29,7 @@ __device__ __forceinline__ float pmul(float a, float b) { return __fmul_rn(a, b)
 __device__ __forceinline__ float padd(float a, float b) { return __fadd_rn(a, b); }
 __device__ __forceinline__ float psub(float a, float b) { return __fsub_rn(a, b); }
 __device__ __forceinline__ float pdiv(float a, float b) { return __fdiv_rn(a, b); }
+#define MINF_F (-INFINITY)         // the reference's MINF: the coordinates of an invalid point
 __device__ __forceinline__ bool finite3(float x, float y, float z) { return isfinite(x) && isfinite(y) && isfinite(z); }
 // The ball of radius r around (x, y, z) lies inside the box [lo, hi].  The ball's bounds are rounded outwards by the explicit _rd / _ru
 // operations, so the answer does not depend on FMA contraction (-fmad) and holds for the exact ball.
@@ -193,9 +194,8 @@ struct MatchArgs {
     float* match_w;
     int* match_idx;          // original target index (API output), may be null
     int* nn_pos;             // nearest neighbour found the last time p was a query (-1 none): seeds the next search
-    float4* seedbuf;         // knn_prep_kernel -> knn_bvh_kernel, per deferred query: {best d2, best idx, best pos, seed leaf} of the seed-leaf
-                             // scan the fast path already made (w = -2: not scanned, the walk starts from nn_pos itself)
-    float4* qbuf;            // transformed query points of the current iteration {x,y,z,rgba}; x = NaN: not searched
+    struct HandOver* seedbuf;  // knn_prep_kernel -> knn_group_kernel / knn_bvh_kernel, per pending query (search.cuh)
+    float4* qbuf;            // transformed query points of the current iteration {x,y,z,rgba}; x = NaN: no search left (search.cuh)
     int desc_index;          // >= 0: fixed descriptor (query_matches); -1: use state->iter
     int brute_norm;          // brute force on rounded Euclidean norms, max_d2 = a plain distance (NearestNeighborSearchBruteForce, NearestNeighbor.h:81-97)
     int proj_tiled;          // projective matching of a full-frame source: src arrays are in ORIGINAL (pixel) order, one 32x4 tile per block
@@ -205,7 +205,7 @@ struct MatchArgs {
     int group_min;           // knn_group_kernel: fewest handed-over queries among 32 consecutive positions that share one descent
 };
 
-// Concurrency inside one iteration (registration.cu, match.cu): the queries are cut into chunks, each chunk's {prep, walk} chain runs on its own
+// Concurrency inside one iteration (registration.cu, knn.cu): the queries are cut into chunks, each chunk's {prep, walk} chain runs on its own
 // stream between a fork and a join event; the per-query results do not depend on the cut.
 #define ICP_MAX_MATCH_CHUNKS 8
 struct MatchChunks {
@@ -269,7 +269,7 @@ cudaError_t icp_launch_pack_pairs(const float* s, const float* sn, const float* 
                                   float4* tp4, float4* tn4, int* pos, float* wo, cudaStream_t st);
 // peak.cu: measured FP32 throughput of the device (mode 0 FFMA, 1 FMUL+FADD), TFLOP/s
 cudaError_t icp_measure_fp32_peak(int mode, int n_sms, cudaStream_t s, double* tflops);
-// ---- launchers (defined in grid.cu / match.cu / solve.cu / lm.cu) ----
+// ---- launchers (defined in grid.cu / match.cu / knn.cu / solve.cu / lm.cu) ----
 // AoS3 -> float4 records, the bounding box of the finite points and from it the grid parameters; clears the sort's histograms
 // (scratch: 8 words, [7] = number of points with a non-finite coordinate afterwards)
 cudaError_t icp_launch_pack_cloud(const float* xyz, const float* nrm, const uint8_t* rgba, int n, float4* pts, float4* nrmo,
@@ -334,6 +334,7 @@ struct NormalArgs {
 cudaError_t icp_launch_pca_normals(const NormalArgs& a, cudaStream_t s);
 cudaError_t icp_launch_match(const MatchArgs& a, int algorithm, int n_sms, cudaStream_t s, int* n_launches, cudaEvent_t after_prep = nullptr,
                              const MatchChunks* chunks = nullptr);
+void icp_launch_knn(const MatchArgs& a, int n_sms, cudaStream_t s, cudaEvent_t after_prep, const MatchChunks* chunks, int& launches);   // knn.cu
 cudaError_t icp_launch_pose_init(DevState* st, const float* pose_dev16, cudaStream_t s, float stop_rot = 0.f, float stop_trans = 0.f);
 cudaError_t icp_launch_reduce(const ReduceArgs& a, int n_blocks, cudaStream_t s, int* n_launches);
 // one phase of the point-sharded iteration: the summed row is left in state->shard_partials

@@ -10,21 +10,12 @@
 // box, only the leaves of its adjacency list (grid.cu) can hold closer points; otherwise the thread walks the BVH with a
 // private stack.  This file is compiled with -fmad=false: the double arithmetic below is the oracle's, operation for
 // operation, so the normals agree bit for bit.
-#include "icp_internal.cuh"
-#include <limits.h>
+#include "search.cuh"
 
 #define NRM_KMAX 8
 #define NRM_STACK (32 * ICP_BVH_MAX_LEVELS)
-#define FLT_BIG 3.4028234e38f
 
 struct KBest { float d[NRM_KMAX]; int idx[NRM_KMAX]; int pos[NRM_KMAX]; int m; };
-
-__device__ __forceinline__ float nrm_box_dist2(float qx, float qy, float qz, const float4 lo, const float4 hi) {
-    const float gx = fmaxf(fmaxf(psub(lo.x, qx), psub(qx, hi.x)), 0.0f);
-    const float gy = fmaxf(fmaxf(psub(lo.y, qy), psub(qy, hi.y)), 0.0f);
-    const float gz = fmaxf(fmaxf(psub(lo.z, qz), psub(qz, hi.z)), 0.0f);
-    return padd(padd(pmul(gx, gx), pmul(gy, gy)), pmul(gz, gz));
-}
 
 // the distance a candidate has to beat: the k-th best so far, or "anything" while the list is not full
 __device__ __forceinline__ float kth(const KBest& b, int k) { return b.m < k ? FLT_BIG : b.d[k - 1]; }
@@ -47,8 +38,7 @@ __device__ __forceinline__ void nrm_scan_leaf(const float4* __restrict__ pts, co
     const unsigned int ls = __ldg(&leaf_start[leaf]), le = __ldg(&leaf_start[leaf + 1]);
     for (unsigned int i = ls; i < le; ++i) {
         const float4 p = __ldg(&pts[i]);
-        const float dx = psub(qx, p.x), dy = psub(qy, p.y), dz = psub(qz, p.z);
-        const float d = padd(padd(pmul(dx, dx), pmul(dy, dy)), pmul(dz, dz));      // D1
+        const float d = dist3(qx, qy, qz, p);
         if (!isfinite(d)) continue;
         kbest_insert(b, k, d, __float_as_int(p.w), (int)i);
     }
@@ -81,8 +71,7 @@ __device__ void nrm_eig3(double* A, double* V, double* evals) {
 
 __global__ void __launch_bounds__(128) pca_normals_kernel(const NormalArgs a) {
     __shared__ BvhDesc s_bvh;
-    if (threadIdx.x < sizeof(BvhDesc) / 4) reinterpret_cast<int*>(&s_bvh)[threadIdx.x] = reinterpret_cast<const int*>(a.bvh)[threadIdx.x];
-    __syncthreads();
+    stage_bvh_desc(s_bvh, a.bvh);
     const BvhDesc& bvh = s_bvh;
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= a.n) return;
@@ -100,13 +89,13 @@ __global__ void __launch_bounds__(128) pca_normals_kernel(const NormalArgs a) {
         nrm_scan_leaf(a.pts, a.leaf_start, (unsigned int)leaf, qx, qy, qz, b, k);
         bool done = false;
         if (b.m == k && leaf < a.adj_capacity) {
-            const float r = __fmul_ru(__fsqrt_ru(b.d[k - 1]), 1.00001f);
+            const float r = search_radius(b.d[k - 1]);
             const float4 ilo = __ldg(&a.adj_box[2 * (size_t)leaf]), ihi = __ldg(&a.adj_box[2 * (size_t)leaf + 1]);
             if (ball_inside(qx, qy, qz, r, ilo, ihi)) {          // never true for the inverted "no list" box
                 const int na = __float_as_int(ilo.w);
                 for (int j = 0; j < na; ++j) {
                     const unsigned int l2 = __ldg(&a.adj[(size_t)leaf * 32 + j]);
-                    const float clb = nrm_box_dist2(qx, qy, qz, __ldg(&a.bvh_box[2 * (size_t)l2]), __ldg(&a.bvh_box[2 * (size_t)l2 + 1]));
+                    const float clb = box_dist2(qx, qy, qz, __ldg(&a.bvh_box[2 * (size_t)l2]), __ldg(&a.bvh_box[2 * (size_t)l2 + 1]));
                     if (!(clb > kth(b, k))) nrm_scan_leaf(a.pts, a.leaf_start, l2, qx, qy, qz, b, k);
                 }
                 done = true;
@@ -126,7 +115,7 @@ __global__ void __launch_bounds__(128) pca_normals_kernel(const NormalArgs a) {
                 while (top > 0) {
                     const unsigned int e = st[--top];
                     const int lvl = (int)(e >> 27); const unsigned int j = e & 0x7FFFFFFu;
-                    const float clb = nrm_box_dist2(qx, qy, qz, __ldg(&a.bvh_box[2 * (size_t)(bvh.offset[lvl] + j)]), __ldg(&a.bvh_box[2 * (size_t)(bvh.offset[lvl] + j) + 1]));
+                    const float clb = box_dist2(qx, qy, qz, __ldg(&a.bvh_box[2 * (size_t)(bvh.offset[lvl] + j)]), __ldg(&a.bvh_box[2 * (size_t)(bvh.offset[lvl] + j) + 1]));
                     if (clb > kth(b, k)) continue;
                     if (lvl == 0) { if ((int)j != leaf) nrm_scan_leaf(a.pts, a.leaf_start, j, qx, qy, qz, b, k); continue; }
                     const unsigned int first = __ldg(&a.child_start[bvh.coffset[lvl] + j]), last = __ldg(&a.child_start[bvh.coffset[lvl] + j + 1]);

@@ -9,7 +9,6 @@
 #include "icp_internal.cuh"
 
 #define PREP_THREADS 256
-#define MINF_F (-INFINITY)
 
 // ---------------------------------------------------------------------------- depth -> cloud
 // One thread per candidate pixel i = k * downsample.  Writes the point, the normal and the colour of the candidate to

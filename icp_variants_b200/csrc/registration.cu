@@ -1,5 +1,5 @@
 // registration.cu -- the registration loop (icp_gpu_estimate_pose[_async/_finish]): iteration planning, CUDA-graph replay of the
-// loop, and the matches at one pose (icp_gpu_query_matches).  Host code only; the kernels live in grid.cu, match.cu, solve.cu and lm.cu.
+// loop, and the matches at one pose (icp_gpu_query_matches).  Host code only; the kernels live in grid.cu, match.cu, knn.cu, solve.cu and lm.cu.
 //
 // What runs where: the host plans the iterations (level strides, selection masks) and enqueues
 // them; every iteration is {match kernel, reduction(+solve) kernel(s)} on one stream with no host
@@ -161,7 +161,7 @@ void fill_match_args(icp_gpu_ctx* c, MatchArgs& a, int algo, int desc_index, boo
     a.max_d2 = c->cfg.max_distance_sq;
     a.weight_max_d2 = c->cfg.weight_max_distance_sq > 0.f ? c->cfg.weight_max_distance_sq : c->cfg.max_distance_sq;
     a.match_pos = (int*)c->match_pos.p; a.match_w = (float*)c->match_w.p; a.match_idx = want_idx ? (int*)c->match_idx.p : nullptr;
-    a.nn_pos = (int*)c->nn_pos.p; a.qbuf = (float4*)c->qbuf.p; a.seedbuf = (float4*)c->seedbuf.p;
+    a.nn_pos = (int*)c->nn_pos.p; a.qbuf = (float4*)c->qbuf.p; a.seedbuf = (HandOver*)c->seedbuf.p;
     a.desc_index = desc_index;
     a.q_begin = 0; a.q_end = c->n_src;
     a.brute_norm = c->cfg.nn_algorithm == ICP_GPU_NN_BRUTE_NORM ? 1 : 0;

@@ -63,7 +63,7 @@ __device__ void finish_sums(DevState* st, const double* row) {
     }
 }
 
-#ifdef ICP_TIMELINE   // diagnostic build (profiles/): see match.cu; per block of iteration 12 {start, loop end}, [511] = {pose written, 0}
+#ifdef ICP_TIMELINE   // diagnostic build (profiles/): see knn.cu; per block of iteration 12 {start, loop end}, [511] = {pose written, 0}
 __device__ unsigned long long g_timeline_r[512][2];
 __device__ __forceinline__ unsigned long long tlr_now() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
 extern "C" int icp_gpu_debug_timeline_reduce(unsigned long long* out, int reset) {

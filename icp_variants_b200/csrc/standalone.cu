@@ -1,5 +1,5 @@
 // standalone.cu -- the value-level operations of the reference's API that its drivers and tests call OUTSIDE estimatePose, on the
-// device behind their own C-ABI entry points (the loop itself runs them fused, match.cu / solve.cu -- same device functions):
+// device behind their own C-ABI entry points (the loop itself runs them fused, match.cu / knn.cu / solve.cu -- same device functions):
 //   transformPoints / transformNormals           utils.h:106-133      icp_gpu_transform_points / _normals
 //   WeightingMethod::applyWeights                weighting.h:39-99    icp_gpu_apply_weights
 //   ProcrustesAligner::estimatePose and the two linear-system solvers of LinearICPOptimizer

@@ -19,7 +19,7 @@ python profiles/probe_pair_costs.py > $F/pair_costs_by_distance.json 2> $F/pair_
 bash profiles/ab_group.sh > $F/group_search_ab.txt 2>&1
 make -C icp_variants_b200/csrc groupprobe > $F/make_groupprobe.log 2>&1
 ICP_GPU_LIB_NAME=libicp_gpu_groupprobe.so PAIRS=0,28,34 GROUP_MINS="0 8" python profiles/probe_group.py > $F/group_search_per_pair.json 2> $F/group_search_per_pair.err
-rm -f icp_variants_b200/lib/libicp_gpu_groupprobe.so icp_variants_b200/lib/match_groupprobe.o
+rm -f icp_variants_b200/lib/libicp_gpu_groupprobe.so icp_variants_b200/lib/knn_groupprobe.o
 python profiles/probe_group_shard.py > $F/group_search_on_a_shard.json 2> $F/group_search_on_a_shard.err
 # per-warp timeline of one iteration, one and two chunk chains (diagnostic build of the library, removed again afterwards)
 make -C icp_variants_b200/csrc timeline > $F/make_timeline.log 2>&1

@@ -1,6 +1,6 @@
 """Timeline of ONE iteration (the 13th) of BASELINE config 2 inside the graph replay: start and end of every warp of knn_prep_kernel
 and knn_bvh_kernel and of every block of reduce_kernel (%globaltimer, plain stores), written by a DIAGNOSTIC build of the library
-(match.cu / solve.cu compiled with -DICP_TIMELINE into lib/libicp_gpu_timeline.so, profiles/README.md).  Shows what the kernels' own
+(knn.cu / solve.cu compiled with -DICP_TIMELINE into lib/libicp_gpu_timeline.so, profiles/README.md).  Shows what the kernels' own
 durations do not: ramps, tails, how many warps are resident over time and the gaps between dependent launches.
 Usage: ICP_GPU_MATCH_CHUNKS=1|2 python profiles/probe_timeline.py"""
 import ctypes as C

@@ -1,4 +1,4 @@
-"""CPU property test of the pruning rule of the group search (csrc/match.cu: GroupBounds / group_keeps): a restatement in numpy
+"""CPU property test of the pruning rule of the group search (csrc/knn.cu: GroupBounds / group_keeps): a restatement in numpy
 fp32 of the two node tests, with round-to-nearest where the device rounds outwards (so the restated bounds are at most as wide as
 the device's: what holds here holds there).  Claim: a box that holds a point p whose D1 distance (contract D1: fp32,
 ((dx*dx + dy*dy) + dz*dz), no FMA) to SOME member is <= that member's bound is never dropped -- whatever the scale of the

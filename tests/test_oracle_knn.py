@@ -89,8 +89,8 @@ def test_6d_colour_search():
 
 
 def test_packed_key_order_equals_lexicographic_distance_index_order():
-    """The grid search kernels compare candidates as ONE unsigned 64-bit key bits(d2) << 32 | idx (match.cu: better_key,
-    thread_scan_leaf).  That is the (d2, idx) lexicographic order of contract D2 for every non-negative fp32 distance --
+    """The grid search kernels compare candidates as ONE unsigned 64-bit key bits(d2) << 32 | idx (search.cuh: better_key;
+    knn.cu: thread_scan_leaf).  That is the (d2, idx) lexicographic order of contract D2 for every non-negative fp32 distance --
     +0, denormals, FLT_MAX, +inf -- and puts NaN distances after every number, as the strict comparisons of
     NearestNeighbor.h:81-97 do."""
     rng = np.random.default_rng(11)
