@@ -113,6 +113,8 @@ def lib():
             "icp_gpu_iterations_bound": (C.c_int, [C.POINTER(Config), i64]),
             "icp_gpu_estimate_pose_batch_configs": (C.c_int, [vp, i32, C.POINTER(Config), i32, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, i32]),
             "icp_gpu_estimate_pose_batch_configs_dev": (C.c_int, [vp, i32, C.POINTER(Config), i32, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, i32]),
+            "icp_gpu_estimate_pose_multistart": (C.c_int, [vp, i32, pf, pf, pf, pf, pf, pf, pf, pf, pf]),
+            "icp_gpu_estimate_pose_multistart_dev": (C.c_int, [vp, i32, pf, pf, pf, pf, pf, pf, pf, pf, pf]),
             "icp_gpu_get_stats": (C.c_int, [vp, C.POINTER(Stats)]),
             "icp_gpu_measure_fp32_peak": (C.c_int, [vp, i32, C.POINTER(C.c_double)]),
             "icp_gpu_alignment_error": (C.c_int, [vp, pf, pf, C.POINTER(C.c_double)]),
@@ -169,6 +171,16 @@ def _config_table(configs, config_index, B):
     if ci.shape != (B,):
         raise ValueError(f"config_index: expected [{B}] indices, got {ci.shape}")
     return table, len(configs), ci
+
+
+def best_start(inliers, rmse) -> int:
+    """The start with the most inliers; ties go to the lower RMSE (NaN last), then to the lower index.  -1 for no start."""
+    inl = np.asarray(inliers, np.int64)
+    if len(inl) == 0:
+        return -1
+    r = np.asarray(rmse, np.float64)
+    r = np.where(np.isnan(r), np.inf, r)
+    return int(np.lexsort((np.arange(len(inl)), r, -inl))[0])
 
 
 def pose_to_c(pose) -> np.ndarray:
@@ -474,6 +486,72 @@ class Context:
             return hist
 
         return self._batch_dev(run, src_xyz, src_off, tgt_xyz, tgt_off, src_nrm, tgt_nrm, init_poses)
+
+    # -- many starts of the context's own pair in one launch
+    def estimate_pose_multistart(self, init_poses, want_history=False, want_matches=False):
+        """K registrations of the context's source against its target from the initial poses init_poses [K,4,4], each scored at
+        its final pose.  Returns a dict: poses [K,4,4], n_iterations [K], status [K] (OK / E_NO_MATCHES / E_NUMERIC per start),
+        inliers [K] int64, rmse [K] float64 (NaN without an inlier), best (the start with the most inliers, ties to the lower RMSE,
+        then the lower index; -1 when K = 0), and with want_history history [K, max_iterations, 4, 4] (rows past a start's last
+        iteration 0), with want_matches match_idx / match_w [K, n_source] (query_matches at each final pose)."""
+        p = np.asarray(init_poses, np.float32)
+        if p.ndim != 3 or p.shape[1:] != (4, 4):
+            raise ValueError(f"init_poses: expected [K,4,4], got {p.shape}")
+        K, n = len(p), self.n_source
+        pin = np.ascontiguousarray(p.transpose(0, 2, 1).reshape(K, 16))
+        pout = np.zeros((K, 16), np.float32)
+        n_it = np.zeros(K, np.int32)
+        status = np.zeros(K, np.int32)
+        inl = np.zeros(K, np.int64)
+        rmse = np.zeros(K, np.float64)
+        rows = max(self.max_iterations(), 0)
+        hist = np.zeros((K, max(rows, 1), 16), np.float32) if want_history else None
+        midx = np.zeros((K, max(n, 1)), np.int32) if want_matches else None
+        mw = np.zeros((K, max(n, 1)), np.float32) if want_matches else None
+        self._check(lib().icp_gpu_estimate_pose_multistart(self._h, K, _ptr(pin), _ptr(pout), _ptr(n_it), _ptr(status), _ptr(inl), _ptr(rmse),
+                                                           _ptr(hist), _ptr(midx), _ptr(mw)))
+        out = {"poses": pout.reshape(K, 4, 4).transpose(0, 2, 1).copy(), "n_iterations": n_it, "status": status, "inliers": inl,
+               "rmse": rmse, "best": best_start(inl, rmse)}
+        if want_history:
+            out["history"] = hist[:, :rows].reshape(K, rows, 4, 4).transpose(0, 1, 3, 2).copy()
+        if want_matches:
+            out["match_idx"], out["match_w"] = midx[:, :n].copy(), mw[:, :n].copy()
+        return out
+
+    def estimate_pose_multistart_dev(self, init_poses, want_history=False, want_matches=False):
+        """The same on CUDA torch tensors of the context's device: init_poses a float32 [K,4,4] tensor; the dict's arrays are CUDA
+        tensors (best a Python int).  Work queued on the current torch stream is waited for; the results are complete when the
+        call returns."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        if not (isinstance(init_poses, torch.Tensor) and init_poses.device == dev and init_poses.dtype == torch.float32
+                and init_poses.dim() == 3 and tuple(init_poses.shape[1:]) == (4, 4)):
+            raise ValueError(f"init_poses: expected a float32 [K,4,4] tensor on {dev}")
+        K, n = init_poses.shape[0], self.n_source
+        pin = init_poses.transpose(1, 2).contiguous()         # column-major per pose (Eigen::Matrix4f::data())
+        pout = torch.empty((K, 4, 4), dtype=torch.float32, device=dev)
+        n_it = torch.empty(K, dtype=torch.int32, device=dev)
+        status = torch.empty(K, dtype=torch.int32, device=dev)
+        inl = torch.empty(K, dtype=torch.int64, device=dev)
+        rmse = torch.empty(K, dtype=torch.float64, device=dev)
+        rows = max(self.max_iterations(), 0)
+        hist = torch.zeros((K, max(rows, 1), 4, 4), dtype=torch.float32, device=dev) if want_history else None
+        midx = torch.empty((K, max(n, 1)), dtype=torch.int32, device=dev) if want_matches else None
+        mw = torch.empty((K, max(n, 1)), dtype=torch.float32, device=dev) if want_matches else None
+
+        def p(x):
+            return None if x is None else C.c_void_p(x.data_ptr())
+
+        torch.cuda.current_stream(dev).synchronize()
+        self._check(lib().icp_gpu_estimate_pose_multistart_dev(self._h, K, p(pin), p(pout), p(n_it), p(status), p(inl), p(rmse), p(hist),
+                                                               p(midx), p(mw)))
+        out = {"poses": pout.transpose(1, 2).contiguous(), "n_iterations": n_it, "status": status, "inliers": inl, "rmse": rmse,
+               "best": best_start(inl.cpu().numpy(), rmse.cpu().numpy())}
+        if want_history:
+            out["history"] = hist[:, :rows].transpose(2, 3).contiguous()
+        if want_matches:
+            out["match_idx"], out["match_w"] = midx[:, :n], mw[:, :n]
+        return out
 
     def cloud_from_depth(self, depth, rgbx, K, extrinsics=None, keep_original_size=False, downsample=1, max_distance=0.1,
                          role: int = 2, download: bool = True):

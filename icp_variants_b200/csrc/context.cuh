@@ -61,6 +61,7 @@ struct icp_gpu_ctx {
     DeviceBuf prep_in, prep_tmp, prep_out, gt_src, gt_ref, met_partial, met_out;
     DeviceBuf scratch[16];                                   // operands of the value-level entry points (transform, weights, solve)
     DeviceBuf batch_io, batch_scratch, batch_plan;           // batched registration: uploaded operands + results, match slices, configs + pair lists + masks
+    DeviceBuf ms_io, ms_nn, ms_scratch, ms_desc, ms_mask;    // multi-start registration: operands + results, per-(start, query) neighbours and match slices, plan
     long long n_gt = 0; int last_iters = 0;
     float* h_pose = nullptr; float* h_history = nullptr; DevState* h_state = nullptr;   // pinned
     IterDesc* h_desc = nullptr;                                                       // pinned, DESC_TOTAL
@@ -107,6 +108,14 @@ int status_error(icp_gpu_ctx* ctx, int status, int iteration, const char* no_mat
 // Offsets of segments of the given byte sizes laid out one after the other in one allocation, each 256-byte aligned; returns the total.
 size_t pack_segments(const size_t* sizes, int n, size_t* off);
 
+// The iterations of one registration (make_plan, registration.cu).
+struct Plan {
+    int n_iters = 0;
+    std::vector<IterDesc> desc;         // n_iters entries
+    std::vector<uint32_t> mask;         // concatenated selection masks, one bit per original source index (mt19937 mode)
+    std::vector<int> voxel_depth;       // voxel pyramid: grid depth of every mask slot built on the device
+};
+
 // 32-bit words of a selection mask over n source points (one word at least)
 inline size_t mask_words(long long n) { return ((size_t)(n > 0 ? n : 1) + 31) / 32; }
 
@@ -132,4 +141,6 @@ int check_ready(icp_gpu_ctx* ctx);                                              
 void fill_match_args(icp_gpu_ctx* c, MatchArgs& a, int algo, int desc_index, bool want_idx);                               // registration.cu
 void fill_reduce_args(icp_gpu_ctx* c, ReduceArgs& r, int algo, int solve);                                                 // registration.cu
 int refresh_seeds(icp_gpu_ctx* ctx, int algo, bool allow_seed);                                                            // registration.cu
+int make_plan(icp_gpu_ctx* ctx, Plan& plan);                                                                               // registration.cu
+int upload_plan(icp_gpu_ctx* ctx, const Plan& plan, IterDesc* desc, DeviceBuf& mask, bool graph_reads);                   // registration.cu
 void peer_close(icp_gpu_ctx* ctx);                                                                                         // sharded.cu

@@ -14,7 +14,7 @@
 // Launches of one target build (no host synchronisation): pack+bbox+grid parameters, keys+hist, (scan, scatter) x passes, gather,
 // leaf flags, leaf ranks, leaf boxes, level-1 flags / ranks / boxes, one single-block kernel for all levels above,
 // two adjacency kernels.
-#include "icp_internal.cuh"
+#include "search.cuh"
 #include <string.h>
 
 // ---------------------------------------------------------------------------- pack AoS3 -> float4, bounding box
@@ -149,25 +149,6 @@ __device__ void grid_params_from_bbox(const unsigned int* bbox, int T, GridParam
     for (int k = 0; k < T; ++k) { const int a = (int)((seq >> (2 * k)) & 3ull); --r[a]; P.bitpos[a][r[a]] = (unsigned char)(T - 1 - k); }
 }
 
-__device__ __forceinline__ int cell_index(const GridParams& g, int a, float x) {
-    const float u = pmul(psub(x, g.o[a]), g.inv_h[a]);
-    int i = (int)floorf(u);
-    const int hi = (1 << g.bits[a]) - 1;
-    return min(max(i, 0), hi);
-}
-
-// The code bits an axis contributes for cell index c: bit j of c lands at bitpos[a][j].
-__device__ __forceinline__ unsigned int axis_spread(const GridParams& g, int a, int c) {
-    unsigned int code = 0;
-#pragma unroll
-    for (int j = 0; j < ICP_MAX_BITS_PER_AXIS; ++j)
-        if (j < g.bits[a]) code |= (((unsigned int)c >> j) & 1u) << g.bitpos[a][j];
-    return code;
-}
-
-__device__ __forceinline__ unsigned int cell_code(const GridParams& g, float x, float y, float z) {
-    return axis_spread(g, 0, cell_index(g, 0, x)) | axis_spread(g, 1, cell_index(g, 1, y)) | axis_spread(g, 2, cell_index(g, 2, z));
-}
 
 // ---------------------------------------------------------------------------- stable LSD radix sort of (key, index)
 // key = cell code (T bits); a point with a non-finite coordinate gets 1 << T: it sorts after every cell (sources keep such
@@ -487,12 +468,10 @@ cudaError_t icp_launch_fill_int(int* p, int n, int v, cudaStream_t s) {
 }
 
 // ---------------------------------------------------------------------------- first-iteration seeds from the sorted keys
-// A query that remembers no neighbour (nn_pos < 0, or `reset`: a new cloud made every remembered neighbour stale) gets a
-// point of the smallest cell-tree node around its transformed position that holds any point: the keys are sorted, so that
-// is the lower bound of the query's cell code or its predecessor -- whichever shares the longer prefix with the code.  The
-// lower bound is searched inside the bucket of the code's most significant digit (msd_start, a by-product of the last
-// sorting pass).  The search uses a seed only as its starting bound and first leaf, so any target point is a valid seed -- a
-// near one lets the first iteration run like the later ones (fast path for most queries).
+// A query that remembers no neighbour (nn_pos < 0, or `reset`: a new cloud made every remembered neighbour stale) gets the
+// point key_seed (search.cuh) reads off the sorted keys at its transformed position.  The search uses a seed only as its
+// starting bound and first leaf, so any target point is a valid seed -- a near one lets the first iteration run like the later
+// ones (fast path for most queries).
 __global__ void seed_from_keys_kernel(const float4* __restrict__ src_pts, int n_src, const DevState* __restrict__ st,
                                       const GridParams* __restrict__ gp, const unsigned int* __restrict__ keys, int n_tgt,
                                       const unsigned int* __restrict__ nonfinite, const unsigned int* __restrict__ msd_start, int msd_shift,
@@ -500,32 +479,15 @@ __global__ void seed_from_keys_kernel(const float4* __restrict__ src_pts, int n_
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n_src) return;
     if (!reset && nn_pos[p] >= 0) return;
-    int out_pos = -1, out_leaf = -1;
-    const int n_finite = n_tgt - (int)*nonfinite;
+    int out_leaf = -1;
     const float4 s = src_pts[p];
     float P[16];
 #pragma unroll
     for (int k = 0; k < 16; ++k) P[k] = st->pose[k];
     float x, y, z;
     xform_point(P, s.x, s.y, s.z, x, y, z);
-    if (n_finite > 0 && finite3(x, y, z)) {
-        const GridParams g = *gp;
-        const unsigned int c = cell_code(g, x, y, z);
-        int lo = (int)msd_start[c >> msd_shift], hi = (int)msd_start[(c >> msd_shift) + 1];
-        if (hi > n_finite) hi = n_finite;
-        if (lo > hi) lo = hi;
-        while (lo < hi) {                                   // lower bound of c
-            const int mid = (lo + hi) >> 1;
-            if (keys[mid] < c) lo = mid + 1; else hi = mid;
-        }
-        int pos = lo;
-        if (pos >= n_finite) pos = n_finite - 1;
-        else if (pos > 0) {
-            const unsigned int xa = keys[pos] ^ c, xb = keys[pos - 1] ^ c;
-            if (xb < xa) pos = pos - 1;                     // smaller xor = longer common prefix
-        }
-        out_pos = pos; out_leaf = (int)(leaf_rank[pos + 1] - 1u);
-    }
+    const int out_pos = key_seed(gp, keys, n_tgt - (int)*nonfinite, msd_start, msd_shift, x, y, z);
+    if (out_pos >= 0) out_leaf = (int)(leaf_rank[out_pos + 1] - 1u);
     if (reset || out_pos >= 0) { nn_pos[p] = out_pos; nn_leaf[p] = out_leaf; }
 }
 

@@ -261,6 +261,30 @@ struct BatchArgs {
 // metric: ICP_GPU_METRIC_*, lm: the minimiser; pairs: n_pairs block indices in device memory (BatchArgs::pairs)
 cudaError_t icp_launch_batch(const BatchArgs& a, int metric, int lm, int n_pairs, int max_tgt, cudaStream_t s);
 
+// multistart.cu: K registrations of the context's source against its indexed target, one thread-block cluster per start
+#define ICP_MS_THREADS 256       // threads per block (the LM jets need up to 255 registers a thread); also the tile: 256 sorted positions
+#define ICP_MS_SLICES 16         // tile t is summed into slice t mod 16, the slices in order: the largest cluster
+struct MsArgs {
+    const float4* src_pts; const float4* src_nrm; int n_src;           // sorted source (MatchArgs)
+    const float4* tgt_pts; const float4* tgt_nrm; int n_tgt;           // target in grid order
+    const float4* bvh_box; const BvhDesc* bvh; const unsigned int* leaf_start; const unsigned int* leaf_rank; const unsigned int* child_start;
+    const unsigned int* adj; const float4* adj_box; int adj_capacity;
+    // the first-iteration seeds (key_seed, search.cuh)
+    const GridParams* grid; const unsigned int* keys; const unsigned int* msd_start; int msd_shift; const unsigned int* nonfinite;
+    const IterDesc* desc; const unsigned int* mask; int n_iters;      // the plan of make_plan (registration.cu)
+    int weighting, rejection, lm_max_iterations;
+    float max_d2, weight_max_d2, stop_rot, stop_trans;
+    const float* poses_in; float* poses_out; int* n_iter_out; int* status_out;   // [K][16] column-major, [K], [K]
+    long long* inliers_out; double* rmse_out;                          // the scoring pass, [K]
+    float* history; int history_rows;                                  // [K][history_rows][16] or null
+    int* match_idx; float* match_w;                                    // [K][n_src] in original source order, or null
+    int* nn_pos;                                                       // [K][n_src]: last neighbour of (start, sorted position), -1 = none
+    int2* scratch;                                                     // [K][n_src] symmetric metric and LM: {target position or -1, weight bits}
+};
+// lm: the minimiser; metric: ICP_GPU_METRIC_*; color: 6-D search.  The cluster size (blocks per start) is chosen from n_starts and the
+// SM count and returned in *cluster.
+cudaError_t icp_launch_multistart(const MsArgs& a, int lm, int metric, int color, int n_starts, int n_sms, cudaStream_t s, int* cluster);
+
 // standalone.cu: the reference API's value-level operations outside the loop
 cudaError_t icp_launch_transform(const float* in, long long n, const float pose16[16], int normals, float* out, cudaStream_t s);
 cudaError_t icp_launch_apply_weights(int method, float max_d2, const float* sp, const float* sn, const unsigned int* sc, const float* tp, const float* tn,

@@ -43,13 +43,6 @@ struct Mt19937 {
 
 long long __float_as_int_host(float f) { int32_t i; memcpy(&i, &f, 4); return (long long)i; }
 
-struct Plan {
-    int n_iters = 0;
-    std::vector<IterDesc> desc;         // n_iters entries
-    std::vector<uint32_t> mask;         // concatenated selection masks, one bit per original source index (mt19937 mode)
-    std::vector<int> voxel_depth;       // voxel pyramid: grid depth of every mask slot built on the device
-};
-
 struct KernelClouds { const float4 *src_pts, *src_nrm, *tgt_pts, *tgt_nrm; bool tiled; };   // kernel_clouds
 
 }  // namespace
@@ -92,7 +85,7 @@ int check_ready(icp_gpu_ctx* ctx) {
 }
 
 // The iteration schedule of estimatePose (ICPOptimizer.h:503-525, :540, :549-550, :634-655; Appendix A of SURVEY.md).
-static int make_plan(icp_gpu_ctx* ctx, Plan& plan) {
+int make_plan(icp_gpu_ctx* ctx, Plan& plan) {
     const icp_gpu_config& cfg = ctx->cfg;
     const int n = ctx->n_src;
     const bool host_rng = cfg.selection == ICP_GPU_SELECT_RANDOM && cfg.selection_rng == ICP_GPU_RNG_MT19937;
@@ -239,6 +232,32 @@ static int enqueue_iterations(icp_gpu_ctx* ctx, const Plan& plan, int algo, std:
     return 0;
 }
 
+// The plan on the device, on the context's stream: the descriptors to desc (plan.n_iters entries, through the pinned staging), the
+// selection masks to mask -- the voxel pyramid's levels built on the device, or the mt19937 masks drawn on the host.  graph_reads:
+// the captured loop reads mask (ensure).
+int upload_plan(icp_gpu_ctx* ctx, const Plan& plan, IterDesc* desc, DeviceBuf& mask, bool graph_reads) {
+    memcpy(ctx->h_desc, plan.desc.data(), sizeof(IterDesc) * (size_t)plan.n_iters);
+    if (plan.n_iters > 0) CU(cudaMemcpyAsync(desc, ctx->h_desc, sizeof(IterDesc) * (size_t)plan.n_iters, cudaMemcpyHostToDevice, ctx->stream));
+    if (!plan.voxel_depth.empty()) {
+        const size_t words = mask_words(ctx->n_src);
+        int dmax = 0; for (int D : plan.voxel_depth) dmax = D > dmax ? D : dmax;
+        if (ensure(ctx, mask, plan.voxel_depth.size() * words * sizeof(uint32_t), graph_reads) ||
+            ensure(ctx, ctx->voxel_table, sizeof(unsigned int) * ((size_t)1 << dmax), graph_reads)) return ICP_GPU_E_CUDA;
+        int launches = 0;
+        for (size_t j = 0; j < plan.voxel_depth.size(); ++j)
+            CU(icp_launch_voxel_level((const float4*)ctx->src_pts.p, (const float4*)ctx->src_nrm.p, ctx->n_src, (const GridParams*)ctx->sgrid.p,
+                                      ctx->Ts, plan.voxel_depth[j], (unsigned int*)ctx->voxel_table.p, (unsigned int*)mask.p + j * words,
+                                      words, ctx->stream, &launches));
+        ctx->stats.n_kernel_launches += (uint64_t)launches;
+    }
+    if (!plan.mask.empty()) {
+        if (ensure(ctx, mask, plan.mask.size() * sizeof(uint32_t), graph_reads)) return ICP_GPU_E_CUDA;
+        CU(cudaMemcpyAsync(mask.p, plan.mask.data(), plan.mask.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));   // plan.mask is pageable and dies with this frame
+    }
+    return 0;
+}
+
 static int start_registration(icp_gpu_ctx* ctx, const float pose_in[16], icp_gpu_timings* timings) {
     if (!pose_in) return ICP_GPU_E_ARG;
     if (int rc = enter(ctx)) return rc;
@@ -254,25 +273,7 @@ static int start_registration(icp_gpu_ctx* ctx, const float pose_in[16], icp_gpu
     const int algo = choose_algorithm(ctx);
     memset(&ctx->stats, 0, sizeof(ctx->stats));
     // descriptors + selection lists + pose up (pinned staging, stream-ordered)
-    memcpy(ctx->h_desc, plan.desc.data(), sizeof(IterDesc) * (size_t)plan.n_iters);
-    if (plan.n_iters > 0) CU(cudaMemcpyAsync(ctx->desc.p, ctx->h_desc, sizeof(IterDesc) * (size_t)plan.n_iters, cudaMemcpyHostToDevice, ctx->stream));
-    if (!plan.voxel_depth.empty()) {
-        const size_t words = mask_words(ctx->n_src);
-        int dmax = 0; for (int D : plan.voxel_depth) dmax = D > dmax ? D : dmax;
-        if (ensure(ctx, ctx->mask, plan.voxel_depth.size() * words * sizeof(uint32_t)) ||
-            ensure(ctx, ctx->voxel_table, sizeof(unsigned int) * ((size_t)1 << dmax))) return ICP_GPU_E_CUDA;
-        int launches = 0;
-        for (size_t j = 0; j < plan.voxel_depth.size(); ++j)
-            CU(icp_launch_voxel_level((const float4*)ctx->src_pts.p, (const float4*)ctx->src_nrm.p, ctx->n_src, (const GridParams*)ctx->sgrid.p,
-                                      ctx->Ts, plan.voxel_depth[j], (unsigned int*)ctx->voxel_table.p, (unsigned int*)ctx->mask.p + j * words,
-                                      words, ctx->stream, &launches));
-        ctx->stats.n_kernel_launches += (uint64_t)launches;
-    }
-    if (!plan.mask.empty()) {
-        if (ensure(ctx, ctx->mask, plan.mask.size() * sizeof(uint32_t))) return ICP_GPU_E_CUDA;
-        CU(cudaMemcpyAsync(ctx->mask.p, plan.mask.data(), plan.mask.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-        CU(cudaStreamSynchronize(ctx->stream));   // plan.mask is pageable and dies with this frame
-    }
+    rc = upload_plan(ctx, plan, (IterDesc*)ctx->desc.p, ctx->mask, true); if (rc) return rc;
     if (upload_pose(ctx, pose_in, ctx->cfg.early_stop_rotation, ctx->cfg.early_stop_translation)) return ICP_GPU_E_CUDA;
     ctx->stats.n_kernel_launches += 1;
     rc = refresh_seeds(ctx, algo, true); if (rc) return rc;

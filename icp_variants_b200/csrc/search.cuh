@@ -90,6 +90,53 @@ __device__ __forceinline__ HandOver load_handover(const HandOver* buf, int p) { 
     HandOver h; h.best.d = __int_as_float(v.x); h.best.idx = v.y; h.best.pos = v.z; h.node = v.w; return h;
 }
 
+// ---------------------------------------------------------------------------- cell codes of the target grid (grid.cu)
+__device__ __forceinline__ int cell_index(const GridParams& g, int a, float x) {
+    const float u = pmul(psub(x, g.o[a]), g.inv_h[a]);
+    int i = (int)floorf(u);
+    const int hi = (1 << g.bits[a]) - 1;
+    return min(max(i, 0), hi);
+}
+
+// The code bits an axis contributes for cell index c: bit j of c lands at bitpos[a][j].
+__device__ __forceinline__ unsigned int axis_spread(const GridParams& g, int a, int c) {
+    unsigned int code = 0;
+#pragma unroll
+    for (int j = 0; j < ICP_MAX_BITS_PER_AXIS; ++j)
+        if (j < g.bits[a]) code |= (((unsigned int)c >> j) & 1u) << g.bitpos[a][j];
+    return code;
+}
+
+__device__ __forceinline__ unsigned int cell_code(const GridParams& g, float x, float y, float z) {
+    return axis_spread(g, 0, cell_index(g, 0, x)) | axis_spread(g, 1, cell_index(g, 1, y)) | axis_spread(g, 2, cell_index(g, 2, z));
+}
+
+// The seed of a query at the transformed position (x, y, z) that remembers no neighbour (seed_from_keys_kernel, grid.cu, and the
+// first iteration of the multi-start kernel): the sorted position of a point of the smallest cell-tree node around the position
+// that holds any point, or -1 (no finite target point, or a non-finite position).  The keys are sorted, so that point is the lower
+// bound of the position's cell code or its predecessor -- whichever shares the longer prefix with the code.  The lower bound is
+// searched inside the bucket of the code's most significant digit (msd_start, a by-product of the last sorting pass).
+__device__ __forceinline__ int key_seed(const GridParams* __restrict__ gp, const unsigned int* __restrict__ keys, int n_finite,
+                                        const unsigned int* __restrict__ msd_start, int msd_shift, float x, float y, float z) {
+    if (!(n_finite > 0 && finite3(x, y, z))) return -1;
+    const GridParams g = *gp;
+    const unsigned int c = cell_code(g, x, y, z);
+    int lo = (int)msd_start[c >> msd_shift], hi = (int)msd_start[(c >> msd_shift) + 1];
+    if (hi > n_finite) hi = n_finite;
+    if (lo > hi) lo = hi;
+    while (lo < hi) {                                   // lower bound of c
+        const int mid = (lo + hi) >> 1;
+        if (keys[mid] < c) lo = mid + 1; else hi = mid;
+    }
+    int pos = lo;
+    if (pos >= n_finite) pos = n_finite - 1;
+    else if (pos > 0) {
+        const unsigned int xa = keys[pos] ^ c, xb = keys[pos - 1] ^ c;
+        if (xb < xa) pos = pos - 1;                     // smaller xor = longer common prefix
+    }
+    return pos;
+}
+
 // Early stop reached: the remaining launches of the registration are no-ops (query_matches, with a fixed descriptor, ignores it).
 __device__ __forceinline__ bool registration_stopped(const MatchArgs& a) { return a.desc_index < 0 && a.state_ro->converged; }
 __device__ __forceinline__ int iter_index(const MatchArgs& a) { return a.desc_index >= 0 ? a.desc_index : a.state_ro->iter; }   // a.desc[...] of this launch

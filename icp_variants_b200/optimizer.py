@@ -270,6 +270,21 @@ class ICPOptimizer:
                 self.last_error.append(f"iteration {n}: singular / non-finite normal equations")
         return list(poses)
 
+    def estimatePoseMultiStart(self, source: PointCloud | None, target: PointCloud | None, initialPoses):
+        """Multi-start registration: estimatePose from every pose of initialPoses [K,4,4] in one launch against one index of the
+        target, each start scored at its final pose by its inliers (the matches that survive the matcher, weighting and rejection)
+        and their RMSE.  Passing None for a cloud reuses the one already resident on the device.  Returns (bestPose, bestIndex,
+        result): the pose of the start with the most inliers (ties to the lower RMSE, then the lower index), its index, and the
+        dict of Context.estimate_pose_multistart (every start's pose, n_iterations, status, inliers, rmse)."""
+        self._ctx.set_config(self.config())
+        if target is not None:
+            self.setTarget(target)
+        if source is not None:
+            self.setSource(source)
+        res = self._ctx.estimate_pose_multistart(initialPoses)
+        best = res["best"]
+        return (res["poses"][best] if best >= 0 else None), best, res
+
     def estimateNormals(self, points, k: int = 5, viewpoint=None):
         """PointCloud(pcl cloud) (PointCloud.h:41-76): k-NN PCA normals of a cloud, computed on the device.  The cloud is
         indexed as the target to do so (set the registration's target afterwards if it is another cloud)."""

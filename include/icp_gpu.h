@@ -251,6 +251,33 @@ int icp_gpu_estimate_pose_batch_configs_dev(icp_gpu_ctx* ctx, int32_t n_configs,
                                             float* poses_out, int32_t* n_iterations_out, int32_t* status_out, float* pose_history,
                                             int32_t history_rows);
 
+/* Multi-start registration: n_starts (K) registrations of the context's source against the context's target, with the context's
+ * configuration, in one launch; start k begins at poses_in[k] (K x 16 floats, column-major).  The target's index is the one
+ * set_target built; every start keeps its own neighbours, so the context's pose, remembered neighbours and graphs are left as they are.
+ * Per start: poses_out[k], n_iterations_out[k] and pose_history (nullable: K x icp_gpu_max_iterations() x 16 floats, rows past a
+ * start's last iteration 0) as icp_gpu_estimate_pose gives them from that start, and status_out[k] = ICP_GPU_OK /
+ * ICP_GPU_E_NO_MATCHES / ICP_GPU_E_NUMERIC, a failed start keeping its last good pose (the call returns OK once the launch ran).
+ * Scoring: after its last iteration each start matches once more at its final pose, every source point (no selection, no stride),
+ * with the configuration's threshold, weighting and rejection -- icp_gpu_query_matches(poses_out[k], NULL).  inliers_out[k] = the
+ * surviving matches; rmse_out[k] = sqrt of the fp64 mean of their D1 squared distances (the 6-D distance with colour ICP; NaN without
+ * an inlier); match_idx_out / match_w_out (nullable, together: K x n_source, original source order) = that call's idx / weight.
+ * n_iterations = 0 makes the call a pose scorer.  Accepted: everything icp_gpu_estimate_pose runs with k-NN matching -- both
+ * minimisers, every metric and weighting, rejection, 3-D or colour 6-D search, select-all / mt19937 / device-stream selection, the
+ * STRIDE and VOXEL pyramids, early stop; nn_algorithm AUTO, BRUTE and GRID all search the index (the same correspondences).
+ * Refused with ICP_GPU_E_ARG: projective matching, ICP_GPU_NN_BRUTE_NORM, attached peers, a null required array, n_starts < 0,
+ * n_starts x n_source above INT32_MAX.  ICP_GPU_E_STATE: no source or target, a pending registration.  n_starts = 0: OK, nothing runs.
+ * Each start runs on a cluster of up to 16 thread blocks (more blocks per start when K is small); its outputs are the same bits
+ * whatever K is.  Where it pays (measured on one B200 at 1000 W, DESIGN.md section 6): subsampled sources of ~10k points, 1.5x a loop
+ * of icp_gpu_estimate_pose at K = 24 and 3x from K = 148 on.  Where it loses: K = 1 (8x slower) and K = 8 (0.76x), and full-size
+ * sources at any K (a loop of icp_gpu_estimate_pose is 1.4x to 18x faster there).
+ * _dev: every array is a device pointer on the context's device.  The call waits for the launch either way. */
+int icp_gpu_estimate_pose_multistart(icp_gpu_ctx* ctx, int32_t n_starts, const float* poses_in, float* poses_out, int32_t* n_iterations_out,
+                                     int32_t* status_out, int64_t* inliers_out, double* rmse_out, float* pose_history, int32_t* match_idx_out,
+                                     float* match_w_out);
+int icp_gpu_estimate_pose_multistart_dev(icp_gpu_ctx* ctx, int32_t n_starts, const float* poses_in, float* poses_out, int32_t* n_iterations_out,
+                                         int32_t* status_out, int64_t* inliers_out, double* rmse_out, float* pose_history, int32_t* match_idx_out,
+                                         float* match_w_out);
+
 int icp_gpu_get_stats(icp_gpu_ctx* ctx, icp_gpu_stats* out);
 /* The FP32 (non-tensor) roofline denominator of the context's device, measured with a register-resident microbenchmark on
  * the context's stream (SURVEY.md 8d; the reference has no counterpart): mode 0 = FFMA (2 flop / instruction), mode 1 =
