@@ -115,6 +115,8 @@ def lib():
             "icp_gpu_estimate_pose_batch_configs_dev": (C.c_int, [vp, i32, C.POINTER(Config), i32, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, i32]),
             "icp_gpu_estimate_pose_multistart": (C.c_int, [vp, i32, pf, pf, pf, pf, pf, pf, pf, pf, pf]),
             "icp_gpu_estimate_pose_multistart_dev": (C.c_int, [vp, i32, pf, pf, pf, pf, pf, pf, pf, pf, pf]),
+            "icp_gpu_estimate_pose_batch_indexed": (C.c_int, [vp, i32, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, i32, pf, pf]),
+            "icp_gpu_estimate_pose_batch_indexed_dev": (C.c_int, [vp, i32, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, pf, i32, pf, pf]),
             "icp_gpu_get_stats": (C.c_int, [vp, C.POINTER(Stats)]),
             "icp_gpu_measure_fp32_peak": (C.c_int, [vp, i32, C.POINTER(C.c_double)]),
             "icp_gpu_alignment_error": (C.c_int, [vp, pf, pf, C.POINTER(C.c_double)]),
@@ -227,6 +229,18 @@ def _concat_clouds(clouds):
     if n3 is not None and len(n3) != len(xyz):
         raise ValueError("every cloud needs one normal per point")
     return xyz, n3, off
+
+
+def _concat_clouds_rgba(clouds):
+    """_concat_clouds plus the colours: (points, normals or None, colours [N,4] uint8 or None, offsets)."""
+    xyz, n3, off = _concat_clouds(clouds)
+    cols = [getattr(c, "colors", None) for c in clouds]
+    if all(c is None for c in cols):
+        return xyz, n3, None, off
+    rgba = np.concatenate([np.zeros((off[b + 1] - off[b], 4), np.uint8) if c is None else _u8(c) for b, c in enumerate(cols)])
+    if len(rgba) != len(xyz):
+        raise ValueError("every cloud needs one colour per point")
+    return xyz, n3, rgba, off
 
 
 def _batch_poses(poses, B):
@@ -552,6 +566,87 @@ class Context:
         if want_matches:
             out["match_idx"], out["match_w"] = midx[:, :n], mw[:, :n]
         return out
+
+    # -- many pairs of any size, each against its own index, in one launch
+    def estimate_pose_batch_indexed(self, sources, targets, init_poses=None, want_history=False, want_matches=False):
+        """B independent registrations with the context's configuration, every target indexed in the call, pairs of any size.
+        sources / targets: sequences of synth.Cloud (points, optional normals and colours) or [N,3] point arrays; init_poses:
+        [B,4,4] or None (identity).  Returns the dict of estimate_pose_multistart with one row per pair: poses, n_iterations,
+        status, inliers, rmse, best, and with want_history history [B, R, 4, 4] (R = the largest iterations_bound of the batch's
+        sources, rows past a pair's last iteration 0), with want_matches match_idx / match_w: one array per pair (query_matches at
+        its final pose).  The context's own clouds and state are left as they are."""
+        if len(sources) != len(targets):
+            raise ValueError(f"{len(sources)} sources, {len(targets)} targets")
+        B = len(sources)
+        sp, sn, sc, so = _concat_clouds_rgba(sources)
+        tp, tn, tc, to = _concat_clouds_rgba(targets)
+        pin = _batch_poses(init_poses, B)
+        pout = np.zeros((B, 16), np.float32)
+        n_it = np.zeros(B, np.int32)
+        status = np.zeros(B, np.int32)
+        inl = np.zeros(B, np.int64)
+        rmse = np.zeros(B, np.float64)
+        cfg = self.get_config()
+        rows = max([iterations_bound(cfg, so[b + 1] - so[b]) for b in range(B)] + [0]) if want_history else 0
+        hist = np.zeros((B, max(rows, 1), 16), np.float32) if want_history else None
+        ns = int(so[-1])
+        midx = np.zeros(max(ns, 1), np.int32) if want_matches else None
+        mw = np.zeros(max(ns, 1), np.float32) if want_matches else None
+        self._check(lib().icp_gpu_estimate_pose_batch_indexed(self._h, B, _ptr(sp), _ptr(sn), _ptr(sc), _ptr(so), _ptr(tp), _ptr(tn), _ptr(tc), _ptr(to),
+                                                              _ptr(pin), _ptr(pout), _ptr(n_it), _ptr(status), _ptr(inl), _ptr(rmse), _ptr(hist), rows,
+                                                              _ptr(midx), _ptr(mw)))
+        out = {"poses": pout.reshape(B, 4, 4).transpose(0, 2, 1).copy(), "n_iterations": n_it, "status": status, "inliers": inl,
+               "rmse": rmse, "best": best_start(inl, rmse)}
+        if want_history:
+            out["history"] = hist[:, :rows].reshape(B, rows, 4, 4).transpose(0, 1, 3, 2).copy()
+        if want_matches:
+            out["match_idx"] = [midx[so[b]:so[b + 1]].copy() for b in range(B)]
+            out["match_w"] = [mw[so[b]:so[b + 1]].copy() for b in range(B)]
+        return out
+
+    def estimate_pose_batch_indexed_dev(self, src_xyz, src_off, tgt_xyz, tgt_off, src_nrm=None, tgt_nrm=None, src_rgba=None, tgt_rgba=None,
+                                        init_poses=None, want_history=False, want_matches=False):
+        """The same on CUDA torch tensors of the context's device: concatenated points / normals [N,3] float32, colours [N,4] uint8,
+        offsets [B+1] int64, init_poses [B,4,4] float32 (None = identity).  Returns the dict with CUDA tensors (best a Python int);
+        match_idx / match_w are [sum n_src] tensors in each pair's original order, pair b's at src_off[b].  Work queued on the
+        current torch stream is waited for; the results are complete when the call returns."""
+        import torch
+        dev = torch.device("cuda", self.device)
+
+        def rgba(x, name, n):
+            if x is None:
+                return None
+            if not (isinstance(x, torch.Tensor) and x.device == dev and x.dtype == torch.uint8 and tuple(x.shape) == (n, 4)):
+                raise ValueError(f"{name}: expected a uint8 [{n},4] tensor on {dev}")
+            return x.contiguous()
+
+        sc, tc = rgba(src_rgba, "src_rgba", len(src_xyz)), rgba(tgt_rgba, "tgt_rgba", len(tgt_xyz))
+        cfg = self.get_config()
+        res = {}
+
+        def run(sp, sn, so, tp, tn, to, pin, pout, n_it, status, p):
+            B = len(so) - 1
+            ns = int(so[-1]) if B > 0 else 0
+            inl = torch.empty(B, dtype=torch.int64, device=dev)
+            rmse = torch.empty(B, dtype=torch.float64, device=dev)
+            rows = 0
+            if want_history:
+                rows = max([iterations_bound(cfg, n) for n in (so[1:] - so[:-1]).tolist()] + [0])
+            hist = torch.zeros((B, max(rows, 1), 4, 4), dtype=torch.float32, device=dev) if want_history else None
+            midx = torch.empty(max(ns, 1), dtype=torch.int32, device=dev) if want_matches else None
+            mw = torch.empty(max(ns, 1), dtype=torch.float32, device=dev) if want_matches else None
+            self._check(lib().icp_gpu_estimate_pose_batch_indexed_dev(self._h, B, p(sp), p(sn), p(sc), p(so), p(tp), p(tn), p(tc), p(to), p(pin), p(pout),
+                                                                      p(n_it), p(status), p(inl), p(rmse), p(hist), rows, p(midx), p(mw)))
+            res.update(inliers=inl, rmse=rmse, best=best_start(inl.cpu().numpy(), rmse.cpu().numpy()))
+            if want_matches:
+                res.update(match_idx=midx[:ns], match_w=mw[:ns])
+            return hist[:, :rows] if want_history else None
+
+        out = self._batch_dev(run, src_xyz, src_off, tgt_xyz, tgt_off, src_nrm, tgt_nrm, init_poses)
+        res.update(poses=out[0], n_iterations=out[1], status=out[2])
+        if want_history:
+            res["history"] = out[3]
+        return res
 
     def cloud_from_depth(self, depth, rgbx, K, extrinsics=None, keep_original_size=False, downsample=1, max_distance=0.1,
                          role: int = 2, download: bool = True):

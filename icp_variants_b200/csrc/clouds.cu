@@ -2,7 +2,7 @@
 // and PCA normals of the target.  Host code only; the kernels live in grid.cu, prep.cu and normals.cu.
 #include "context.cuh"
 
-static int pick_T(int n, bool source = false) {
+int pick_T(int n, bool source) {
     // Target: the finest grid the 32-bit keys hold (10 bits per axis) -- the radix sort costs the same for any T, and fine
     // cells give compact leaves.  Source: 4 cells per point; its grid also defines the voxel pyramid levels, which the
     // oracle restates (oracle/icp_oracle.c:orc_pick_T).
@@ -20,6 +20,50 @@ static int ensure_sort(icp_gpu_ctx* ctx, icp_gpu_ctx::SortBufs& sb, int n, int T
     return 0;
 }
 
+// The context's buffers of one cloud as a CloudBufs (kind 0: the target with its index, 1: the source).
+static CloudBufs context_bufs(icp_gpu_ctx* ctx, int kind) {
+    CloudBufs b; memset(&b, 0, sizeof(b));
+    icp_gpu_ctx::SortBufs& sb = kind == 0 ? ctx->tsort : ctx->ssort;
+    b.pts = (float4*)(kind == 0 ? ctx->tgt_pts.p : ctx->src_raw_pts.p); b.nrm = (float4*)(kind == 0 ? ctx->tgt_nrm.p : ctx->src_raw_nrm.p);
+    b.bbox = (unsigned int*)(kind == 0 ? ctx->bbox.p : ctx->sbbox.p); b.grid = (GridParams*)(kind == 0 ? ctx->grid.p : ctx->sgrid.p);
+    b.keys_a = (unsigned int*)sb.keys_a.p; b.keys_b = (unsigned int*)sb.keys_b.p; b.idx_a = (unsigned int*)sb.idx_a.p; b.idx_b = (unsigned int*)sb.idx_b.p;
+    b.hist = (unsigned int*)sb.hist.p; b.msd = kind == 0 ? (unsigned int*)sb.msd.p : nullptr;
+    b.pts_sorted = (float4*)(kind == 0 ? ctx->tgt_pts_sorted.p : ctx->src_pts.p); b.nrm_sorted = (float4*)(kind == 0 ? ctx->tgt_nrm_sorted.p : ctx->src_nrm.p);
+    if (kind == 0) {
+        b.lv_flags = (unsigned char*)ctx->lv_flags.p; b.lv_tiles = (unsigned int*)ctx->lv_tiles.p; b.delta_a = (int*)ctx->delta_a.p; b.delta_b = (int*)ctx->delta_b.p;
+        b.leaf_start = (unsigned int*)ctx->leaf_start.p; b.leaf_rank = (unsigned int*)ctx->leaf_rank.p; b.node_rank = (unsigned int*)ctx->node_rank.p;
+        b.child_start = (unsigned int*)ctx->child_start.p; b.bvh_desc = (BvhDesc*)ctx->bvh_desc.p; b.bvh_box = (float4*)ctx->bvh_box.p;
+        b.adj = (unsigned int*)ctx->adj.p; b.adj_box = (float4*)ctx->adj_box.p; b.adj_gap = (float*)ctx->adj_gap.p; b.adj_capacity = ctx->adj_capacity;
+        b.adj1 = (unsigned int*)ctx->adj1.p; b.adj1_box = (float4*)ctx->adj1_box.p; b.adj1_capacity = ctx->adj1_capacity;
+    }
+    b.keys_sorted = sb.keys_sorted; b.msd_shift = sb.msd_shift;
+    return b;
+}
+
+int pack_cloud(icp_gpu_ctx* ctx, CloudBufs& b, const float* xyz, const float* nrm, const uint8_t* rgba, int n, int T, bool with_normals) {
+    const long long hist_words = (long long)icp_radix_hist_words(n, T);
+    if (n == 0) CU(icp_launch_pack_cloud(nullptr, nullptr, nullptr, 0, b.pts, b.nrm, b.bbox, T, b.grid, b.hist, hist_words, 1, ctx->stream));
+    else CU(icp_launch_pack_cloud(xyz, nrm, rgba, n, b.pts, b.nrm, b.bbox, T, b.grid, b.hist, hist_words, with_normals ? 1 : 0, ctx->stream));
+    return 0;
+}
+
+int sort_cloud(icp_gpu_ctx* ctx, CloudBufs& b, int n, int T, const IcpLatePack* late, int* launches) {
+    CU(icp_launch_cloud_sort(b.pts, b.nrm, n, T, b.grid, b.keys_a, b.keys_b, b.idx_a, b.idx_b, b.hist, b.pts_sorted, b.nrm_sorted, b.msd,
+                             &b.keys_sorted, &b.msd_shift, late, ctx->stream, launches));
+    return 0;
+}
+
+// The index over a sorted target (after sort_cloud): tree levels, tight boxes, adjacency lists, on stream s.
+int build_tree(icp_gpu_ctx* ctx, const CloudBufs& b, int n, int T, cudaStream_t s, int* launches) {
+    CU(icp_launch_bvh_build(b.pts_sorted, b.nrm_sorted, n, T, b.keys_sorted, b.bbox + 7, b.lv_flags, b.lv_tiles, b.delta_a, b.delta_b, b.leaf_rank,
+                            b.leaf_start, b.node_rank, b.child_start, b.bvh_desc, b.bvh_box, ctx->n_sms, s, launches));
+    CU(icp_launch_leaf_adjacency(b.bvh_desc, b.bvh_box, b.child_start, b.adj1, b.adj1_box, b.adj1_capacity, 1, nullptr, nullptr, nullptr, 0, ctx->n_sms, s,
+                                 launches, nullptr));
+    CU(icp_launch_leaf_adjacency(b.bvh_desc, b.bvh_box, b.child_start, b.adj, b.adj_box, b.adj_capacity, 0, b.node_rank, b.adj1, b.adj1_box,
+                                 b.adj1_capacity, ctx->n_sms, s, launches, b.adj_gap));
+    return 0;
+}
+
 static int upload_cloud(icp_gpu_ctx* ctx, const float* xyz, const float* nrm, const uint8_t* rgba, int64_t n, bool device_ptrs,
                         DeviceBuf& pts, DeviceBuf& nrmb, int kind /*0 target, 1 source*/) {
     const size_t n1 = (size_t)(n > 0 ? n : 1);
@@ -31,10 +75,9 @@ static int upload_cloud(icp_gpu_ctx* ctx, const float* xyz, const float* nrm, co
     if (kind == 0) ctx->T = T; else ctx->Ts = T;
     if (ensure(ctx, pts, n1 * sizeof(float4)) || ensure(ctx, nrmb, n1 * sizeof(float4)) || ensure(ctx, bbox, 64) || ensure(ctx, grid, sizeof(GridParams)) ||
         ensure_sort(ctx, sb, (int)n, T)) return ICP_GPU_E_CUDA;
-    const long long hist_words = (long long)icp_radix_hist_words((int)n, T);
+    CloudBufs b = context_bufs(ctx, kind);
     if (n == 0) {
-        CU(icp_launch_pack_cloud(nullptr, nullptr, nullptr, 0, (float4*)pts.p, (float4*)nrmb.p, (unsigned int*)bbox.p, T, (GridParams*)grid.p,
-                                 (unsigned int*)sb.hist.p, hist_words, 1, ctx->stream));
+        if (pack_cloud(ctx, b, nullptr, nullptr, nullptr, 0, T, true)) return ICP_GPU_E_CUDA;
         ctx->late_pending[kind] = false;
         return 0;
     }
@@ -59,8 +102,7 @@ static int upload_cloud(icp_gpu_ctx* ctx, const float* xyz, const float* nrm, co
         ctx->late[kind].nrm = dn; ctx->late[kind].rgba = dc; ctx->late[kind].nrmo = (float4*)nrmb.p; ctx->late[kind].ready = ctx->ev_copied[kind];
     }
     ctx->late_pending[kind] = !device_ptrs;
-    CU(icp_launch_pack_cloud(dx, dn, dc, (int)n, (float4*)pts.p, (float4*)nrmb.p, (unsigned int*)bbox.p, T, (GridParams*)grid.p,
-                             (unsigned int*)sb.hist.p, hist_words, device_ptrs ? 1 : 0, ctx->stream));
+    if (pack_cloud(ctx, b, dx, dn, dc, (int)n, T, device_ptrs)) return ICP_GPU_E_CUDA;
     ctx->stats.n_kernel_launches += 1;
     return 0;
 }
@@ -77,9 +119,8 @@ static int build_grid(icp_gpu_ctx* ctx) {
         ensure(ctx, ctx->node_rank, (icp_bvh_max_nodes(n) + ICP_BVH_MAX_LEVELS) * 4) ||
         ensure(ctx, ctx->child_start, (icp_bvh_max_nodes(n) + ICP_BVH_MAX_LEVELS) * 4))
         return ICP_GPU_E_CUDA;
-    // adjacency lists for up to n/4 leaves (a healthy tree has ~n/20); a cloud with more leaves simply gets no shortcut for the rest
-    ctx->adj_capacity = (int)(n1 / 4 + 64);
-    ctx->adj1_capacity = (int)(n1 / 32 + 64);
+    ctx->adj_capacity = adj_capacity_for(n);
+    ctx->adj1_capacity = adj1_capacity_for(n);
     if (ensure(ctx, ctx->adj, (size_t)ctx->adj_capacity * 32 * 4) || ensure(ctx, ctx->adj_gap, (size_t)ctx->adj_capacity * 32 * 4) ||
         ensure(ctx, ctx->adj_box, (size_t)ctx->adj_capacity * 2 * sizeof(float4)) ||
         ensure(ctx, ctx->adj1, (size_t)ctx->adj1_capacity * 32 * 4) || ensure(ctx, ctx->adj1_box, (size_t)ctx->adj1_capacity * 2 * sizeof(float4)))
@@ -87,25 +128,13 @@ static int build_grid(icp_gpu_ctx* ctx) {
     int launches = 0;
     if (join_index(ctx)) return ICP_GPU_E_CUDA;              // a build still running on aux_stream reads what this one overwrites
     CU(cudaEventRecord(ctx->ev[0], ctx->stream));
-    CU(icp_launch_cloud_sort((const float4*)ctx->tgt_pts.p, (const float4*)ctx->tgt_nrm.p, n, ctx->T, (const GridParams*)ctx->grid.p,
-                             (unsigned int*)ctx->tsort.keys_a.p, (unsigned int*)ctx->tsort.keys_b.p, (unsigned int*)ctx->tsort.idx_a.p,
-                             (unsigned int*)ctx->tsort.idx_b.p, (unsigned int*)ctx->tsort.hist.p, (float4*)ctx->tgt_pts_sorted.p,
-                             (float4*)ctx->tgt_nrm_sorted.p, (unsigned int*)ctx->tsort.msd.p, &ctx->tsort.keys_sorted, &ctx->tsort.msd_shift,
-                             ctx->late_pending[0] ? &ctx->late[0] : nullptr, ctx->stream, &launches));
+    CloudBufs b = context_bufs(ctx, 0);
+    if (sort_cloud(ctx, b, n, ctx->T, ctx->late_pending[0] ? &ctx->late[0] : nullptr, &launches)) return ICP_GPU_E_CUDA;
+    ctx->tsort.keys_sorted = b.keys_sorted; ctx->tsort.msd_shift = b.msd_shift;
     if (ctx->late_pending[0]) { CU(cudaEventRecord(ctx->ev_packed[0], ctx->stream)); ctx->packed_once[0] = true; ctx->late_pending[0] = false; }
     cudaStream_t ts = ctx->aux_stream;
     CU(cudaEventRecord(ctx->ev_fork, ctx->stream)); CU(cudaStreamWaitEvent(ts, ctx->ev_fork, 0));
-    CU(icp_launch_bvh_build((float4*)ctx->tgt_pts_sorted.p, (float4*)ctx->tgt_nrm_sorted.p, n, ctx->T, ctx->tsort.keys_sorted,
-                            (const unsigned int*)ctx->bbox.p + 7, (unsigned char*)ctx->lv_flags.p, (unsigned int*)ctx->lv_tiles.p, (int*)ctx->delta_a.p,
-                            (int*)ctx->delta_b.p, (unsigned int*)ctx->leaf_rank.p, (unsigned int*)ctx->leaf_start.p, (unsigned int*)ctx->node_rank.p,
-                            (unsigned int*)ctx->child_start.p, (BvhDesc*)ctx->bvh_desc.p, (float4*)ctx->bvh_box.p, ctx->n_sms, ts, &launches));
-    CU(icp_launch_leaf_adjacency((const BvhDesc*)ctx->bvh_desc.p, (const float4*)ctx->bvh_box.p, (const unsigned int*)ctx->child_start.p,
-                                 (unsigned int*)ctx->adj1.p, (float4*)ctx->adj1_box.p, ctx->adj1_capacity, 1, nullptr, nullptr, nullptr, 0, ctx->n_sms, ts, &launches,
-                                 nullptr));
-    CU(icp_launch_leaf_adjacency((const BvhDesc*)ctx->bvh_desc.p, (const float4*)ctx->bvh_box.p, (const unsigned int*)ctx->child_start.p,
-                                 (unsigned int*)ctx->adj.p, (float4*)ctx->adj_box.p, ctx->adj_capacity, 0, (const unsigned int*)ctx->node_rank.p,
-                                 (const unsigned int*)ctx->adj1.p, (const float4*)ctx->adj1_box.p, ctx->adj1_capacity, ctx->n_sms, ts, &launches,
-                                 (float*)ctx->adj_gap.p));
+    if (build_tree(ctx, b, n, ctx->T, ts, &launches)) return ICP_GPU_E_CUDA;
     CU(cudaEventRecord(ctx->ev[1], ts));
     CU(cudaEventRecord(ctx->ev_index_ready, ts)); ctx->index_pending = true;
     ctx->stats.n_kernel_launches += (uint64_t)launches;
@@ -119,11 +148,9 @@ static int build_source(icp_gpu_ctx* ctx) {
     const size_t n1 = (size_t)(n > 0 ? n : 1);
     if (ensure(ctx, ctx->src_pts, n1 * sizeof(float4)) || ensure(ctx, ctx->src_nrm, n1 * sizeof(float4))) return ICP_GPU_E_CUDA;
     int launches = 0;
-    CU(icp_launch_cloud_sort((const float4*)ctx->src_raw_pts.p, (const float4*)ctx->src_raw_nrm.p, n, ctx->Ts, (const GridParams*)ctx->sgrid.p,
-                             (unsigned int*)ctx->ssort.keys_a.p, (unsigned int*)ctx->ssort.keys_b.p, (unsigned int*)ctx->ssort.idx_a.p,
-                             (unsigned int*)ctx->ssort.idx_b.p, (unsigned int*)ctx->ssort.hist.p, (float4*)ctx->src_pts.p,
-                             (float4*)ctx->src_nrm.p, nullptr, &ctx->ssort.keys_sorted, &ctx->ssort.msd_shift,
-                             ctx->late_pending[1] ? &ctx->late[1] : nullptr, ctx->stream, &launches));
+    CloudBufs b = context_bufs(ctx, 1);
+    if (sort_cloud(ctx, b, n, ctx->Ts, ctx->late_pending[1] ? &ctx->late[1] : nullptr, &launches)) return ICP_GPU_E_CUDA;
+    ctx->ssort.keys_sorted = b.keys_sorted; ctx->ssort.msd_shift = b.msd_shift;
     if (ctx->late_pending[1]) { CU(cudaEventRecord(ctx->ev_packed[1], ctx->stream)); ctx->packed_once[1] = true; ctx->late_pending[1] = false; }
     ctx->stats.n_kernel_launches += (uint64_t)launches;
     return 0;

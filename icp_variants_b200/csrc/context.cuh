@@ -62,6 +62,7 @@ struct icp_gpu_ctx {
     DeviceBuf scratch[16];                                   // operands of the value-level entry points (transform, weights, solve)
     DeviceBuf batch_io, batch_scratch, batch_plan;           // batched registration: uploaded operands + results, match slices, configs + pair lists + masks
     DeviceBuf ms_io, ms_nn, ms_scratch, ms_desc, ms_mask;    // multi-start registration: operands + results, per-(start, query) neighbours and match slices, plan
+    DeviceBuf bi_io, bi_arena, bi_scratch, bi_plan;          // indexed batch: operands + results, per-pair clouds and indices, build scratch, plans + pair table
     long long n_gt = 0; int last_iters = 0;
     float* h_pose = nullptr; float* h_history = nullptr; DevState* h_state = nullptr;   // pinned
     IterDesc* h_desc = nullptr;                                                       // pinned, DESC_TOTAL
@@ -131,6 +132,29 @@ inline bool point_finite(const float* p, const float* m) {
     return isfinite(p[0]) && isfinite(p[1]) && isfinite(p[2]) && (!m || (isfinite(m[0]) && isfinite(m[1]) && isfinite(m[2])));
 }
 
+// Where one cloud's build writes: the packed records, the grid and the sort, and for a target its index (grid.cu's launchers).  The
+// context's clouds point it at their own buffers; the indexed batch at one pair's slices of its arena and at scratch the pairs share.
+struct CloudBufs {
+    float4 *pts, *nrm;                                       // packed records, upload order
+    unsigned int* bbox; GridParams* grid;                    // 8 words ([7]: points with a non-finite coordinate); the grid
+    unsigned int *keys_a, *keys_b, *idx_a, *idx_b, *hist, *msd;   // the sort (msd null: no MSD table)
+    float4 *pts_sorted, *nrm_sorted;
+    unsigned char* lv_flags; unsigned int* lv_tiles; int *delta_a, *delta_b;    // the index: tree scratch, then the tree
+    unsigned int *leaf_start, *leaf_rank, *node_rank, *child_start; BvhDesc* bvh_desc; float4* bvh_box;
+    unsigned int *adj, *adj1; float4 *adj_box, *adj1_box; float* adj_gap; int adj_capacity, adj1_capacity;
+    unsigned int* keys_sorted; int msd_shift;                // set by sort_cloud: keys_a or keys_b, and the MSD table's shift
+};
+// Adjacency capacities of a target of n points: lists for up to n/4 leaves (a healthy tree has ~n/20) and n/32 level-1 nodes; a
+// cloud with more simply gets no shortcut for the rest.
+inline int adj_capacity_for(int n) { return (n > 0 ? n : 1) / 4 + 64; }
+inline int adj1_capacity_for(int n) { return (n > 0 ? n : 1) / 32 + 64; }
+
+int pick_T(int n, bool source);                                                                                            // clouds.cu
+// AoS3 (device arrays; n = 0: nothing) -> b.pts / b.nrm, b.bbox, b.grid; clears b.hist for the sort.  with_normals = false: the
+// normal records follow through the sort's IcpLatePack.
+int pack_cloud(icp_gpu_ctx* ctx, CloudBufs& b, const float* xyz, const float* nrm, const uint8_t* rgba, int n, int T, bool with_normals); // clouds.cu
+int sort_cloud(icp_gpu_ctx* ctx, CloudBufs& b, int n, int T, const IcpLatePack* late, int* launches);                     // clouds.cu
+int build_tree(icp_gpu_ctx* ctx, const CloudBufs& b, int n, int T, cudaStream_t s, int* launches);                        // clouds.cu
 int check_config(icp_gpu_ctx* ctx, const icp_gpu_config* c, const char* who);                                          // context.cu
 int set_cloud(icp_gpu_ctx* ctx, bool target, const float* xyz, const float* nrm, const uint8_t* rgba, int64_t n, bool dev);  // clouds.cu
 int fetch_src_rank(icp_gpu_ctx* ctx);                                                                                      // clouds.cu
@@ -141,6 +165,13 @@ int check_ready(icp_gpu_ctx* ctx);                                              
 void fill_match_args(icp_gpu_ctx* c, MatchArgs& a, int algo, int desc_index, bool want_idx);                               // registration.cu
 void fill_reduce_args(icp_gpu_ctx* c, ReduceArgs& r, int algo, int solve);                                                 // registration.cu
 int refresh_seeds(icp_gpu_ctx* ctx, int algo, bool allow_seed);                                                            // registration.cu
+// The plan of a registration with cfg of a source of n points whose grid has depth Ts; finite: its "point and normal finite" flags
+// per original index (read with mt19937 selection and multires only).
+int plan_iterations(icp_gpu_ctx* ctx, const icp_gpu_config& cfg, int n, int Ts, const uint8_t* finite, Plan& plan);    // registration.cu
 int make_plan(icp_gpu_ctx* ctx, Plan& plan);                                                                               // registration.cu
 int upload_plan(icp_gpu_ctx* ctx, const Plan& plan, IterDesc* desc, DeviceBuf& mask, bool graph_reads);                   // registration.cu
+// The plan's voxel pyramid levels of the sorted source (src_pts / src_nrm, its grid of depth Ts) into mask (slot j at j * words);
+// table: scratch of 2^(deepest level) entries.
+int build_voxel_levels(icp_gpu_ctx* ctx, const Plan& plan, const float4* src_pts, const float4* src_nrm, int n, const GridParams* grid, int Ts,
+                       unsigned int* table, unsigned int* mask, size_t words);                                             // registration.cu
 void peer_close(icp_gpu_ctx* ctx);                                                                                         // sharded.cu

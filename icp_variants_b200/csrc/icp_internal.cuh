@@ -261,10 +261,12 @@ struct BatchArgs {
 // metric: ICP_GPU_METRIC_*, lm: the minimiser; pairs: n_pairs block indices in device memory (BatchArgs::pairs)
 cudaError_t icp_launch_batch(const BatchArgs& a, int metric, int lm, int n_pairs, int max_tgt, cudaStream_t s);
 
-// multistart.cu: K registrations of the context's source against its indexed target, one thread-block cluster per start
+// multistart.cu: K registrations of the context's source against its indexed target, one thread-block cluster per start; or B pairs,
+// each against its own index (icp_gpu_estimate_pose_batch_indexed), one cluster per pair
 #define ICP_MS_THREADS 256       // threads per block (the LM jets need up to 255 registers a thread); also the tile: 256 sorted positions
 #define ICP_MS_SLICES 16         // tile t is summed into slice t mod 16, the slices in order: the largest cluster
-struct MsArgs {
+// What one cluster reads of its pair: the clouds, the index, the first-iteration seeds and the plan.
+struct MsPair {
     const float4* src_pts; const float4* src_nrm; int n_src;           // sorted source (MatchArgs)
     const float4* tgt_pts; const float4* tgt_nrm; int n_tgt;           // target in grid order
     const float4* bvh_box; const BvhDesc* bvh; const unsigned int* leaf_start; const unsigned int* leaf_rank; const unsigned int* child_start;
@@ -272,18 +274,25 @@ struct MsArgs {
     // the first-iteration seeds (key_seed, search.cuh)
     const GridParams* grid; const unsigned int* keys; const unsigned int* msd_start; int msd_shift; const unsigned int* nonfinite;
     const IterDesc* desc; const unsigned int* mask; int n_iters;      // the plan of make_plan (registration.cu)
+    float max_d2;                                                      // the matching threshold (the configuration's; the search reads it here)
+    long long q_off;                                                   // batch: the pair's first entry of nn_pos, scratch and the matches
+};
+struct MsArgs : MsPair {                                               // multi-start: the one pair; the batch reads pairs[] instead
     int weighting, rejection, lm_max_iterations;
-    float max_d2, weight_max_d2, stop_rot, stop_trans;
+    float weight_max_d2, stop_rot, stop_trans;
     const float* poses_in; float* poses_out; int* n_iter_out; int* status_out;   // [K][16] column-major, [K], [K]
     long long* inliers_out; double* rmse_out;                          // the scoring pass, [K]
     float* history; int history_rows;                                  // [K][history_rows][16] or null
-    int* match_idx; float* match_w;                                    // [K][n_src] in original source order, or null
+    int* match_idx; float* match_w;                                    // [K][n_src] in original source order, or null (batch: [sum n_src])
     int* nn_pos;                                                       // [K][n_src]: last neighbour of (start, sorted position), -1 = none
     int2* scratch;                                                     // [K][n_src] symmetric metric and LM: {target position or -1, weight bits}
+    const MsPair* pairs; const int* order;                             // batch: cluster k registers pair order[k], described by pairs[order[k]]
 };
-// lm: the minimiser; metric: ICP_GPU_METRIC_*; color: 6-D search.  The cluster size (blocks per start) is chosen from n_starts and the
-// SM count and returned in *cluster.
-cudaError_t icp_launch_multistart(const MsArgs& a, int lm, int metric, int color, int n_starts, int n_sms, cudaStream_t s, int* cluster);
+// batch: one cluster per pair of a.pairs (n_clusters of them), else one per start of the MsArgs' own pair; lm: the minimiser; metric:
+// ICP_GPU_METRIC_*; color: 6-D search.  The cluster size (blocks per cluster) is chosen from n_clusters, the largest source (max_src)
+// and the SM count and returned in *cluster.
+cudaError_t icp_launch_multistart(const MsArgs& a, bool batch, int lm, int metric, int color, int n_clusters, int max_src, int n_sms, cudaStream_t s,
+                                  int* cluster);
 
 // standalone.cu: the reference API's value-level operations outside the loop
 cudaError_t icp_launch_transform(const float* in, long long n, const float pose16[16], int normals, float* out, cudaStream_t s);

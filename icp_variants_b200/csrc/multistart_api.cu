@@ -68,7 +68,7 @@ static int estimate_pose_multistart(icp_gpu_ctx* ctx, int32_t n_starts, const fl
     }
     if (hist_floats) CU(cudaMemsetAsync(a.history, 0, hist_floats * 4, ctx->stream));   // rows past a start's last iteration read 0
     int cluster = 1;
-    CU(icp_launch_multistart(a, lm ? 1 : 0, cfg.metric, cfg.color_icp ? 1 : 0, n_starts, ctx->n_sms, ctx->stream, &cluster));
+    CU(icp_launch_multistart(a, false, lm ? 1 : 0, cfg.metric, cfg.color_icp ? 1 : 0, n_starts, n, ctx->n_sms, ctx->stream, &cluster));
     ctx->stats.n_kernel_launches += 1;
     if (!dev) {
         CU(cudaMemcpyAsync(poses_out, a.poses_out, K * 64, cudaMemcpyDeviceToHost, ctx->stream));

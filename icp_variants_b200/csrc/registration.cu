@@ -85,19 +85,16 @@ int check_ready(icp_gpu_ctx* ctx) {
 }
 
 // The iteration schedule of estimatePose (ICPOptimizer.h:503-525, :540, :549-550, :634-655; Appendix A of SURVEY.md).
-int make_plan(icp_gpu_ctx* ctx, Plan& plan) {
-    const icp_gpu_config& cfg = ctx->cfg;
-    const int n = ctx->n_src;
+int plan_iterations(icp_gpu_ctx* ctx, const icp_gpu_config& cfg, int n, int Ts, const uint8_t* finite, Plan& plan) {
     const bool host_rng = cfg.selection == ICP_GPU_SELECT_RANDOM && cfg.selection_rng == ICP_GPU_RNG_MT19937;
     const bool dev_rng = cfg.selection == ICP_GPU_SELECT_RANDOM && cfg.selection_rng == ICP_GPU_RNG_DEVICE;
-    if (host_rng && cfg.multires && fetch_src_finite(ctx)) return ICP_GPU_E_CUDA;
     const size_t words = mask_words(n);
     const bool voxel = cfg.multires && cfg.pyramid_mode == ICP_GPU_PYRAMID_VOXEL;
     const IcpSchedule sch = icp_schedule(cfg.n_iterations, cfg.multires, n);
     if (sch.n_iters > ICP_MAX_ITERS) return fail(ctx, ICP_GPU_E_ARG, "more than %d iterations", ICP_MAX_ITERS);
     if (host_rng) {
         plan.mask.assign((size_t)sch.n_iters * words, 0u);
-        draw_selection_masks(cfg, sch, n, ctx->src_finite.data(), plan.mask.data());
+        draw_selection_masks(cfg, sch, n, finite, plan.mask.data());
     }
     for (int i = 0; i < sch.n_iters; ++i) {
         const int stride = icp_schedule_stride(sch, i);
@@ -106,7 +103,7 @@ int make_plan(icp_gpu_ctx* ctx, Plan& plan) {
         if (voxel && stride > 1) {
             // level = one point per occupied source-grid cell at depth Ts' - ceil(1.5 log2 stride)
             int k = 0; while ((1 << k) < stride) ++k;
-            int D = (ctx->Ts < 22 ? ctx->Ts : 22) - (3 * k + 1) / 2; if (D < 0) D = 0;
+            int D = (Ts < 22 ? Ts : 22) - (3 * k + 1) / 2; if (D < 0) D = 0;
             int slot = -1;
             for (size_t j = 0; j < plan.voxel_depth.size(); ++j) if (plan.voxel_depth[j] == D) slot = (int)j;
             if (slot < 0) { slot = (int)plan.voxel_depth.size(); plan.voxel_depth.push_back(D); }
@@ -118,6 +115,12 @@ int make_plan(icp_gpu_ctx* ctx, Plan& plan) {
     }
     plan.n_iters = sch.n_iters;
     return 0;
+}
+
+int make_plan(icp_gpu_ctx* ctx, Plan& plan) {
+    const icp_gpu_config& cfg = ctx->cfg;
+    if (cfg.selection == ICP_GPU_SELECT_RANDOM && cfg.selection_rng == ICP_GPU_RNG_MT19937 && cfg.multires && fetch_src_finite(ctx)) return ICP_GPU_E_CUDA;
+    return plan_iterations(ctx, cfg, ctx->n_src, ctx->Ts, ctx->src_finite.data(), plan);
 }
 
 // Projective matching of a full-frame source (one point per pixel of the camera the target was taken with): the kernels
@@ -232,6 +235,15 @@ static int enqueue_iterations(icp_gpu_ctx* ctx, const Plan& plan, int algo, std:
     return 0;
 }
 
+int build_voxel_levels(icp_gpu_ctx* ctx, const Plan& plan, const float4* src_pts, const float4* src_nrm, int n, const GridParams* grid, int Ts,
+                       unsigned int* table, unsigned int* mask, size_t words) {
+    int launches = 0;
+    for (size_t j = 0; j < plan.voxel_depth.size(); ++j)
+        CU(icp_launch_voxel_level(src_pts, src_nrm, n, grid, Ts, plan.voxel_depth[j], table, mask + j * words, words, ctx->stream, &launches));
+    ctx->stats.n_kernel_launches += (uint64_t)launches;
+    return 0;
+}
+
 // The plan on the device, on the context's stream: the descriptors to desc (plan.n_iters entries, through the pinned staging), the
 // selection masks to mask -- the voxel pyramid's levels built on the device, or the mt19937 masks drawn on the host.  graph_reads:
 // the captured loop reads mask (ensure).
@@ -243,12 +255,8 @@ int upload_plan(icp_gpu_ctx* ctx, const Plan& plan, IterDesc* desc, DeviceBuf& m
         int dmax = 0; for (int D : plan.voxel_depth) dmax = D > dmax ? D : dmax;
         if (ensure(ctx, mask, plan.voxel_depth.size() * words * sizeof(uint32_t), graph_reads) ||
             ensure(ctx, ctx->voxel_table, sizeof(unsigned int) * ((size_t)1 << dmax), graph_reads)) return ICP_GPU_E_CUDA;
-        int launches = 0;
-        for (size_t j = 0; j < plan.voxel_depth.size(); ++j)
-            CU(icp_launch_voxel_level((const float4*)ctx->src_pts.p, (const float4*)ctx->src_nrm.p, ctx->n_src, (const GridParams*)ctx->sgrid.p,
-                                      ctx->Ts, plan.voxel_depth[j], (unsigned int*)ctx->voxel_table.p, (unsigned int*)mask.p + j * words,
-                                      words, ctx->stream, &launches));
-        ctx->stats.n_kernel_launches += (uint64_t)launches;
+        if (build_voxel_levels(ctx, plan, (const float4*)ctx->src_pts.p, (const float4*)ctx->src_nrm.p, ctx->n_src, (const GridParams*)ctx->sgrid.p,
+                               ctx->Ts, (unsigned int*)ctx->voxel_table.p, (unsigned int*)mask.p, words)) return ICP_GPU_E_CUDA;
     }
     if (!plan.mask.empty()) {
         if (ensure(ctx, mask, plan.mask.size() * sizeof(uint32_t), graph_reads)) return ICP_GPU_E_CUDA;

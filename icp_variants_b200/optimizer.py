@@ -270,6 +270,22 @@ class ICPOptimizer:
                 self.last_error.append(f"iteration {n}: singular / non-finite normal equations")
         return list(poses)
 
+    def estimatePoseBatchIndexed(self, sources, targets, initialPoses=None):
+        """Many independent registrations of any size with this optimizer's configuration, every target indexed on the device and
+        every pair run on its own thread-block cluster in one launch.  Returns the list of estimated poses; last_error as
+        estimatePoseBatch sets it.  The clouds set with setSource / setTarget are left as they are."""
+        self._ctx.set_config(self.config())
+        res = self._ctx.estimate_pose_batch_indexed(sources, targets, initialPoses)
+        self.last_error = []
+        for s, n in zip(res["status"], res["n_iterations"]):
+            if s == capi.OK:
+                self.last_error.append(None)
+            elif s == capi.E_NO_MATCHES:
+                self.last_error.append(f"iteration {n} had no surviving correspondence")
+            else:
+                self.last_error.append(f"iteration {n}: singular / non-finite normal equations")
+        return list(res["poses"])
+
     def estimatePoseMultiStart(self, source: PointCloud | None, target: PointCloud | None, initialPoses):
         """Multi-start registration: estimatePose from every pose of initialPoses [K,4,4] in one launch against one index of the
         target, each start scored at its final pose by its inliers (the matches that survive the matcher, weighting and rejection)

@@ -278,6 +278,38 @@ int icp_gpu_estimate_pose_multistart_dev(icp_gpu_ctx* ctx, int32_t n_starts, con
                                          int32_t* status_out, int64_t* inliers_out, double* rmse_out, float* pose_history, int32_t* match_idx_out,
                                          float* match_w_out);
 
+/* ---- many pairs of any size, each against its own index, in one launch --------------------------------------------------
+ * icp_gpu_estimate_pose_batch_indexed: B = n_pairs independent registrations with the context's configuration.  The clouds are
+ * concatenated as in icp_gpu_estimate_pose_batch: pair b owns source points [src_off[b], src_off[b+1]) and target points
+ * [tgt_off[b], tgt_off[b+1]) (B+1 offsets each, starting at 0); normals and colours (RGBA, 4 bytes a point) are nullable with the
+ * meaning icp_gpu_set_source / icp_gpu_set_target give to NULL.  The call builds an index of every pair's target (the one set_target
+ * builds), then runs every pair on its own thread-block cluster in one launch.  Per pair the outputs are exactly those of
+ * icp_gpu_estimate_pose_multistart with one start on a context holding that pair: poses_out[b] (B x 16 floats, column-major; pair b
+ * starts at poses_in[b]), n_iterations_out[b], status_out[b] (a failed pair keeps its last good pose), the scoring pass's
+ * inliers_out[b] and rmse_out[b], and with match_idx_out / match_w_out (nullable, together) sum(n_src) entries in each pair's original
+ * source order, pair b's at src_off[b].  pose_history (nullable): B x history_rows x 16 floats, history_rows at least the largest
+ * icp_gpu_iterations_bound over the batch's sources; rows past a pair's last iteration 0.  Accepted: what multistart accepts, pairs of
+ * any size, empty sources and targets included.  Refused with ICP_GPU_E_ARG: projective matching, ICP_GPU_NN_BRUTE_NORM, attached
+ * peers, a null required array or only one of the two match arrays, n_pairs < 0, offsets that do not start at 0 or are not monotone,
+ * a pair above set_target's size limit, sum(n_src) above INT32_MAX, history_rows below the bound when a history is asked for.
+ * ICP_GPU_E_STATE while a registration is pending.  n_pairs = 0: OK, nothing runs.  The context's clouds, index, pose, remembered
+ * neighbours and graphs are left as they are.  _dev: every array is a device pointer on the context's device.  The call waits for
+ * its work either way.  Measured on one B200 at 1000 W, point-to-plane, from host arrays, every arm on warmed contexts (DESIGN.md
+ * section 6): against a loop of set_target + set_source + icp_gpu_estimate_pose on one context it pays 2.2x to 2.7x for 64 to 4096
+ * small or ~12.9k-point pairs, only 1.2x to 1.3x for ~45k-point pairs, and it LOSES for a single pair (0.48x).  Against the same
+ * registrations spread over three contexts (alignPairs) it is 0.93x to 1.02x for ~12.9k-point, 8192-point and bunny-sized pairs and
+ * 0.5x for ~45k-point pairs and for a single pair.  Against icp_gpu_estimate_pose_batch it is 35x faster on 8192-point pairs and
+ * 0.19x on bunny-sized pairs.  The pairs' index builds run one after another and take 0.5 to 0.97 of the call. */
+int icp_gpu_estimate_pose_batch_indexed(icp_gpu_ctx* ctx, int32_t n_pairs, const float* src_xyz, const float* src_nrm, const uint8_t* src_rgba,
+                                        const int64_t* src_off, const float* tgt_xyz, const float* tgt_nrm, const uint8_t* tgt_rgba, const int64_t* tgt_off,
+                                        const float* poses_in, float* poses_out, int32_t* n_iterations_out, int32_t* status_out, int64_t* inliers_out,
+                                        double* rmse_out, float* pose_history, int32_t history_rows, int32_t* match_idx_out, float* match_w_out);
+int icp_gpu_estimate_pose_batch_indexed_dev(icp_gpu_ctx* ctx, int32_t n_pairs, const float* src_xyz, const float* src_nrm, const uint8_t* src_rgba,
+                                            const int64_t* src_off, const float* tgt_xyz, const float* tgt_nrm, const uint8_t* tgt_rgba,
+                                            const int64_t* tgt_off, const float* poses_in, float* poses_out, int32_t* n_iterations_out,
+                                            int32_t* status_out, int64_t* inliers_out, double* rmse_out, float* pose_history, int32_t history_rows,
+                                            int32_t* match_idx_out, float* match_w_out);
+
 int icp_gpu_get_stats(icp_gpu_ctx* ctx, icp_gpu_stats* out);
 /* The FP32 (non-tensor) roofline denominator of the context's device, measured with a register-resident microbenchmark on
  * the context's stream (SURVEY.md 8d; the reference has no counterpart): mode 0 = FFMA (2 flop / instruction), mode 1 =
