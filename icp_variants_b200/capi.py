@@ -126,6 +126,8 @@ def lib():
             "icp_gpu_solve_linear": (C.c_int, [vp, i32, pf, pf, pf, pf, pf, i64, pf]),
             "icp_gpu_cloud_from_depth": (C.c_int, [vp, pf, pf, pf, pf, u32, u32, C.c_int, u32, C.c_float, C.c_int, pf, pf, pf, C.POINTER(i64)]),
             "icp_gpu_target_normals": (C.c_int, [vp, i32, pf, pf, pf]),
+            "icp_gpu_voxel_downsample": (C.c_int, [vp, i32, pf, pf, pf, pf, C.c_float, C.c_int, pf, pf, pf, pf]),
+            "icp_gpu_voxel_downsample_dev": (C.c_int, [vp, i32, pf, pf, pf, pf, C.c_float, C.c_int, pf, pf, pf, pf]),
             "icp_gpu_set_correspondences": (C.c_int, [vp, pf, pf, i64]),
             "icp_gpu_set_correspondences_pose": (C.c_int, [vp, pf]),
             "icp_gpu_convergence_errors": (C.c_int, [vp, pf, pf, i32, C.POINTER(i32)]),
@@ -669,6 +671,78 @@ class Context:
         if not download:
             return n.value
         return po[:n.value].copy(), no[:n.value].copy(), co[:n.value].copy()
+
+    def voxel_downsample(self, xyz, voxel_size, nrm=None, rgba=None, role: int = 2):
+        """Voxel-grid filter of one cloud on the device (icp_gpu_voxel_downsample): one centroid per occupied voxel of edge
+        voxel_size.  role 0: the result becomes the target (indexed), 1: the source, 2: only returned.  Returns (points [M,3],
+        normals [M,3] or None, colours [M,4] uint8 or None)."""
+        xyz, nrm, rgba = _f32(xyz, 3), _f32(nrm, 3), _u8(rgba)
+        for x, name in ((nrm, "nrm"), (rgba, "rgba")):
+            if x is not None and len(x) != len(xyz):
+                raise ValueError(f"{name}: {len(x)} rows for {len(xyz)} points")
+        off = np.array([0, len(xyz)], np.int64)
+        out = self._voxel_host(xyz, nrm, rgba, off, voxel_size, role)
+        if role == 1:
+            self.n_source = len(out[0])
+        return out[:3]
+
+    def voxel_downsample_batch(self, clouds, voxel_size):
+        """The filter of many clouds in one call (synth.Cloud or [N,3] arrays, optional normals and colours): a list of clouds
+        (points, normals or None, colours or None), in the order given."""
+        xyz, n3, c4, off = _concat_clouds_rgba(clouds)
+        po, no, co, oo = self._voxel_host(xyz, n3, c4, off, voxel_size, 2)
+        return [(po[oo[b]:oo[b + 1]], None if no is None else no[oo[b]:oo[b + 1]], None if co is None else co[oo[b]:oo[b + 1]])
+                for b in range(len(off) - 1)]
+
+    def _voxel_host(self, xyz, nrm, rgba, off, voxel_size, role):
+        cap = max(int(off[-1]), 1)
+        po = np.empty((cap, 3), np.float32)
+        no = np.empty((cap, 3), np.float32) if nrm is not None else None
+        co = np.empty((cap, 4), np.uint8) if rgba is not None else None
+        oo = np.zeros(len(off), np.int64)
+        self._check(lib().icp_gpu_voxel_downsample(self._h, len(off) - 1, _ptr(xyz), _ptr(nrm), _ptr(rgba), _ptr(off), float(voxel_size), int(role),
+                                                   _ptr(po), _ptr(no), _ptr(co), _ptr(oo)))
+        m = int(oo[-1])
+        return po[:m].copy(), None if no is None else no[:m].copy(), None if co is None else co[:m].copy(), oo
+
+    def voxel_downsample_dev(self, xyz, off, voxel_size, nrm=None, rgba=None, role: int = 2):
+        """The filter on CUDA torch tensors of the context's device: concatenated points / normals [N,3] float32, colours [N,4] uint8,
+        offsets [B+1] int64.  Returns (points [M,3], normals or None, colours or None, offsets [B+1] int64), CUDA tensors, cloud b's
+        voxels at [off_out[b], off_out[b+1]).  Work queued on the current torch stream is waited for; the results are complete when
+        the call returns."""
+        import torch
+        dev = torch.device("cuda", self.device)
+
+        def arr(x, name, dtype, cols):
+            if x is None:
+                return None
+            if not (isinstance(x, torch.Tensor) and x.device == dev and x.dtype == dtype and x.dim() == 2 and x.shape[1] == cols):
+                raise ValueError(f"{name}: expected a {dtype} [N,{cols}] tensor on {dev}")
+            return x.contiguous()
+
+        xyz, nrm, rgba = arr(xyz, "xyz", torch.float32, 3), arr(nrm, "nrm", torch.float32, 3), arr(rgba, "rgba", torch.uint8, 4)
+        if not (isinstance(off, torch.Tensor) and off.device == dev and off.dtype == torch.int64 and off.dim() == 1 and len(off) >= 1):
+            raise ValueError(f"off: expected an int64 [B+1] tensor on {dev}")
+        off = off.contiguous()
+        for x, name in ((nrm, "nrm"), (rgba, "rgba")):
+            if x is not None and len(x) != len(xyz):
+                raise ValueError(f"{name}: {len(x)} rows for {len(xyz)} points")
+        cap = max(len(xyz), 1)
+        po = torch.empty((cap, 3), dtype=torch.float32, device=dev)
+        no = torch.empty((cap, 3), dtype=torch.float32, device=dev) if nrm is not None else None
+        co = torch.empty((cap, 4), dtype=torch.uint8, device=dev) if rgba is not None else None
+        oo = torch.zeros(len(off), dtype=torch.int64, device=dev)
+
+        def p(x):
+            return None if x is None else C.c_void_p(x.data_ptr())
+
+        torch.cuda.current_stream(dev).synchronize()
+        self._check(lib().icp_gpu_voxel_downsample_dev(self._h, len(off) - 1, p(xyz), p(nrm), p(rgba), p(off), float(voxel_size), int(role),
+                                                       p(po), p(no), p(co), p(oo)))
+        m = int(oo[-1]) if len(off) > 1 else 0
+        if role == 1:
+            self.n_source = m
+        return po[:m], None if no is None else no[:m], None if co is None else co[:m], oo
 
     def target_normals(self, k: int = 5, viewpoint=None, n: int | None = None, curvature: bool = False):
         """PointCloud(pcl cloud) (PointCloud.h:41-76): k-NN PCA normals of the resident target (n = its size); they also

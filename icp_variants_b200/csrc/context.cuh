@@ -63,6 +63,7 @@ struct icp_gpu_ctx {
     DeviceBuf batch_io, batch_scratch, batch_plan;           // batched registration: uploaded operands + results, match slices, configs + pair lists + masks
     DeviceBuf ms_io, ms_nn, ms_scratch, ms_desc, ms_mask;    // multi-start registration: operands + results, per-(start, query) neighbours and match slices, plan
     DeviceBuf bi_io, bi_arena, bi_scratch, bi_plan;          // indexed batch: operands + results, per-pair clouds and indices, build scratch, plans + pair table
+    DeviceBuf vox_io, vox_tmp;                               // voxel downsampling: operands + results, voxel records + sort + compaction
     long long n_gt = 0; int last_iters = 0;
     float* h_pose = nullptr; float* h_history = nullptr; DevState* h_state = nullptr;   // pinned
     IterDesc* h_desc = nullptr;                                                       // pinned, DESC_TOTAL

@@ -404,6 +404,31 @@ size_t icp_radix_hist_words(int n, int T) {
     return (size_t)p.n_pass * RS_MAX_BINS * p.tiles_pad + RS_MAX_BINS;
 }
 
+void icp_radix_passes(const IcpRadixPlan& p, int n, unsigned int* kin, unsigned int* kout, unsigned int* iin, unsigned int* idx_a, unsigned int* idx_b,
+                      unsigned int* hist, unsigned int* msd_start, cudaStream_t s, unsigned int** keys_sorted_out, unsigned int** idx_sorted_out,
+                      int* launches) {
+    unsigned int* iout = idx_a;
+    const size_t mat = (size_t)RS_MAX_BINS * p.tiles_pad;
+    unsigned int* totals = hist + (size_t)p.n_pass * mat;
+    for (int k = 0; k < p.n_pass && n > 0; ++k) {
+        const bool last = k == p.n_pass - 1;
+        const int bins = 1 << p.bits[k];
+        radix_scan_kernel<<<(bins * 32 + 255) / 256, 256, 0, s>>>(hist + k * mat, bins, p.n_tiles, p.tiles_pad, totals); ++*launches;
+        unsigned int* hn = last ? nullptr : hist + (k + 1) * mat;
+        const int sn = last ? 0 : p.shift[k + 1], bn = last ? 1 : p.bits[k + 1];
+        if (p.ipt <= RS_REG_IPT)
+            radix_scatter_kernel<true><<<p.n_tiles, RS_THREADS, 0, s>>>(kin, iin, kout, iout, n, p.ipt, p.tiles_pad, p.shift[k], p.bits[k], hist + k * mat, totals, hn, sn, bn,
+                                                                       last ? msd_start : nullptr);
+        else
+            radix_scatter_kernel<false><<<p.n_tiles, RS_THREADS, 0, s>>>(kin, iin, kout, iout, n, p.ipt, p.tiles_pad, p.shift[k], p.bits[k], hist + k * mat, totals, hn, sn, bn,
+                                                                        last ? msd_start : nullptr);
+        ++*launches;
+        unsigned int* t = kin; kin = kout; kout = t;
+        iin = iout; iout = (iout == idx_a) ? idx_b : idx_a;
+    }
+    *keys_sorted_out = kin; *idx_sorted_out = iin;
+}
+
 // Sorts a packed cloud into (cell code, original index) order.  grid / hist: written / cleared by icp_launch_pack_cloud on the
 // same stream before.  keys_a / keys_b: n entries each (the sorted keys end up in *keys_sorted_out, one of the two);
 // idx_a / idx_b: n entries each; hist: icp_radix_hist_words(); msd_start: ICP_MSD_WORDS entries (nullable).
@@ -414,27 +439,9 @@ cudaError_t icp_launch_cloud_sort(const float4* pts_in, const float4* nrm_in, in
     IcpRadixPlan p; icp_radix_plan(n, T, &p);
     int launches = 0;
     if (msd_shift_out) *msd_shift_out = p.shift[p.n_pass - 1];
-    unsigned int* kin = keys_a; unsigned int* kout = keys_b;
-    unsigned int* iin = nullptr; unsigned int* iout = idx_a;
-    const size_t mat = (size_t)RS_MAX_BINS * p.tiles_pad;
-    unsigned int* totals = hist + (size_t)p.n_pass * mat;
-    if (n > 0) { keys_kernel<<<(n + KEY_THREADS - 1) / KEY_THREADS, KEY_THREADS, 0, s>>>(pts_in, n, grid, kin, p.tile_items, p.tiles_pad, p.shift[0], p.bits[0], hist); ++launches; }
-    for (int k = 0; k < p.n_pass && n > 0; ++k) {
-        const bool last = k == p.n_pass - 1;
-        const int bins = 1 << p.bits[k];
-        radix_scan_kernel<<<(bins * 32 + 255) / 256, 256, 0, s>>>(hist + k * mat, bins, p.n_tiles, p.tiles_pad, totals); ++launches;
-        unsigned int* hn = last ? nullptr : hist + (k + 1) * mat;
-        const int sn = last ? 0 : p.shift[k + 1], bn = last ? 1 : p.bits[k + 1];
-        if (p.ipt <= RS_REG_IPT)
-            radix_scatter_kernel<true><<<p.n_tiles, RS_THREADS, 0, s>>>(kin, iin, kout, iout, n, p.ipt, p.tiles_pad, p.shift[k], p.bits[k], hist + k * mat, totals, hn, sn, bn,
-                                                                       last ? msd_start : nullptr);
-        else
-            radix_scatter_kernel<false><<<p.n_tiles, RS_THREADS, 0, s>>>(kin, iin, kout, iout, n, p.ipt, p.tiles_pad, p.shift[k], p.bits[k], hist + k * mat, totals, hn, sn, bn,
-                                                                        last ? msd_start : nullptr);
-        ++launches;
-        unsigned int* t = kin; kin = kout; kout = t;
-        iin = iout; iout = (iout == idx_a) ? idx_b : idx_a;
-    }
+    if (n > 0) { keys_kernel<<<(n + KEY_THREADS - 1) / KEY_THREADS, KEY_THREADS, 0, s>>>(pts_in, n, grid, keys_a, p.tile_items, p.tiles_pad, p.shift[0], p.bits[0], hist); ++launches; }
+    unsigned int *kin, *iin;
+    icp_radix_passes(p, n, keys_a, keys_b, nullptr, idx_a, idx_b, hist, msd_start, s, &kin, &iin, &launches);
     if (n > 0) {
         if (late) {
             // the normal records (nrm_in) are packed only now: their upload had the whole sort to finish

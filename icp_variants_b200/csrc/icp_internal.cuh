@@ -300,6 +300,27 @@ cudaError_t icp_launch_apply_weights(int method, float max_d2, const float* sp, 
                                      const unsigned int* tc, long long n_tgt, const int* idx, float* w, long long n, cudaStream_t s);
 cudaError_t icp_launch_pack_pairs(const float* s, const float* sn, const float* t, const float* tn, const float* w, int n, float4* sp4, float4* sn4,
                                   float4* tp4, float4* tn4, int* pos, float* wo, cudaStream_t st);
+// prep.cu: the count and scan of an order-preserving compaction of n 0/1 flags: block_offset[k] = flags set before block k of
+// ICP_FLAG_SCAN_BLOCK flags, *total = flags set.  block_offset: one entry per block.
+#define ICP_FLAG_SCAN_BLOCK 256
+cudaError_t icp_launch_flag_scan(const unsigned int* flag, long long n, unsigned int* block_offset, unsigned int* total, cudaStream_t s, int* n_launches);
+// voxel.cu: voxel-grid downsampling of n_clouds concatenated clouds (DESIGN.md section 4, V1-V5).
+// Widths of the fields of a voxel key (cloud, iz - min_z, iy - min_y, ix - min_x), most significant first, and its 32-bit words.
+struct VoxKeyLayout { int bx, by, bz, bc; int n_words; int top_bits; };
+// Each point's voxel (vox[i] = {ix, iy, iz, cloud}; cloud -1: a non-finite point) and each cloud's bounds: bounds[6c..6c+5] =
+// min x, y, z (initially INT_MAX), max x, y, z (initially INT_MIN); bad[c] = 1 when a voxel index of cloud c does not fit int32.
+cudaError_t icp_launch_voxel_coords(const float* xyz, int n, const long long* off, int n_clouds, float inv, int4* vox, int* bounds, unsigned int* bad,
+                                    cudaStream_t s, int* n_launches);
+// Stable sort of the points by voxel key (non-finite points last), key word by key word from the least significant.  keys_a / keys_b /
+// idx_a / idx_b: n entries each; hist: icp_radix_hist_words(n, 31) words.  *idx_sorted: original index per sorted position.
+cudaError_t icp_launch_voxel_sort(const int4* vox, int n, const int* bounds, const VoxKeyLayout& L, unsigned int* keys_a, unsigned int* keys_b,
+                                  unsigned int* idx_a, unsigned int* idx_b, unsigned int* hist, cudaStream_t s, unsigned int** idx_sorted, int* n_launches);
+// Runs of equal voxels in the sorted order -> one output record per voxel (V3-V5) and off_out (n_clouds + 1 entries, cleared by the
+// caller).  flag / run_start: n + 1 entries; block_offset: one per ICP_FLAG_SCAN_BLOCK points; *n_vox: the voxel count afterwards.
+// nrm / rgba and their outputs are nullable together.
+cudaError_t icp_launch_voxel_centroids(const unsigned int* idx_sorted, const int4* vox, int n, const float* xyz, const float* nrm, const uint8_t* rgba,
+                                       int n_clouds, unsigned int* flag, unsigned int* block_offset, unsigned int* n_vox, unsigned int* run_start,
+                                       float* xyz_out, float* nrm_out, uint8_t* rgba_out, long long* off_out, cudaStream_t s, int* n_launches);
 // peak.cu: measured FP32 throughput of the device (mode 0 FFMA, 1 FMUL+FADD), TFLOP/s
 cudaError_t icp_measure_fp32_peak(int mode, int n_sms, cudaStream_t s, double* tflops);
 // ---- launchers (defined in grid.cu / match.cu / knn.cu / solve.cu / lm.cu) ----
@@ -315,6 +336,13 @@ struct IcpRadixPlan { int n_pass; int shift[4]; int bits[4]; int ipt; int tile_i
 void icp_radix_plan(int n, int T, IcpRadixPlan* p);
 size_t icp_radix_hist_words(int n, int T);
 #define ICP_MSD_WORDS 257
+// The passes of that sort (plan p) over keys kin whose pass-0 digit histogram the caller's key kernel has counted into the cleared
+// hist (icp_radix_hist_words, digit-major per tile, as keys_kernel counts it).  iin: the items' indices (null: the identity); the
+// indices move through idx_a / idx_b, starting with idx_a, so iin may be idx_b but not idx_a.  kout: scratch of n keys.  The sorted
+// keys and indices are left in *keys_sorted_out / *idx_sorted_out (kin or kout, idx_a or idx_b).
+void icp_radix_passes(const IcpRadixPlan& p, int n, unsigned int* kin, unsigned int* kout, unsigned int* iin, unsigned int* idx_a, unsigned int* idx_b,
+                      unsigned int* hist, unsigned int* msd_start, cudaStream_t s, unsigned int** keys_sorted_out, unsigned int** idx_sorted_out,
+                      int* launches);
 cudaError_t icp_launch_cloud_sort(const float4* pts_in, const float4* nrm_in, int n, int T, const GridParams* grid,
                                   unsigned int* keys_a, unsigned int* keys_b, unsigned int* idx_a, unsigned int* idx_b,
                                   unsigned int* hist, float4* pts_sorted, float4* nrm_sorted, unsigned int* msd_start,

@@ -116,6 +116,16 @@ cudaError_t icp_launch_depth_cloud(const float* depth, const unsigned char* colo
     return cudaGetLastError();
 }
 
+static_assert(PREP_THREADS == ICP_FLAG_SCAN_BLOCK, "the compaction's blocks are PREP_THREADS flags");
+cudaError_t icp_launch_flag_scan(const unsigned int* flag, long long n, unsigned int* block_offset, unsigned int* total, cudaStream_t s, int* n_launches) {
+    if (n <= 0) return cudaMemsetAsync(total, 0, 4, s);
+    const int nb = (int)((n + PREP_THREADS - 1) / PREP_THREADS);
+    flag_count_kernel<<<nb, PREP_THREADS, 0, s>>>(flag, n, block_offset);
+    block_scan_kernel<<<1, 1024, 0, s>>>(block_offset, nb, total);
+    if (n_launches) *n_launches += 2;
+    return cudaGetLastError();
+}
+
 // ---------------------------------------------------------------------------- convergence metrics
 // The correspondences reconstructRoom uses (main.cpp:300-307): every source point against itself under a ground-truth
 // pose, gtTargetPoints = transformPoints(source.getPoints(), currentToZeroCoordinates), built from the resident source.

@@ -338,6 +338,32 @@ int icp_gpu_cloud_from_depth(icp_gpu_ctx* ctx, const float* depth, const uint8_t
  * target's own for the following registrations and are returned in the caller's point order (nrm_out: 3*n floats,
  * curvature_out: n floats, both nullable).  3 <= k <= 8. */
 int icp_gpu_target_normals(icp_gpu_ctx* ctx, int32_t k, const float viewpoint[3], float* nrm_out, float* curvature_out);
+/* icp_gpu_voxel_downsample: a voxel-grid filter (pcl::VoxelGrid, Open3D's voxel_down_sample) of n_clouds clouds in one pass: one
+ * point per occupied voxel of edge voxel_size, the centroid of the voxel's points.  Cloud b is points [off[b], off[b+1]) (n_clouds+1
+ * offsets, starting at 0, monotone, as icp_gpu_estimate_pose_batch_indexed takes them); nrm and rgba are nullable.  Cloud b's voxels
+ * come back at [off_out[b], off_out[b+1]) of xyz_out / nrm_out / rgba_out, each of which needs room for off[n_clouds] points.
+ * Arithmetic (DESIGN.md section 4, V1-V5): only points with three finite coordinates are used; a point's voxel is
+ * floorf(x * (1.0f / voxel_size)) per axis (PCL's world-anchored grid: clouds filtered at one size share it); a cloud's voxels come in
+ * ascending (iz, iy, ix); a coordinate is the fp64 sum of the voxel's points in ascending input order over their count, rounded once
+ * to fp32; a normal the same sum over the points whose normal is finite, over its fp64 norm (MINF when there is none or the norm is
+ * 0); a colour channel (2 sum + k) / 2k in integers.  The result is a fixed function of the input, bit for bit.  nrm_out / rgba_out
+ * are written only when nrm / rgba are given.  role (the values of icp_gpu_cloud_from_depth): with TARGET or SOURCE (n_clouds must
+ * be 1) the result becomes the context's target, indexed, or source, as set_target / set_source of the returned arrays would make
+ * it, and every output is nullable; with ONLY the context's clouds, index, pose, remembered neighbours and graphs stay as they are,
+ * and xyz_out and off_out are required.  Refused with ICP_GPU_E_ARG: n_clouds < 0, a null required array, a non-null nrm_out /
+ * rgba_out without its input, offsets that do not start at 0 or are not monotone, voxel_size not finite and > 0, a role out of range
+ * or TARGET / SOURCE with n_clouds != 1, more than set_target's limit of points in all, a cloud whose finite points span more than
+ * 2^21 voxels on an axis or whose voxel index does not fit int32 (the message names the cloud).  ICP_GPU_E_STATE while a
+ * registration is pending.  n_clouds = 0: OK, nothing runs.  The kernels launched do not depend on n_clouds.  _dev: every array is
+ * a device pointer on the context's device.  The call waits for its work either way.  Measured on one B200 at 1000 W (DESIGN.md
+ * section 6): a 370k-point lidar scan takes 0.64 ms (_dev) at 2 cm and 5.9 ms at 20 cm -- one thread sums each voxel, so the largest
+ * voxel bounds the call -- 85x to 7.6x the host round trip (download, filter on one core, upload); a 3 M-point scan at 5 cm 15.7 ms
+ * (27x); batches of 44 to 512 scans in one call 17x to 24x a loop of single-cloud calls.  Where it loses: tiny clouds (the 1k-point
+ * bunny: 0.18 ms, 0.72x a host filter on one core). */
+int icp_gpu_voxel_downsample(icp_gpu_ctx* ctx, int32_t n_clouds, const float* xyz, const float* nrm, const uint8_t* rgba, const int64_t* off,
+                             float voxel_size, int role, float* xyz_out, float* nrm_out, uint8_t* rgba_out, int64_t* off_out);
+int icp_gpu_voxel_downsample_dev(icp_gpu_ctx* ctx, int32_t n_clouds, const float* xyz, const float* nrm, const uint8_t* rgba, const int64_t* off,
+                                 float voxel_size, int role, float* xyz_out, float* nrm_out, uint8_t* rgba_out, int64_t* off_out);
 /* ConvergenceMeasure(sourcePoints, unchangedPoints) (ConvergenceMeasure.h:32-41): m known correspondences
  * (source point i of the UNTRANSFORMED source <-> reference point i). */
 int icp_gpu_set_correspondences(icp_gpu_ctx* ctx, const float* src_xyz, const float* ref_xyz, int64_t m);
